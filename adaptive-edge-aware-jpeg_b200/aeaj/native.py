@@ -20,12 +20,12 @@ EXPORTS = [
     "aeaj_percentile_thresholds", "aeaj_canny_u8", "aeaj_canny", "aeaj_quadtree_caps", "aeaj_quadtree",
     "aeaj_dct_quant", "aeaj_dequant_idct", "aeaj_plan_create", "aeaj_plan_destroy", "aeaj_plan_get_info",
     "aeaj_plan_set_qtables", "aeaj_encode", "aeaj_decode", "aeaj_plan_last_launches",
-    "aeaj_plan_enable_timing", "aeaj_plan_read_timing", "aeaj_encode_phase", "aeaj_decode_phase", "aeaj_plan_buffers",
+    "aeaj_plan_enable_timing", "aeaj_plan_read_timing",
     "aeaj_plan_set_stream_layout", "aeaj_plan_set_tensor_dct", "aeaj_tensor_dct_status",
     "aeaj_states_to_leaves_host", "aeaj_pack_states_host",
     "aeaj_pack_coefficients", "aeaj_unpack_coefficients", "aeaj_pack_coefficients_host", "aeaj_unpack_coefficients_host",
     "aeaj_peer_alloc", "aeaj_peer_free", "aeaj_peer_export", "aeaj_peer_open", "aeaj_peer_close",
-    "aeaj_plan_set_peers", "aeaj_plan_peer_barrier", "aeaj_plan_peer_gather", "aeaj_copy_segments",
+    "aeaj_plan_set_peers", "aeaj_copy_segments",
     "aeaj_encode_halo", "aeaj_decode_halo", "aeaj_set_fast_transfer",
 ]
 
@@ -59,12 +59,6 @@ class PackedIO(C.Structure):
 
 class Segment(C.Structure):
     _fields_ = [("src", C.c_void_p), ("dst", C.c_void_p), ("bytes", C.c_int64)]
-
-
-class PlanBuffers(C.Structure):
-    _fields_ = [("layer", C.c_void_p * 3), ("u8a", C.c_void_p * 3), ("u8b", C.c_void_p * 3), ("strong", C.c_void_p * 3),
-                ("weak", C.c_void_p * 3), ("h", C.c_int * 3), ("w", C.c_int * 3), ("wpr", C.c_int * 3),
-                ("clahe_hist", C.c_void_p), ("clahe_hist_bytes", C.c_int64), ("hist", C.c_void_p), ("hist_bytes", C.c_int64)]
 
 
 _lib = None
@@ -117,16 +111,13 @@ def load():
         lib.aeaj_plan_set_stream_layout.argtypes = [vp, i]
         lib.aeaj_plan_set_tensor_dct.argtypes = [vp, i]
         lib.aeaj_tensor_dct_status.argtypes = [vp, C.POINTER(i)]
-        lib.aeaj_encode_phase.argtypes = [vp, C.POINTER(EncodeIO), vp, vp, i, i, i]
-        lib.aeaj_decode_phase.argtypes = [vp, C.POINTER(DecodeIO), vp, vp, i, i, i]
-        lib.aeaj_plan_buffers.argtypes = [vp, vp, C.POINTER(PlanBuffers)]
         lib.aeaj_plan_enable_timing.argtypes = [vp, i]
         lib.aeaj_plan_read_timing.argtypes = [vp, C.c_char_p, sz, vp, i, C.POINTER(i)]
         lib.aeaj_states_to_leaves_host.argtypes = [vp, i, i, i, i, i, i, vp, C.POINTER(i), C.POINTER(C.c_int64)]
         lib.aeaj_pack_states_host.argtypes = [vp, i, vp]
         lib.aeaj_set_fast_transfer.argtypes = [vp, i]
-        lib.aeaj_encode_halo.argtypes = [vp, C.POINTER(EncodeIO), vp, vp, i, i]
-        lib.aeaj_decode_halo.argtypes = [vp, C.POINTER(DecodeIO), vp, vp, i, i]
+        lib.aeaj_encode_halo.argtypes = [vp, C.POINTER(EncodeIO), vp, vp, i]
+        lib.aeaj_decode_halo.argtypes = [vp, C.POINTER(DecodeIO), vp, vp, i]
         lib.aeaj_copy_segments.argtypes = [C.POINTER(Segment), i, vp, vp]
         lib.aeaj_peer_alloc.argtypes = [sz, C.POINTER(vp)]
         lib.aeaj_peer_free.argtypes = [vp]
@@ -134,8 +125,6 @@ def load():
         lib.aeaj_peer_open.argtypes = [vp, C.POINTER(vp)]
         lib.aeaj_peer_close.argtypes = [vp]
         lib.aeaj_plan_set_peers.argtypes = [vp, i, i, C.POINTER(vp), C.POINTER(vp)]
-        lib.aeaj_plan_peer_barrier.argtypes = [vp, vp]
-        lib.aeaj_plan_peer_gather.argtypes = [vp, i, vp, vp]
         lib.aeaj_pack_coefficients.argtypes = [vp, C.POINTER(vp), vp, C.POINTER(PackedIO), vp, vp]
         lib.aeaj_unpack_coefficients.argtypes = [vp, C.POINTER(PackedIO), C.POINTER(vp), vp, vp]
         lib.aeaj_pack_coefficients_host.argtypes = [vp, C.c_int64, vp, vp, C.POINTER(C.c_int64), C.POINTER(i)]

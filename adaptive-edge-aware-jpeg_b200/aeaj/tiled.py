@@ -8,11 +8,11 @@ prefilter, Sobel / NMS, the quadtree and the DCT -- and nothing on the data path
     workspace is at offset o of every peer's, so the stencil kernels read the 3 / 2 / 1 halo rows outside their band
     straight from the neighbour GPU over NVLink, and the CLAHE / percentile kernels sum the per-rank partial
     histograms on the fly;
-  * between phases the ranks meet at a device-side barrier (``aeaj_plan_peer_barrier``: one tiny kernel per rank that
-    stores an epoch into every peer's flag array and spins on its own, ordered with the data by the stream);
-  * two small gathers (``aeaj_plan_peer_gather``) copy the other bands' rows of the strong / weak bitmaps (the
-    hysteresis fixed point is global; at 0.15 ms per 64 MP it runs replicated) and of the quadtree block totals (the
-    scan over all top blocks needs them; counting and emitting are sharded).
+  * between phases the ranks meet at a device-side barrier (one tiny kernel per rank that stores an epoch into every
+    peer's flag array and spins on its own, ordered with the data by the stream);
+  * two small gathers copy the other bands' rows of the strong / weak bitmaps (the hysteresis fixed point is global;
+    at 0.15 ms per 64 MP it runs replicated) and of the quadtree block totals (the scan over all top blocks needs
+    them; counting and emitting are sharded).
 
     barrier                                   (the previous call's readers are done with this rank's planes)
     colour + subsample + u8 cast (band), CLAHE histograms (band)
@@ -25,12 +25,12 @@ prefilter, Sobel / NMS, the quadtree and the DCT -- and nothing on the data path
     DCT + quantise (band's leaves, coefficients at their global offsets)
 
 Decode: IDCT per band, barrier, upsample (1 chroma halo row from the neighbour) + inverse colour per band.
-Every rank ends with its band's leaves / states / coefficients at their global positions of the reference-ordered
-streams, bit-identical to the single-GPU result (tests/multi_gpu_halo.py, bench.py's C4 leg).  ``transport="nccl"`` is the
-round-1 exchange (whole-plane all-gathers, replicated quadtree), kept as a fallback for boxes without CUDA IPC.
+The library holds this schedule (``aeaj_encode_halo`` / ``aeaj_decode_halo``, one call per direction).  Every rank
+ends with its band's leaves / states / coefficients at their global positions of the reference-ordered streams,
+bit-identical to the single-GPU result (tests/multi_gpu_halo.py, bench.py's C4 leg).
 
-``emulate`` runs the G bands one after the other on ONE GPU through exactly the same phase calls (the buffers are
-shared, so the barriers and gathers are no-ops); the GPU tests use it to check the band-restricted kernels.
+``emulate=G`` runs the same library schedule for all G bands on ONE GPU, band after band within each phase (the
+buffers are shared, so the barriers and gathers are no-ops); the GPU tests use it to check the band-restricted kernels.
 """
 from __future__ import annotations
 
@@ -42,8 +42,6 @@ import torch
 from . import native
 from .codec import DeviceCodec, EncodedBatch, _stream
 
-PH_COLOR, PH_HIST, PH_PREFILTER, PH_NMS, PH_TREE, PH_DCT, PH_HYST, PH_QT_COUNT, PH_QT_EMIT = range(9)
-DPH_IDCT, DPH_COLOR = range(2)
 BAND_ALIGN = 256
 
 
@@ -97,16 +95,15 @@ class _Peers:
 
 
 class TiledCodec:
-    def __init__(self, codec: DeviceCodec, rank: int = 0, world: int = 1, group=None, emulate: int = 0, transport: str = "peer"):
+    def __init__(self, codec: DeviceCodec, rank: int = 0, world: int = 1, group=None, emulate: int = 0):
         self.codec, self.rank, self.world, self.group, self.emulate = codec, rank, world, group, emulate
         self.lib = codec.lib
-        self.transport = transport if (world > 1 and not emulate) else "none"
         self._peers = {}
 
     # -- shared workspace --------------------------------------------------------------------------
     def _ws(self, p):
-        """device address of the plan workspace the phase calls use (the shared allocation in peer mode)"""
-        if self.transport != "peer":
+        """device address of the plan workspace the halo calls use (the shared allocation when the ranks are real GPUs)"""
+        if self.world <= 1 or self.emulate:
             return p.workspace.data_ptr()
         key = id(p)
         pe = self._peers.get(key)
@@ -128,44 +125,14 @@ class TiledCodec:
         p = self.codec._plan(1, H, W, space, brange, qrange)
         self.codec.check_status(p.out.status, "encode")
 
-    def _barrier(self, p):
-        if self.transport == "peer":
-            native.check(self.lib.aeaj_plan_peer_barrier(p.ptr, _stream()), "aeaj_plan_peer_barrier")
-
-    def _gather(self, p, what, ws):
-        if self.transport == "peer":
-            native.check(self.lib.aeaj_plan_peer_gather(p.ptr, what, ws, _stream()), "aeaj_plan_peer_gather")
-
-    # -- round-1 transport: NCCL all-gathers of whole planes -----------------------------------------
-    def _views(self, p):
-        buf = native.PlanBuffers()
-        native.check(self.lib.aeaj_plan_buffers(p.ptr, p.workspace.data_ptr(), C.byref(buf)), "aeaj_plan_buffers")
-        base = p.workspace.data_ptr()
-
-        def view(ptr, nbytes, dtype, shape):
-            off = ptr - base
-            return p.workspace[off:off + nbytes].view(dtype).view(shape)
-
-        v = dict(u8a=[], u8b=[], strong=[], weak=[], layer=[])
-        for l in range(3):
-            h, w, wpr = buf.h[l], buf.w[l], buf.wpr[l]
-            v["u8a"].append(view(buf.u8a[l], h * w, torch.uint8, (h, w)))
-            v["u8b"].append(view(buf.u8b[l], h * w, torch.uint8, (h, w)))
-            v["strong"].append(view(buf.strong[l], h * wpr * 4, torch.int32, (h, wpr)))
-            v["weak"].append(view(buf.weak[l], h * wpr * 4, torch.int32, (h, wpr)))
-            v["layer"].append(view(buf.layer[l], h * w * 4, torch.float32, (h, w)))
-        v["clahe_hist"] = view(buf.clahe_hist, buf.clahe_hist_bytes, torch.int32, (-1,))
-        v["hist"] = view(buf.hist, buf.hist_bytes, torch.int32, (-1,))
-        return v
-
-    def _gather_rows(self, full: torch.Tensor, H_layer: int):
-        import torch.distributed as dist
-        rows = H_layer // self.world
-        dist.all_gather_into_tensor(full.view(-1), full[self.rank * rows:(self.rank + 1) * rows].reshape(-1), group=self.group)
-
     def _reduce(self, t: torch.Tensor):
         import torch.distributed as dist
         dist.all_reduce(t, group=self.group)
+
+    def _band(self, H: int, brange):
+        """(number of bands, first row of this process's band): every band in emulation, this rank's otherwise"""
+        G = self.emulate or self.world
+        return G, band_of(0 if self.emulate else self.rank, G, H, brange[1])[0]
 
     # -- encode ---------------------------------------------------------------------------------
     def encode(self, rgb: torch.Tensor, H: int, W: int, space: str, qrange, brange, exchange_coef: bool = False) -> EncodedBatch:
@@ -181,71 +148,22 @@ class TiledCodec:
             io.coef[l], io.leaves[l], io.states[l] = o.coef[l].data_ptr(), o.leaves[l].data_ptr(), o.states[l].data_ptr()
         io.counts, io.status = o.counts.data_ptr(), o.status.data_ptr()
         ws = self._ws(p)
-        G = self.emulate or self.world
-        ranks = range(G) if self.emulate else [self.rank]
+        G, lo = self._band(H, brange)
         rgb = rgb.contiguous()
+        # the kernel indexes rows from the top of the full image: hand it the (virtual) address of row 0
+        io.rgb = rgb.data_ptr() - lo * W * 12
         multi = not self.emulate and self.world > 1
-
-        def run(phase, r):
-            lo, hi = band_of(r, G, H, brange[1])
-            # the kernel indexes rows from the top of the full image: hand it the (virtual) address of row 0
-            io.rgb = rgb.data_ptr() - (0 if self.emulate else lo * W * 12)
-            native.check(self.lib.aeaj_encode_phase(p.ptr, C.byref(io), ws, _stream(), phase, lo, hi), f"aeaj_encode_phase({phase})")
-
-        def each(phase):
-            for r in ranks:
-                run(phase, r)
-
         if multi and exchange_coef:
             for l in range(3):
                 o.coef[l].zero_(); o.leaves[l].zero_(); o.states[l].zero_()
-        if self.transport == "nccl":
-            v = self._views(p)
-            each(PH_COLOR); each(PH_HIST)
-            self._reduce(v["clahe_hist"])
-            for l in range(3):
-                self._gather_rows(v["u8a"][l], p.info.layer_h[l])
-            each(PH_PREFILTER)
-            self._reduce(v["hist"])
-            for l in range(3):
-                self._gather_rows(v["u8b"][l], p.info.layer_h[l])
-            each(PH_NMS)
-            for l in range(3):
-                self._gather_rows(v["strong"][l], p.info.layer_h[l])
-                self._gather_rows(v["weak"][l], p.info.layer_h[l])
-            lo, hi = band_of(self.rank, G, H, brange[1])
-            io.rgb = rgb.data_ptr() - lo * W * 12
-            native.check(self.lib.aeaj_encode_phase(p.ptr, C.byref(io), ws, _stream(), PH_TREE, 0, H), "aeaj_encode_phase(tree)")
-            each(PH_DCT)
-        elif self.transport == "peer":
-            # one foreign call runs the whole schedule below for this rank (the phase calls are what emulation uses)
-            lo, hi = band_of(self.rank, G, H, brange[1])
-            io.rgb = rgb.data_ptr() - lo * W * 12
-            native.check(self.lib.aeaj_encode_halo(p.ptr, C.byref(io), ws, _stream(), lo, hi), "aeaj_encode_halo")
-        else:
-            self._barrier(p)                  # the previous call's neighbours are done reading this rank's planes
-            each(PH_COLOR)                    # also clears the histogram accumulators (before any histogram work)
-            each(PH_HIST)
-            self._barrier(p)
-            each(PH_PREFILTER)
-            self._barrier(p)
-            each(PH_NMS)
-            self._barrier(p)
-            self._gather(p, 0, ws)
-            run(PH_HYST, ranks[0])            # whole image, replicated (the band argument is irrelevant for this phase)
-            each(PH_QT_COUNT)
-            self._barrier(p)
-            self._gather(p, 1, ws)
-            each(PH_QT_EMIT)
-            each(PH_DCT)
+        native.check(self.lib.aeaj_encode_halo(p.ptr, C.byref(io), ws, _stream(), G), "aeaj_encode_halo")
         if multi and exchange_coef:
             import torch.distributed as dist
             for l in range(3):
-                if self.transport == "peer":
-                    # sharded quadtree: every rank wrote only its band's leaves / states (zero elsewhere: sum); the all-split levels
-                    # above the top blocks and the absent nodes are written by every rank with the same value: maximum
-                    self._reduce(o.leaves[l])
-                    dist.all_reduce(o.states[l], op=dist.ReduceOp.MAX, group=self.group)
+                # sharded quadtree: every rank wrote only its band's leaves / states (zero elsewhere: sum); the all-split levels
+                # above the top blocks and the absent nodes are written by every rank with the same value: maximum
+                self._reduce(o.leaves[l])
+                dist.all_reduce(o.states[l], op=dist.ReduceOp.MAX, group=self.group)
                 self._reduce(o.coef[l])
         return o
 
@@ -259,26 +177,6 @@ class TiledCodec:
             io.coef[l], io.leaves[l] = enc.coef[l].data_ptr(), enc.leaves[l].data_ptr()
         io.counts, io.rgb = enc.counts.data_ptr(), p.rgb_out.data_ptr()
         ws = self._ws(p)
-        G = self.emulate or self.world
-        ranks = range(G) if self.emulate else [self.rank]
-
-        def run(phase, r):
-            lo, hi = band_of(r, G, H, brange[1])
-            native.check(self.lib.aeaj_decode_phase(p.ptr, C.byref(io), ws, _stream(), phase, lo, hi), f"aeaj_decode_phase({phase})")
-
-        if self.transport == "peer":
-            lo, hi = band_of(self.rank, G, H, brange[1])
-            native.check(self.lib.aeaj_decode_halo(p.ptr, C.byref(io), ws, _stream(), lo, hi), "aeaj_decode_halo")
-            return p.rgb_out[0]
-        for r in ranks:
-            run(DPH_IDCT, r)
-        if self.transport == "nccl":
-            v = self._views(p)
-            for l in (1, 2):
-                if p.info.layer_h[l] != H or p.info.layer_w[l] != W:
-                    self._gather_rows(v["layer"][l], p.info.layer_h[l])
-        else:
-            self._barrier(p)
-        for r in ranks:
-            run(DPH_COLOR, r)
+        G, _ = self._band(H, brange)
+        native.check(self.lib.aeaj_decode_halo(p.ptr, C.byref(io), ws, _stream(), G), "aeaj_decode_halo")
         return p.rgb_out[0]

@@ -674,6 +674,19 @@ static int set_band(aeaj_plan* p, int band0, int band1) {
     return 0;
 }
 
+// The phases of an encode / decode, in the order one call runs them.  `phases` of encode_impl / decode_impl is a bit set of them;
+// [band0, band1) restricts every phase but hysteresis to a band of full-resolution rows (the halo-split schedule below).
+enum { AEAJ_PHASE_COLOR = 0,      /* clears accumulators; colour + subsample + u8 cast of the band                             */
+       AEAJ_PHASE_CLAHE_HIST = 1, /* CLAHE tile histograms of the band                                                         */
+       AEAJ_PHASE_PREFILTER = 2,  /* LUTs (sum of every band's partial histograms) + CLAHE / Gauss / bilateral of the band      */
+       AEAJ_PHASE_NMS = 3,        /* thresholds (sum of every band's partial histograms) + Sobel / NMS of the band              */
+       AEAJ_PHASE_HYST = 4,       /* hysteresis, whole image (needs every band's strong / weak rows)                           */
+       AEAJ_PHASE_QT_COUNT = 5,   /* quadtree: node counts of the band's top blocks                                            */
+       AEAJ_PHASE_QT_EMIT = 6,    /* needs every band's counts; scan + states / leaves / work lists of the band                */
+       AEAJ_PHASE_DCT = 7 };      /* DCT + quantise of the band's leaves (coefficients at global offsets)                      */
+enum { AEAJ_DPHASE_IDCT = 0,      /* dequantise + IDCT + merge of the band's leaves                                            */
+       AEAJ_DPHASE_COLOR = 1 };   /* needs the neighbouring chroma rows; upsample + inverse colour of the band                  */
+
 static int encode_impl(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, cudaStream_t st, unsigned phases, int band0, int band1) {
     AEAJ_REQUIRE(p && io && workspace && (io->rgb || io->rgb_u8) && io->counts, "aeaj_encode: bad arguments (rgb or rgb_u8 required)");
     AEAJ_REQUIRE(p->qtab_dev, "aeaj_encode: quantisation tables not set (aeaj_plan_set_qtables)");
@@ -736,8 +749,7 @@ static int encode_impl(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, 
         p->mark("canny_nms");
         launches += 2;
     }
-    const bool tree_all = (phases & (1u << AEAJ_PHASE_TREE)) != 0;
-    if (tree_all || (phases & (1u << AEAJ_PHASE_HYST))) {
+    if (phases & (1u << AEAJ_PHASE_HYST)) {
         rc = launch_hysteresis(h, p->planes_dev, p->planes.data(), NP, p->ntiles, p->ring_cap, A.flags, A.ring, A.ctrl, io->status, st); if (rc) return rc;
         p->mark("hysteresis");
         launches += 1;
@@ -752,7 +764,7 @@ static int encode_impl(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, 
                                           cudaMemcpyDeviceToDevice, st));
     }
     // quadtree: per-top-block counts (band), scan over all top blocks (needs every band's counts), emit (band)
-    const int qt_parts = (tree_all ? 7 : 0) | ((phases & (1u << AEAJ_PHASE_QT_COUNT)) ? 1 : 0) | ((phases & (1u << AEAJ_PHASE_QT_EMIT)) ? 6 : 0);
+    const int qt_parts = ((phases & (1u << AEAJ_PHASE_QT_COUNT)) ? 1 : 0) | ((phases & (1u << AEAJ_PHASE_QT_EMIT)) ? 6 : 0);
     if (qt_parts) {
         rc = launch_quadtree(p->planes_dev, p->planes.data(), NP, p->info.block_min, p->info.block_max, A.class_lists, A.class_counts,
                              p->class_off_dev, st, &launches, qt_parts);
@@ -774,11 +786,7 @@ static int encode_impl(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, 
 }
 
 extern "C" int aeaj_encode(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, void* stream) {
-    return encode_impl(p, io, workspace, ST(stream), 0x3fu, 0, -1);
-}
-extern "C" int aeaj_encode_phase(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, void* stream, int phase, int band0, int band1) {
-    AEAJ_REQUIRE(phase >= AEAJ_PHASE_COLOR && phase <= AEAJ_PHASE_QT_EMIT, "aeaj_encode_phase: bad phase");
-    return encode_impl(p, io, workspace, ST(stream), 1u << phase, band0, band1);
+    return encode_impl(p, io, workspace, ST(stream), (1u << (AEAJ_PHASE_DCT + 1)) - 1, 0, -1);      // every phase, whole image
 }
 
 static int decode_impl(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, cudaStream_t st, unsigned phases, int band0, int band1) {
@@ -832,10 +840,6 @@ static int decode_impl(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, 
 }
 extern "C" int aeaj_decode(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream) {
     return decode_impl(p, io, workspace, ST(stream), 0x3u, 0, -1);
-}
-extern "C" int aeaj_decode_phase(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream, int phase, int band0, int band1) {
-    AEAJ_REQUIRE(phase >= AEAJ_DPHASE_IDCT && phase <= AEAJ_DPHASE_COLOR, "aeaj_decode_phase: bad phase");
-    return decode_impl(p, io, workspace, ST(stream), 1u << phase, band0, band1);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -960,24 +964,23 @@ extern "C" int aeaj_plan_set_peers(aeaj_plan* p, int rank, int world, void* cons
     return 0;
 }
 
+// band b of n: full-resolution rows [b*H/n, (b+1)*H/n) (H is a multiple of n, run_halo checks it)
+static int band_row(const aeaj_plan* p, int b, int n) { return p->info.height / n * b; }
+
 // all ranks meet: everything the ranks enqueued before the barrier is complete and visible before anything enqueued after it runs
-extern "C" int aeaj_plan_peer_barrier(aeaj_plan* p, void* stream) {
-    AEAJ_REQUIRE(p, "aeaj_plan_peer_barrier: NULL plan");
+static int peer_barrier(aeaj_plan* p, cudaStream_t st) {
     if (p->peers.world <= 1) return 0;
     p->peer_epoch++;
-    return launch_peer_barrier(p->peer_flags, p->peers.rank, p->peers.world, p->peer_epoch, p->h->tc_err_dev, ST(stream));
+    return launch_peer_barrier(p->peer_flags, p->peers.rank, p->peers.world, p->peer_epoch, p->h->tc_err_dev, st);
 }
 
 // copy the other ranks' rows into this rank's buffers.  what = 0: the strong / weak candidate bitmaps (before the replicated
-// hysteresis); what = 1: the per-top-block quadtree totals (before the scan).  Bands are the equal split used by aeaj/tiled.py.
-extern "C" int aeaj_plan_peer_gather(aeaj_plan* p, int what, void* workspace, void* stream) {
-    AEAJ_REQUIRE(p && workspace && (what == 0 || what == 1), "aeaj_plan_peer_gather: bad arguments");
+// hysteresis); what = 1: the per-top-block quadtree totals (before the scan).  Rank r owns band r of world.
+static int peer_gather(aeaj_plan* p, int what, void* workspace, cudaStream_t st) {
     const int world = p->peers.world, rank = p->peers.rank;
     if (world <= 1) return 0;
-    AEAJ_REQUIRE(workspace == p->peer_ws[rank], "aeaj_plan_peer_gather: the workspace must be the shared allocation registered with aeaj_plan_set_peers");
     plan_carve(p, workspace);
     const int H = p->info.height;
-    AEAJ_REQUIRE(H % world == 0, "halo-split bands: the height must be a multiple of the number of ranks");
     std::vector<PeerSeg> segs;
     long long maxb = 0;
     auto add = [&](const void* mine, long long off, long long bytes, int r) {
@@ -988,7 +991,7 @@ extern "C" int aeaj_plan_peer_gather(aeaj_plan* p, int what, void* workspace, vo
     };
     for (int r = 0; r < world; r++) {
         if (r == rank) continue;
-        const int b0 = (H / world) * r, b1 = (H / world) * (r + 1);
+        const int b0 = band_row(p, r, world), b1 = band_row(p, r + 1, world);
         for (int l = 0; l < 3; l++) {
             const PlaneDesc& P = p->planes[l];
             const int rh = H / P.h;
@@ -1005,53 +1008,55 @@ extern "C" int aeaj_plan_peer_gather(aeaj_plan* p, int what, void* workspace, vo
     }
     AEAJ_REQUIRE(segs.size() <= 64, "too many gather segments");
     PeerSeg* dev = p->peer_segs_dev + (what ? 64 : 0);
-    AEAJ_CUDA(cudaMemcpyAsync(dev, segs.data(), sizeof(PeerSeg) * segs.size(), cudaMemcpyHostToDevice, ST(stream)));
-    return launch_peer_gather(dev, (int)segs.size(), maxb, ST(stream));
+    AEAJ_CUDA(cudaMemcpyAsync(dev, segs.data(), sizeof(PeerSeg) * segs.size(), cudaMemcpyHostToDevice, st));
+    return launch_peer_gather(dev, (int)segs.size(), maxb, st);
 }
 
-// The whole schedule of one rank of a multi-GPU halo-split in ONE call (aeaj/tiled.py documents it; the phase-wise entry
-// points stay for callers that bring their own exchange): ~45 launches behind a single foreign call instead of twenty.
-extern "C" int aeaj_encode_halo(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, void* stream, int band0, int band1) {
-    AEAJ_REQUIRE(p && p->peers.world > 1, "aeaj_encode_halo: the plan has no peers (aeaj_plan_set_peers)");
-    AEAJ_REQUIRE(workspace == p->peer_ws[p->peers.rank], "aeaj_encode_halo: the workspace must be the shared allocation registered with aeaj_plan_set_peers");
-    const cudaStream_t st = ST(stream);
-    auto ph = [](int k) { return 1u << k; };
-    int rc;
-    if ((rc = aeaj_plan_peer_barrier(p, stream))) return rc;          // the previous call's neighbours are done reading this rank's planes
-    if ((rc = encode_impl(p, io, workspace, st, ph(AEAJ_PHASE_COLOR) | ph(AEAJ_PHASE_CLAHE_HIST), band0, band1))) return rc;
-    if ((rc = aeaj_plan_peer_barrier(p, stream))) return rc;
-    if ((rc = encode_impl(p, io, workspace, st, ph(AEAJ_PHASE_PREFILTER), band0, band1))) return rc;
-    if ((rc = aeaj_plan_peer_barrier(p, stream))) return rc;
-    if ((rc = encode_impl(p, io, workspace, st, ph(AEAJ_PHASE_NMS), band0, band1))) return rc;
-    if ((rc = aeaj_plan_peer_barrier(p, stream))) return rc;
-    if ((rc = aeaj_plan_peer_gather(p, 0, workspace, stream))) return rc;
-    if ((rc = encode_impl(p, io, workspace, st, ph(AEAJ_PHASE_HYST) | ph(AEAJ_PHASE_QT_COUNT), band0, band1))) return rc;
-    if ((rc = aeaj_plan_peer_barrier(p, stream))) return rc;
-    if ((rc = aeaj_plan_peer_gather(p, 1, workspace, stream))) return rc;
-    return encode_impl(p, io, workspace, st, ph(AEAJ_PHASE_QT_EMIT) | ph(AEAJ_PHASE_DCT), band0, band1);
-}
-extern "C" int aeaj_decode_halo(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream, int band0, int band1) {
-    AEAJ_REQUIRE(p && p->peers.world > 1, "aeaj_decode_halo: the plan has no peers (aeaj_plan_set_peers)");
-    AEAJ_REQUIRE(workspace == p->peer_ws[p->peers.rank], "aeaj_decode_halo: the workspace must be the shared allocation registered with aeaj_plan_set_peers");
-    int rc;
-    if ((rc = decode_impl(p, io, workspace, ST(stream), 1u << AEAJ_DPHASE_IDCT, band0, band1))) return rc;
-    if ((rc = aeaj_plan_peer_barrier(p, stream))) return rc;
-    return decode_impl(p, io, workspace, ST(stream), 1u << AEAJ_DPHASE_COLOR, band0, band1);
-}
+// The halo-split schedule, written once.  A step is a barrier of all ranks, a gather, or one phase.  A phase step runs once for
+// every band the call covers, in band order: phase-major, because COLOR clears the histogram accumulators that every band's
+// CLAHE_HIST adds to.  Hysteresis covers the whole image and runs once.
+enum HaloStepKind { STEP_BARRIER, STEP_GATHER, STEP_PHASE, STEP_PHASE_ONCE };
+struct HaloStep { HaloStepKind kind; int arg; };
+static const HaloStep ENCODE_HALO[] = {
+    {STEP_BARRIER, 0},                                    // the previous call's neighbours are done reading this rank's planes
+    {STEP_PHASE, AEAJ_PHASE_COLOR}, {STEP_PHASE, AEAJ_PHASE_CLAHE_HIST}, {STEP_BARRIER, 0},
+    {STEP_PHASE, AEAJ_PHASE_PREFILTER}, {STEP_BARRIER, 0},
+    {STEP_PHASE, AEAJ_PHASE_NMS}, {STEP_BARRIER, 0},
+    {STEP_GATHER, 0}, {STEP_PHASE_ONCE, AEAJ_PHASE_HYST}, {STEP_PHASE, AEAJ_PHASE_QT_COUNT}, {STEP_BARRIER, 0},
+    {STEP_GATHER, 1}, {STEP_PHASE, AEAJ_PHASE_QT_EMIT}, {STEP_PHASE, AEAJ_PHASE_DCT}};
+static const HaloStep DECODE_HALO[] = {{STEP_PHASE, AEAJ_DPHASE_IDCT}, {STEP_BARRIER, 0}, {STEP_PHASE, AEAJ_DPHASE_COLOR}};
 
-// device pointers of the planes a halo-split caller exchanges between phases (batch 1)
-extern "C" int aeaj_plan_buffers(aeaj_plan* p, void* workspace, aeaj_plan_buffers_t* out) {
-    AEAJ_REQUIRE(p && workspace && out, "aeaj_plan_buffers: bad arguments");
-    plan_carve(p, workspace);
-    memset(out, 0, sizeof *out);
-    for (int l = 0; l < 3; l++) {
-        const PlaneDesc& P = p->planes[l];
-        out->layer[l] = P.layer_f32; out->u8a[l] = P.u8a; out->u8b[l] = P.u8b; out->strong[l] = P.strong; out->weak[l] = P.weak;
-        out->h[l] = P.h; out->w[l] = P.w; out->wpr[l] = P.wpr;
+// Walks `steps` for the bands this call covers: on a plan with peers this rank's band (bands == world), without peers every band
+// in turn on this GPU (barriers and gathers do nothing there).  run(phases, band0, band1) is encode_impl / decode_impl.
+template <size_t N, class Run>
+static int run_halo(aeaj_plan* p, const HaloStep (&steps)[N], int bands, void* workspace, cudaStream_t st, Run run) {
+    AEAJ_REQUIRE(p && bands >= 1 && p->info.height % bands == 0, "halo-split: the image height must be a multiple of bands >= 1");
+    int first = 0, last = bands;
+    if (p->peers.world > 1) {
+        AEAJ_REQUIRE(bands == p->peers.world, "halo-split: a plan with peers runs one band per rank (bands == world)");
+        AEAJ_REQUIRE(workspace == p->peer_ws[p->peers.rank], "halo-split: the workspace must be the shared allocation registered with aeaj_plan_set_peers");
+        first = p->peers.rank; last = first + 1;
     }
-    out->clahe_hist = p->planes[0].clahe_hist; out->clahe_hist_bytes = (int64_t)p->nplanes * 16 * 256 * 4;
-    out->hist = p->planes[0].hist; out->hist_bytes = (int64_t)p->nplanes * 256 * 4;
+    for (const HaloStep& s : steps) {
+        int rc = 0;
+        if (s.kind == STEP_BARRIER) rc = peer_barrier(p, st);
+        else if (s.kind == STEP_GATHER) rc = peer_gather(p, s.arg, workspace, st);
+        else
+            for (int b = first; b < (s.kind == STEP_PHASE_ONCE ? first + 1 : last) && !rc; b++)
+                rc = run(1u << s.arg, band_row(p, b, bands), band_row(p, b + 1, bands));
+        if (rc) return rc;
+    }
     return 0;
+}
+extern "C" int aeaj_encode_halo(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, void* stream, int bands) {
+    const cudaStream_t st = ST(stream);
+    return run_halo(p, ENCODE_HALO, bands, workspace, st,
+                    [&](unsigned ph, int b0, int b1) { return encode_impl(p, io, workspace, st, ph, b0, b1); });
+}
+extern "C" int aeaj_decode_halo(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream, int bands) {
+    const cudaStream_t st = ST(stream);
+    return run_halo(p, DECODE_HALO, bands, workspace, st,
+                    [&](unsigned ph, int b0, int b1) { return decode_impl(p, io, workspace, st, ph, b0, b1); });
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define AEAJ_VERSION 2
+#define AEAJ_VERSION 3
 
 #if defined(__GNUC__)
 #define AEAJ_API __attribute__((visibility("default")))
@@ -181,58 +181,33 @@ AEAJ_API int aeaj_encode(aeaj_plan* p, const aeaj_encode_io* io, void* workspace
 AEAJ_API int aeaj_decode(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
- * halo-split of ONE large image over several GPUs (SURVEY 8e, config C4): the same pipeline, one phase
- * per call, restricted to the band [band0, band1) of full-resolution rows this rank owns (batch 1; band
- * boundaries multiples of 256 rows, or the image end).  Between phases the caller exchanges the small
- * planes over NVLink (NCCL): u8 planes and bitmaps are all-gathered, the CLAHE / percentile histograms
- * all-reduced; hysteresis and the quadtree then run replicated on every rank, colour and DCT stay sharded.
- * aeaj_encode == all six phases on the full image.  Sequence and collectives: aeaj/tiled.py.
- * ------------------------------------------------------------------------------------------- */
-enum { AEAJ_PHASE_COLOR = 0,      /* clears accumulators; colour + subsample + u8 cast of the band            */
-       AEAJ_PHASE_CLAHE_HIST = 1, /* CLAHE tile histograms of the band            -> all-reduce clahe_hist    */
-       AEAJ_PHASE_PREFILTER = 2,  /* needs all-gathered u8a; LUTs + CLAHE/Gauss/bilateral of the band         */
-       AEAJ_PHASE_NMS = 3,        /* needs all-gathered u8b, all-reduced hist; thresholds + NMS of the band   */
-       AEAJ_PHASE_TREE = 4,       /* needs all-gathered strong/weak; hysteresis + quadtree, whole image       */
-       AEAJ_PHASE_DCT = 5,        /* DCT + quantise of the band's leaves (coefficients at global offsets)     */
-       /* AEAJ_PHASE_TREE in three steps, for ranks that shard the quadtree as well:                           */
-       AEAJ_PHASE_HYST = 6,       /* hysteresis, whole image (needs every band's strong / weak rows)          */
-       AEAJ_PHASE_QT_COUNT = 7,   /* quadtree: node counts of the band's top blocks                           */
-       AEAJ_PHASE_QT_EMIT = 8 };  /* needs every band's counts; scan + states / leaves / work lists of the band */
-enum { AEAJ_DPHASE_IDCT = 0,      /* dequantise + IDCT + merge of the band's leaves                           */
-       AEAJ_DPHASE_COLOR = 1 };   /* needs the neighbouring chroma rows; upsample + inverse colour of the band */
-typedef struct {
-    void* layer[3]; void* u8a[3]; void* u8b[3]; void* strong[3]; void* weak[3];
-    int h[3], w[3], wpr[3];
-    void* clahe_hist; int64_t clahe_hist_bytes;
-    void* hist; int64_t hist_bytes;
-} aeaj_plan_buffers_t;
-AEAJ_API int aeaj_encode_phase(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, void* stream, int phase, int band0, int band1);
-AEAJ_API int aeaj_decode_phase(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream, int phase, int band0, int band1);
-AEAJ_API int aeaj_plan_buffers(aeaj_plan* p, void* workspace, aeaj_plan_buffers_t* out);
-
-/* The same split WITHOUT collectives on the data path: the ranks (one process per GPU of one node) share their plan
- * workspaces through CUDA IPC and the kernels read the few rows they need from the neighbour GPU directly over NVLink.
+ * halo-split of ONE large image over several GPUs of one node (SURVEY 8e, config C4) into `bands` row bands: band b is the
+ * full-resolution rows [b*H/bands, (b+1)*H/bands).  H must be a multiple of `bands`; with more than one band the plan holds
+ * one image and every band boundary is a multiple of max(128, block_max) rows in every layer, so that no leaf, filter tile
+ * or chroma cell straddles two bands.
+ * One process per GPU; the ranks share their plan workspaces through CUDA IPC and the kernels read the few rows they need
+ * from the neighbour GPU directly over NVLink -- no collective library on the data path.
  *   aeaj_peer_alloc / aeaj_peer_export: allocate the workspace (and a 64-byte-per-rank flag array) as exportable device
  *   memory and produce its 64-byte IPC handle; aeaj_peer_open / aeaj_peer_close: map / unmap another rank's allocation.
  *   aeaj_plan_set_peers: rank, world (<= 8) and, per rank, the address of its workspace and of its flag array as mapped in
- *   THIS process (own entries: the local allocations).  Afterwards aeaj_encode_phase / aeaj_decode_phase with a band read
- *   the halo rows outside the band from the neighbour's workspace, and the CLAHE / percentile kernels sum the per-rank
- *   partial histograms.  aeaj_plan_peer_barrier: a device-side barrier of all ranks on `stream` (one small kernel; it
- *   orders the ranks' earlier work before their later reads).  aeaj_plan_peer_gather: copies the other ranks' rows of the
- *   strong / weak bitmaps (what = 0) or of the quadtree block totals (what = 1) into this rank's workspace.
- * Sequence: aeaj/tiled.py.  Every rank must issue the same sequence of barriers. */
+ *   THIS process (own entries: the local allocations).
+ *   aeaj_encode_halo / aeaj_decode_halo: one rank's whole schedule in one call, on `stream`.  With peers (world > 1) `bands`
+ *   must equal world, `workspace` must be the shared allocation, and the call runs band `rank`: the CLAHE / percentile kernels
+ *   sum the per-rank partial histograms, the stencil kernels read the halo rows outside the band from the neighbours'
+ *   workspaces, device-side barriers order each rank's writes before the others' reads, and two gathers copy the other bands'
+ *   rows of the strong / weak bitmaps (hysteresis runs on the whole image on every rank) and of the quadtree block totals.
+ *   Every rank ends with its band's leaves / states / coefficients at their global positions of the streams.  Without peers
+ *   the call runs every band in turn on this GPU, through the same schedule, and ends with the whole image's result.
+ * Every rank of a split must make the same sequence of calls (each one issues the same barriers).
+ * ------------------------------------------------------------------------------------------- */
 AEAJ_API int aeaj_peer_alloc(size_t bytes, void** ptr);
 AEAJ_API int aeaj_peer_free(void* ptr);
 AEAJ_API int aeaj_peer_export(void* ptr, void* handle64_host);
 AEAJ_API int aeaj_peer_open(const void* handle64_host, void** ptr);
 AEAJ_API int aeaj_peer_close(void* ptr);
 AEAJ_API int aeaj_plan_set_peers(aeaj_plan* p, int rank, int world, void* const* peer_workspaces_host, void* const* peer_flags_host);
-AEAJ_API int aeaj_plan_peer_barrier(aeaj_plan* p, void* stream);
-AEAJ_API int aeaj_plan_peer_gather(aeaj_plan* p, int what, void* workspace, void* stream);
-/* One rank's whole halo-split schedule in a single call: barriers, the band-restricted phases (reading halo rows / partial
- * histograms from the neighbours), the two gathers -- what aeaj/tiled.py otherwise issues as twenty calls. */
-AEAJ_API int aeaj_encode_halo(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, void* stream, int band0, int band1);
-AEAJ_API int aeaj_decode_halo(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream, int band0, int band1);
+AEAJ_API int aeaj_encode_halo(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, void* stream, int bands);
+AEAJ_API int aeaj_decode_halo(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream, int bands);
 
 /* ---------------------------------------------------------------------------------------------
  * host-side helpers for the entropy-coding side (plain CPU code, no device work):

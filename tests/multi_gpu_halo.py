@@ -3,8 +3,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 tests/multi_gpu_halo.py
 
 Every rank encodes/decodes only its band of ONE image, reading halo rows and partial histograms from its neighbours'
-shared workspaces over NVLink (aeaj/tiled.py; `--nccl` selects the round-1 NCCL exchange instead) and compares the
-result with the fused single-GPU path computed locally."""
+shared workspaces over NVLink (aeaj/tiled.py) and compares the result with the fused single-GPU path computed locally."""
 import json
 import os
 import sys
@@ -29,7 +28,6 @@ def main():
     torch.cuda.set_device(local)
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     args = [a for a in sys.argv[1:] if not a.startswith("--")]
-    transport = "nccl" if "--nccl" in sys.argv else "peer"
     H, W = (int(a) for a in (args[:2] if len(args) >= 2 else (2048, 2048)))
     q, b = (30, 95), (4, 128)
     codec = get_codec(local)
@@ -42,7 +40,7 @@ def main():
         ref_dec = codec.decode(eg.coef, eg.leaves, eg.counts, 1, H, W, space, q, b, instance=4000)[0].clone()
         lo, hi = band_of(rank, world, H)
         band = full[lo:hi].contiguous()
-        t = TiledCodec(codec, rank, world, transport=transport)
+        t = TiledCodec(codec, rank, world)
         enc = t.encode(band, H, W, space, q, b, exchange_coef=True)          # parity: the whole stream on every rank
         got = codec.download(enc)[0]
         ok = all(np.array_equal(got[l][k], ref[l][k]) for l in range(3) for k in ("states", "leaves", "coef"))
@@ -76,7 +74,7 @@ def main():
         out[space] = {"identical_to_single_gpu": bool(flag.item()), "ms_halo_split": float(ms.item()), "ms_single_gpu": e0.elapsed_time(e1) / 5,
                       "mp_per_s_halo_split": H * W / 1e6 / (float(ms.item()) / 1e3)}
     if rank == 0:
-        print(json.dumps({"halo_split": {"gpus": world, "transport": transport, "image": [H, W], "results": out}}))
+        print(json.dumps({"halo_split": {"gpus": world, "image": [H, W], "results": out}}))
     dist.destroy_process_group()
     if not all(v["identical_to_single_gpu"] for v in out.values()):
         sys.exit(1)

@@ -19,7 +19,7 @@ def test_library_exports_every_declared_symbol():
     for name in declared:
         assert hasattr(lib, name), f"{name} declared in include/aeaj.h but not exported"
     assert sorted(native.EXPORTS) == declared
-    assert lib.aeaj_version() == 2
+    assert lib.aeaj_version() == 3
 
 
 def test_no_cpu_fallback_without_cuda():

@@ -1,5 +1,5 @@
 """for compute-sanitizer: small encode / decode runs through every kernel family (all size classes incl. the tcgen05 ones, stream
-layout, packing, segment copies, the host pipeline, the band-restricted phases, a PQ space).
+layout, packing, segment copies, the host pipeline, the halo-split schedule over emulated bands, a PQ space).
     compute-sanitizer --tool memcheck python tools/sanitize_small.py"""
 import sys, torch, numpy as np
 sys.path.insert(0, 'adaptive-edge-aware-jpeg_b200'); sys.path.insert(0, 'tests')
