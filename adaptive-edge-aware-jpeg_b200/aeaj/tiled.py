@@ -156,6 +156,10 @@ class TiledCodec:
         if multi and exchange_coef:
             for l in range(3):
                 o.coef[l].zero_(); o.leaves[l].zero_(); o.states[l].zero_()
+        # the plan is shared with DeviceCodec.encode for B = 1: set what it may have left behind (stream layout, tensor mask)
+        native.check(self.lib.aeaj_plan_set_stream_layout(p.ptr, 0), "aeaj_plan_set_stream_layout")
+        native.check(self.lib.aeaj_plan_set_tensor_dct(p.ptr, c._tensor_mask()), "aeaj_plan_set_tensor_dct")
+        o.zigzag = False
         native.check(self.lib.aeaj_encode_halo(p.ptr, C.byref(io), ws, _stream(), G), "aeaj_encode_halo")
         if multi and exchange_coef:
             import torch.distributed as dist
@@ -178,5 +182,7 @@ class TiledCodec:
         io.counts, io.rgb = enc.counts.data_ptr(), p.rgb_out.data_ptr()
         ws = self._ws(p)
         G, _ = self._band(H, brange)
+        native.check(self.lib.aeaj_plan_set_stream_layout(p.ptr, int(enc.zigzag)), "aeaj_plan_set_stream_layout")
+        native.check(self.lib.aeaj_plan_set_tensor_dct(p.ptr, c._tensor_mask()), "aeaj_plan_set_tensor_dct")
         native.check(self.lib.aeaj_decode_halo(p.ptr, C.byref(io), ws, _stream(), G), "aeaj_decode_halo")
         return p.rgb_out[0]
