@@ -57,6 +57,15 @@ class PackedBatch:
 
 
 @dataclass
+class DeflatedBatch:
+    """Device deflate of one batch's coefficient streams (include/aeaj.h, aeaj_deflate_coefficients): per plane one complete
+    zlib stream, readable by any inflate -- what travels over PCIe to the .ajpg writer instead of the int32 streams."""
+    out: List[torch.Tensor]        # 3 x uint8 [B, cap_out_l]
+    lengths: torch.Tensor          # int32 [B, 3]  bytes of each stream
+    status: torch.Tensor           # int32 [4]     [0] planes whose stream did not fit (0 = ok)
+
+
+@dataclass
 class _Plan:
     ptr: C.c_void_p
     info: native.PlanInfo
@@ -68,6 +77,8 @@ class _Plan:
     keep: list = field(default_factory=list)
     dec_status: Optional[torch.Tensor] = None     # int32 [64]: [2] tensor-IDCT timeout flag, [3] leaves rejected by the device guard
     packed: Optional[PackedBatch] = None
+    deflated: Optional[DeflatedBatch] = None
+    deflate_scratch: Optional[torch.Tensor] = None
     nbytes: int = 0
 
 
@@ -273,6 +284,58 @@ class DeviceCodec:
         native.check(self.lib.aeaj_pack_coefficients(p.ptr, coef, enc.counts.data_ptr(), C.byref(io), p.workspace.data_ptr(), _stream()),
                      "aeaj_pack_coefficients")
         return pk
+
+    def _deflated(self, p: _Plan) -> DeflatedBatch:
+        if p.deflated is None:
+            B, dev = p.info.batch, p.rgb_out.device
+            cap = (C.c_int64 * 3)()
+            scratch = C.c_int64()
+            native.check(self.lib.aeaj_deflate_caps(p.ptr, cap, C.byref(scratch)), "aeaj_deflate_caps")
+            p.deflated = DeflatedBatch(out=[torch.empty((B, int(cap[l])), dtype=torch.uint8, device=dev) for l in range(3)],
+                                       lengths=torch.zeros((B, 3), dtype=torch.int32, device=dev),
+                                       status=torch.zeros(4, dtype=torch.int32, device=dev))
+            p.deflate_scratch = torch.empty(int(scratch.value), dtype=torch.uint8, device=dev)
+            p.nbytes += sum(t.numel() for t in p.deflated.out) + p.deflate_scratch.numel()
+            self._evict(keep=next(k for k, v in self._plans.items() if v is p))
+        return p.deflated
+
+    def deflate(self, enc: EncodedBatch, space, qrange, brange, instance: int = 0) -> DeflatedBatch:
+        """One zlib stream per plane of enc.coef, on the device (aeaj_deflate_coefficients): the entropy coder of the .ajpg
+        container without the int32 streams crossing PCIe.  With encode(stream=True) the payloads are exactly the streams the
+        host path hands to zlib.  Asynchronous; the buffers belong to the plan and are reused by the next call."""
+        B, H, W = enc.shape
+        p = self._plan(B, H, W, space, brange, qrange, instance)
+        df = self._deflated(p)
+        io = native.DeflateIO()
+        for l in range(3):
+            io.out[l] = df.out[l].data_ptr()
+        io.lengths = df.lengths.data_ptr()
+        io.status = df.status.data_ptr()
+        coef = (C.c_void_p * 3)(*[enc.coef[l].data_ptr() for l in range(3)])
+        native.check(self.lib.aeaj_deflate_coefficients(p.ptr, coef, enc.counts.data_ptr(), C.byref(io), p.deflate_scratch.data_ptr(),
+                                                         _stream()), "aeaj_deflate_coefficients")
+        return df
+
+    def download_deflated(self, enc: EncodedBatch, df: DeflatedBatch):
+        """D2H of what the .ajpg writer needs after deflate() of an encode(stream=True) batch: per image a list of 3
+        dicts(zlib, packed_states, n_states, root) -- the used zlib bytes, the packed state streams and the counts; the
+        coefficients stay on the device.  Synchronises the stream."""
+        if not enc.zigzag or enc.packed_states is None:
+            raise ValueError("download_deflated needs the .ajpg stream layout: encode(..., stream=True)")
+        counts = enc.counts.cpu().numpy()
+        lengths = df.lengths.cpu().numpy()
+        self.check_status(enc.status, "encode")
+        if int(df.status[0].item()) != 0:
+            raise native.AeajError("a deflated coefficient stream did not fit its buffer")
+        out = []
+        for b in range(enc.shape[0]):
+            layers = []
+            for l in range(3):
+                ns, root = int(counts[b, l, 1]), int(counts[b, l, 3])
+                layers.append(dict(zlib=df.out[l][b, :int(lengths[b, l])].cpu().numpy().tobytes(),
+                                   packed_states=enc.packed_states[l][b, :(ns + 3) // 4].cpu().numpy(), n_states=ns, root=root))
+            out.append(layers)
+        return out
 
     def unpack(self, pk: PackedBatch, B, H, W, space, qrange, brange, instance: int = 0) -> List[torch.Tensor]:
         """Inverse of pack(): expands into the plan's int32 coefficient buffers (returned); asynchronous."""

@@ -27,6 +27,7 @@ EXPORTS = [
     "aeaj_peer_alloc", "aeaj_peer_free", "aeaj_peer_export", "aeaj_peer_open", "aeaj_peer_close",
     "aeaj_plan_set_peers", "aeaj_copy_segments",
     "aeaj_encode_halo", "aeaj_decode_halo", "aeaj_set_fast_transfer",
+    "aeaj_deflate_caps", "aeaj_deflate_coefficients",
 ]
 
 
@@ -55,6 +56,10 @@ class DecodeIO(C.Structure):
 
 class PackedIO(C.Structure):
     _fields_ = [("mask", C.c_void_p * 3), ("vals", C.c_void_p * 3), ("counts", C.c_void_p)]
+
+
+class DeflateIO(C.Structure):
+    _fields_ = [("out", C.c_void_p * 3), ("lengths", C.c_void_p), ("status", C.c_void_p)]
 
 
 class Segment(C.Structure):
@@ -129,6 +134,8 @@ def load():
         lib.aeaj_unpack_coefficients.argtypes = [vp, C.POINTER(PackedIO), C.POINTER(vp), vp, vp]
         lib.aeaj_pack_coefficients_host.argtypes = [vp, C.c_int64, vp, vp, C.POINTER(C.c_int64), C.POINTER(i)]
         lib.aeaj_unpack_coefficients_host.argtypes = [vp, vp, C.c_int64, C.c_int64, vp]
+        lib.aeaj_deflate_caps.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+        lib.aeaj_deflate_coefficients.argtypes = [vp, C.POINTER(vp), vp, C.POINTER(DeflateIO), vp, vp]
         _lib = lib
         return lib
 

@@ -237,6 +237,25 @@ struct PackPlane {
 size_t aeaj_pack_scratch_ints(int64_t cap_coef);
 int launch_pack(const PackPlane* planes_host, PackPlane* planes_dev, int nplanes, int64_t max_cap_coef, int unpack, cudaStream_t st);
 
+// one plane's zlib stream (deflate.cu, deflate_core.h)
+struct DeflatePlane {
+    const uint8_t* in;        // the plane's int32 coefficient stream, as bytes
+    const int32_t* n_coef;    // device: number of coefficients of this plane
+    int64_t cap_coef;         // capacity of the coefficient buffer
+    uint8_t* out;             // [cap_out]: the zlib stream
+    int64_t cap_out;
+    int32_t* length;          // device: bytes of `out` written (0 if the stream did not fit)
+    int32_t* status;          // optional device counter of planes whose stream did not fit
+    uint8_t* slots;           // scratch [chunks][DF_CHUNK_BOUND]: each chunk's deflate output
+    uint16_t* tok;            // scratch [chunks][DF_CHUNK]: each chunk's tokens
+    int32_t* chunk_len;       // scratch [chunks]
+    uint32_t* chunk_adler;    // scratch [chunks]
+    int64_t* chunk_off;       // scratch [chunks]
+};
+size_t deflate_chunk_scratch_bytes();
+int aeaj_deflate_init();
+int launch_deflate(const DeflatePlane* planes_host, DeflatePlane* planes_dev, int nplanes, int max_chunks, cudaStream_t st);
+
 // kernels' host launchers (defined in the .cu files)
 int aeaj_canny_init(aeaj_handle* h);
 int aeaj_dct_init(aeaj_handle* h);

@@ -6,6 +6,7 @@
 #include <string>
 #include <vector>
 #include "aeaj_internal.cuh"
+#include "deflate_core.h"
 
 // ---------------------------------------------------------------------------------------------
 // errors
@@ -117,6 +118,8 @@ extern "C" int aeaj_create(int device, aeaj_handle** out) {
     rc = aeaj_dct_tc_init(h);
     if (rc) { free(h); return rc; }
     rc = aeaj_color_init(h);
+    if (rc) { free(h); return rc; }
+    rc = aeaj_deflate_init();
     if (rc) { free(h); return rc; }
     AEAJ_CUDA(cudaMalloc(&h->srgb_lut_dev, 256 * sizeof(float)));
     AEAJ_CUDA(cudaMalloc(&h->stage_plane_dev, sizeof(PlaneDesc)));
@@ -397,6 +400,9 @@ struct aeaj_plan {
     PackPlane* pack_planes_dev;          // [2][nplanes]: the pack and the unpack flavour of the table (they differ in n_coef)
     std::vector<PackPlane> pack_pushed[2];   // what the device tables hold (upload skipped when unchanged: no per-call pageable copy,
     cudaStream_t pack_pushed_stream[2] = {nullptr, nullptr};   // which may synchronise the stream and is not capturable)
+    std::vector<DeflatePlane> df_planes, df_pushed;   // deflate descriptors, the same scheme
+    DeflatePlane* df_planes_dev = nullptr;
+    cudaStream_t df_pushed_stream = nullptr;
     // one image over several GPUs (peer.cu): the other ranks' workspaces / barrier flags, opened through CUDA IPC by the caller
     PeerSet peers = {1, 0, {0}};
     void* peer_ws[AEAJ_MAX_PEERS] = {nullptr};
@@ -538,7 +544,7 @@ extern "C" int aeaj_plan_create(aeaj_handle* h, int batch, int height, int width
 extern "C" int aeaj_plan_destroy(aeaj_plan* p) {
     if (!p) return 0;
     cudaSetDevice(p->h->device);
-    cudaFree(p->planes_dev); cudaFree(p->class_off_dev); cudaFree(p->outs_dev); cudaFree(p->qtab_dev); cudaFree(p->qtabf_dev); cudaFree(p->pack_planes_dev); cudaFree(p->peer_segs_dev);
+    cudaFree(p->planes_dev); cudaFree(p->class_off_dev); cudaFree(p->outs_dev); cudaFree(p->qtab_dev); cudaFree(p->qtabf_dev); cudaFree(p->pack_planes_dev); cudaFree(p->peer_segs_dev); cudaFree(p->df_planes_dev);
     delete p;
     return 0;
 }
@@ -883,6 +889,60 @@ extern "C" int aeaj_pack_coefficients(aeaj_plan* p, const int32_t* const* coef3,
 extern "C" int aeaj_unpack_coefficients(aeaj_plan* p, const aeaj_packed_io* in, int32_t* const* coef3, void* workspace, void* stream) {
     return pack_impl(p, coef3, nullptr, in, workspace, ST(stream), 1);
 }
+// ---------------------------------------------------------------------------------------------
+// device deflate of the coefficient streams (deflate.cu)
+// ---------------------------------------------------------------------------------------------
+static int64_t deflate_chunks_cap(const aeaj_plan* p, int l) { return df_chunks(4 * p->info.cap_coef[l]); }
+static int64_t deflate_cap_out(const aeaj_plan* p, int l) { return (df_stream_bound(4 * p->info.cap_coef[l]) + 15) & ~(int64_t)15; }
+
+extern "C" int aeaj_deflate_caps(const aeaj_plan* p, int64_t* cap_out3, int64_t* scratch_bytes) {
+    AEAJ_REQUIRE(p && cap_out3 && scratch_bytes, "aeaj_deflate_caps: bad arguments");
+    int64_t s = 0;
+    for (int l = 0; l < 3; l++) {
+        cap_out3[l] = deflate_cap_out(p, l);
+        s += p->info.batch * deflate_chunks_cap(p, l) * (int64_t)deflate_chunk_scratch_bytes();
+    }
+    *scratch_bytes = s + 256;
+    return 0;
+}
+
+extern "C" int aeaj_deflate_coefficients(aeaj_plan* p, const int32_t* const* coef3, const int32_t* counts, const aeaj_deflate_io* io,
+                                         void* scratch, void* stream) {
+    AEAJ_REQUIRE(p && coef3 && counts && io && io->lengths && scratch, "aeaj_deflate_coefficients: bad arguments");
+    const cudaStream_t st = ST(stream);
+    const int B = p->info.batch;
+    if (!p->df_planes_dev) AEAJ_CUDA(cudaMalloc(&p->df_planes_dev, sizeof(DeflatePlane) * p->nplanes));
+    p->df_planes.resize(p->nplanes);
+    // scratch: per layer, per image, per chunk: output slot | tokens | length, Adler-32, offset
+    uint8_t* base = (uint8_t*)(((uintptr_t)scratch + 255) & ~(uintptr_t)255);
+    int max_chunks = 1;
+    for (int l = 0; l < 3; l++) {
+        AEAJ_REQUIRE(coef3[l] && io->out[l], "aeaj_deflate_coefficients: NULL buffer");
+        const int64_t cap = p->info.cap_coef[l], nch = deflate_chunks_cap(p, l), cap_out = deflate_cap_out(p, l);
+        max_chunks = std::max<int>(max_chunks, (int)nch);
+        for (int i = 0; i < B; i++) {
+            DeflatePlane& P = p->df_planes[i * 3 + l];
+            P.in = (const uint8_t*)(coef3[l] + (size_t)i * cap);
+            P.n_coef = counts + ((size_t)i * 3 + l) * 4 + 2;
+            P.cap_coef = cap;
+            P.out = io->out[l] + (size_t)i * cap_out;
+            P.cap_out = cap_out;
+            P.length = io->lengths + (size_t)i * 3 + l;
+            P.status = io->status;
+            P.slots = base; base += nch * DF_CHUNK_BOUND;
+            P.tok = (uint16_t*)base; base += nch * DF_CHUNK * 2;
+            P.chunk_off = (int64_t*)base; base += nch * 8;
+            P.chunk_len = (int32_t*)base; base += nch * 4;
+            P.chunk_adler = (uint32_t*)base; base += nch * 4;
+        }
+    }
+    if (io->status) AEAJ_CUDA(cudaMemsetAsync(io->status, 0, 4 * sizeof(int32_t), st));
+    const bool same = p->df_pushed_stream == st && p->df_pushed.size() == p->df_planes.size() &&
+                      memcmp(p->df_pushed.data(), p->df_planes.data(), sizeof(DeflatePlane) * p->df_planes.size()) == 0;
+    if (!same) { p->df_pushed = p->df_planes; p->df_pushed_stream = st; }
+    return launch_deflate(same ? nullptr : p->df_planes.data(), p->df_planes_dev, p->nplanes, max_chunks, st);
+}
+
 extern "C" int aeaj_pack_coefficients_host(const int32_t* coef, int64_t n, uint32_t* mask, int16_t* vals, int64_t* nnz, int* overflow) {
     AEAJ_REQUIRE(coef && mask && vals && nnz && n >= 0, "aeaj_pack_coefficients_host: bad arguments");
     int64_t k = 0;

@@ -3,7 +3,8 @@
 ``compress`` / ``decompress`` keep the reference's signatures, exceptions and the byte-compatible
 .ajpg container (jpeg.py:531-674); everything between the colour transform and the quantised
 coefficients -- and back -- runs on the GPU through libaeaj.so (aeaj_encode / aeaj_decode).
-Entropy coding (zigzag gather, state packing, zlib level 9) stays on the host, as in the reference.
+Entropy coding (zigzag gather, state packing, zlib level 9) stays on the host, as in the reference -- unless
+``Jpeg(settings, deflate="device")`` selects the device coder, which writes valid zlib streams that are not zlib's bytes.
 ``compress_batch`` / ``decompress_batch`` are additions for same-shape batches.
 """
 from __future__ import annotations
@@ -70,7 +71,14 @@ def _zigzag_stream(coef: np.ndarray, sizes: np.ndarray, zz_cache: dict, inverse:
 class Jpeg:
     """Adaptive-block JPEG codec (jpeg.py:177-800) backed by the B200 hot path."""
 
-    def __init__(self, settings: JpegCompressionSettings) -> None:
+    def __init__(self, settings: JpegCompressionSettings, deflate: str = "host") -> None:
+        """deflate: "host" (default) codes the coefficient streams with zlib level 9 on the host, the reference's own bytes;
+        "device" deflates them on the GPU (aeaj_deflate_coefficients) and moves only the compressed bytes -- faster end to end
+        and about 15 % larger (DESIGN.md section 5), readable by every .ajpg decoder, the reference's included, but not
+        byte-identical to its files."""
+        if deflate not in ("host", "device"):
+            raise ValueError("deflate must be 'host' or 'device'")
+        self.deflate = deflate
         self.update_settings(settings)
 
     # -- settings / caches ----------------------------------------------------------------------
@@ -143,6 +151,12 @@ class Jpeg:
                 host = np.stack([np.ascontiguousarray(imgs[i].data.reshape(H, W, 3), dtype=np.float32) for i in idxs])
             rgb = torch.from_numpy(host).pin_memory().to(f"cuda:{codec.device}", non_blocking=True)
             enc = codec.encode(rgb, s.color_space, s.quality_range, s.block_size_range, stream=True)
+            if self.deflate == "device":
+                df = codec.deflate(enc, s.color_space, s.quality_range, s.block_size_range)
+                downloaded = codec.download_deflated(enc, df)
+                for k, i in enumerate(idxs):
+                    out[i] = self._entropy_encode(downloaded[k], (H, W), imgs[i].extension, [L["zlib"] for L in downloaded[k]])
+                continue
             downloaded = codec.download(enc)
             # zlib level 9 is the end-to-end bottleneck once the hot path is on the GPU (SURVEY 8f-2): deflate every layer of
             # every image of the group concurrently (zlib releases the GIL; same bytes as the sequential reference loop)
@@ -198,13 +212,15 @@ class Jpeg:
             with ThreadPoolExecutor(max_workers=len(layers)) as pool:
                 streams = list(pool.map(self._deflate_layer, layers))
         for L, z in zip(layers, streams):
-            states = np.ascontiguousarray(L["states"], dtype=np.uint8)
             if "packed_states" in L:
                 packed = L["packed_states"]
+                n_states = L["n_states"] if "n_states" in L else len(L["states"])
             else:
+                states = np.ascontiguousarray(L["states"], dtype=np.uint8)
+                n_states = len(states)
                 packed = np.empty((len(states) + 3) // 4, dtype=np.uint8)
                 native.check(lib.aeaj_pack_states_host(states.ctypes.data, len(states), packed.ctypes.data), "aeaj_pack_states_host")
-            out.write((2 * len(states)).to_bytes(4, byteorder="big"))
+            out.write((2 * n_states).to_bytes(4, byteorder="big"))
             out.write(int(L["root"]).to_bytes(4, byteorder="big"))
             out.write(packed.tobytes())
             out.write(len(z).to_bytes(4, byteorder="big"))

@@ -255,6 +255,26 @@ AEAJ_API int aeaj_unpack_coefficients_host(const uint32_t* mask_host, const int1
 typedef struct { const void* src; void* dst; int64_t bytes; } aeaj_segment;
 AEAJ_API int aeaj_copy_segments(const aeaj_segment* segs_host, int n, void* table_dev, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Device entropy coder: deflate of the coefficient streams on the GPU, an alternative to the host's zlib level 9
+ * (jpeg.py:590) that moves only the compressed bytes over PCIe.  Each plane's stream of n_coef int32 (little-endian, as
+ * stored; with aeaj_plan_set_stream_layout(1) the bytes _entropy_encode hands to zlib) becomes ONE complete zlib stream
+ * (RFC 1950) that any inflate reads.  The bytes are not zlib's: the stream is coded in independent 64 KiB chunks, each one
+ * deflate block (dynamic, fixed or stored, whichever is smallest) ending byte-aligned.  They depend only on the input bytes
+ * -- not on the batch, the position in it, the stream or the GPU.  n_coef is read from counts[b][l][2] on the device (no
+ * host sync).  aeaj_deflate_caps: per-layer capacity of one plane's output (every input fits) and the bytes of the
+ * caller-owned device scratch the call needs (separate from the plan workspace).  Asynchronous on `stream`; after the first
+ * call on a plan, steady-state calls issue no host-to-device copy and can be captured in a CUDA graph.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct {
+    uint8_t* out[3];         /* [batch][cap_out[l]]: one zlib stream per plane */
+    int32_t* lengths;        /* [batch][3] bytes written, on the device (0 if a stream did not fit) */
+    int32_t* status;         /* optional device int32[4]: [0] planes whose stream did not fit (0 = ok) */
+} aeaj_deflate_io;
+AEAJ_API int aeaj_deflate_caps(const aeaj_plan* p, int64_t* cap_out3, int64_t* scratch_bytes);
+AEAJ_API int aeaj_deflate_coefficients(aeaj_plan* p, const int32_t* const* coef3, const int32_t* counts,
+                                       const aeaj_deflate_io* io, void* scratch, void* stream);
+
 /* Stream layout (SURVEY 8f rank 1).  zigzag = 0 (default): each block of the coefficient stream is row-major,
  * i.e. the reference's img_quantized blocks.  zigzag = 1: each block is stored in the zigzag order of
  * Jpeg._zigzag_ordering (jpeg.py:726-766), i.e. the stream is byte-for-byte what _entropy_encode hands to zlib
