@@ -66,6 +66,24 @@ class DeflatedBatch:
 
 
 @dataclass
+class InflatedBatch:
+    """Device inflate of one batch's zlib streams into the plan's coefficient buffers (include/aeaj.h,
+    aeaj_inflate_coefficients); the per-plane results stay on the device until read."""
+    coef: List[torch.Tensor]       # 3 x int32 [B, cap_coef_l]: the plan's buffers, as aeaj_decode reads them
+    status: torch.Tensor           # int32 [B, 3]  0 ok, else the INFLATE_ERRORS code
+    out_bytes: torch.Tensor        # int64 [B, 3]  bytes written
+    segments: torch.Tensor         # int32 [B, 3]  parts decoded independently (sync points of the stream)
+
+
+# statuses of aeaj_inflate_coefficients (csrc/inflate_core.h), worded like zlib's messages
+INFLATE_ERRORS = {1: "incorrect header check", 2: "preset dictionary required", 3: "invalid block type",
+                  4: "invalid stored block lengths", 5: "invalid code lengths", 6: "invalid literal/length or distance code",
+                  7: "invalid distance too far back", 8: "incomplete or truncated stream", 9: "incorrect data check",
+                  10: "coefficient stream length does not match the quadtree header"}
+INFLATE_LENGTH = 10
+
+
+@dataclass
 class _Plan:
     ptr: C.c_void_p
     info: native.PlanInfo
@@ -79,6 +97,8 @@ class _Plan:
     packed: Optional[PackedBatch] = None
     deflated: Optional[DeflatedBatch] = None
     deflate_scratch: Optional[torch.Tensor] = None
+    inflated: Optional[InflatedBatch] = None
+    inflate_scratch: Optional[torch.Tensor] = None
     nbytes: int = 0
 
 
@@ -336,6 +356,96 @@ class DeviceCodec:
                                    packed_states=enc.packed_states[l][b, :(ns + 3) // 4].cpu().numpy(), n_states=ns, root=root))
             out.append(layers)
         return out
+
+    def inflate(self, zbuf: torch.Tensor, offsets: torch.Tensor, lengths: torch.Tensor, counts: torch.Tensor, B, H, W, space,
+                qrange, brange, instance: int = 0) -> InflatedBatch:
+        """Inflate plane (b, l)'s zlib stream zbuf[offsets[b, l] : + lengths[b, l]] (device uint8; int64 [B, 3] device
+        arrays) into the plan's coefficient buffers, on the device (aeaj_inflate_coefficients): the .ajpg reader's zlib
+        layer without the int32 streams crossing PCIe.  Each stream must inflate to exactly 4 * counts[b, l, 2] bytes
+        (counts as decode() takes them).  Asynchronous; the results belong to the plan and are reused by the next call."""
+        p = self._plan(B, H, W, space, brange, qrange, instance)
+        if zbuf.dtype != torch.uint8 or not zbuf.is_cuda or not zbuf.is_contiguous():
+            raise TypeError("inflate expects a contiguous uint8 CUDA tensor")
+        for t, dt in ((offsets, torch.int64), (lengths, torch.int64), (counts, torch.int32)):
+            if t.dtype != dt or not t.is_cuda or not t.is_contiguous() or t.shape[:2] != (B, 3):
+                raise TypeError("offsets / lengths: int64 [B, 3], counts: int32 [B, 3, 4], contiguous CUDA tensors")
+        dev = p.rgb_out.device
+        if p.inflated is None:
+            p.inflated = InflatedBatch(coef=p.out.coef, status=torch.zeros((B, 3), dtype=torch.int32, device=dev),
+                                       out_bytes=torch.zeros((B, 3), dtype=torch.int64, device=dev),
+                                       segments=torch.zeros((B, 3), dtype=torch.int32, device=dev))
+        need = C.c_int64()
+        native.check(self.lib.aeaj_inflate_scratch_bytes(p.ptr, zbuf.numel(), C.byref(need)), "aeaj_inflate_scratch_bytes")
+        if p.inflate_scratch is None or p.inflate_scratch.numel() < need.value:
+            if p.inflate_scratch is not None:
+                p.nbytes -= p.inflate_scratch.numel()
+            p.inflate_scratch = torch.empty(int(need.value), dtype=torch.uint8, device=dev)
+            p.nbytes += p.inflate_scratch.numel()
+            self._evict(keep=next(k for k, v in self._plans.items() if v is p))
+        ib = p.inflated
+        io = native.InflateIO()
+        io.inp = zbuf.data_ptr() if zbuf.numel() else None
+        io.offsets, io.lengths = offsets.data_ptr(), lengths.data_ptr()
+        for l in range(3):
+            io.coef[l] = ib.coef[l].data_ptr()
+        io.status, io.out_bytes, io.segments = ib.status.data_ptr(), ib.out_bytes.data_ptr(), ib.segments.data_ptr()
+        native.check(self.lib.aeaj_inflate_coefficients(p.ptr, C.byref(io), counts.data_ptr(), zbuf.numel(),
+                                                        p.inflate_scratch.data_ptr(), _stream()), "aeaj_inflate_coefficients")
+        return ib
+
+    def upload_for_inflate(self, per_image_layers, B, H, W, space, qrange, brange):
+        """per_image_layers[b][l] = dict(leaves (n,4) int32 incl. coef offsets, zlib bytes, ncoef): the zlib bytes, leaves,
+        counts, offsets and lengths in ONE pinned host-to-device copy; the leaves land in the plan's buffers.  Returns the
+        device (zbuf, offsets, lengths, leaves, counts); asynchronous."""
+        p = self._plan(B, H, W, space, brange, qrange)
+        o = p.out
+        counts = np.zeros((B, 3, 4), dtype=np.int32)
+        offs = np.zeros((B, 3), dtype=np.int64)
+        lens = np.zeros((B, 3), dtype=np.int64)
+        zl = 0
+        for b in range(B):
+            for l in range(3):
+                d = per_image_layers[b][l]
+                nl = len(d["leaves"])
+                if nl > p.info.cap_leaves[l] or d["ncoef"] > p.info.cap_coef[l]:
+                    raise ValueError("stream does not fit the layer geometry (corrupt input?)")
+                counts[b, l, 0], counts[b, l, 2] = nl, d["ncoef"]
+                offs[b, l], lens[b, l] = zl, len(d["zlib"])
+                zl += len(d["zlib"])
+        zpad = (zl + 15) & ~15
+        nleaf = [[len(per_image_layers[b][l]["leaves"]) * 16 for l in range(3)] for b in range(B)]
+        total = zpad + sum(map(sum, nleaf)) + counts.nbytes + offs.nbytes + lens.nbytes
+        host = torch.empty(total, dtype=torch.uint8, pin_memory=True)
+        h = host.numpy()
+        pos = 0
+        for b in range(B):
+            for l in range(3):
+                z = per_image_layers[b][l]["zlib"]
+                h[pos:pos + len(z)] = np.frombuffer(z, dtype=np.uint8)
+                pos += len(z)
+        pos = zpad
+        for b in range(B):
+            for l in range(3):
+                n = nleaf[b][l]
+                h[pos:pos + n] = np.require(per_image_layers[b][l]["leaves"], dtype=np.int32, requirements=["C"]).view(np.uint8).ravel()
+                pos += n
+        tail = pos
+        for a in (counts, offs, lens):
+            h[pos:pos + a.nbytes] = a.view(np.uint8).ravel()
+            pos += a.nbytes
+        dev = host.to(p.rgb_out.device, non_blocking=True)
+        pos = zpad
+        for b in range(B):
+            for l in range(3):
+                n = nleaf[b][l]
+                if n:
+                    o.leaves[l][b, :n // 16].view(-1).view(torch.uint8).copy_(dev[pos:pos + n], non_blocking=True)
+                pos += n
+        o.counts.view(-1).view(torch.uint8).copy_(dev[tail:tail + counts.nbytes], non_blocking=True)
+        pos = tail + counts.nbytes
+        d_offs = dev[pos:pos + offs.nbytes].view(torch.int64).view(B, 3)
+        d_lens = dev[pos + offs.nbytes:pos + offs.nbytes + lens.nbytes].view(torch.int64).view(B, 3)
+        return dev[:zl], d_offs, d_lens, o.leaves, o.counts
 
     def unpack(self, pk: PackedBatch, B, H, W, space, qrange, brange, instance: int = 0) -> List[torch.Tensor]:
         """Inverse of pack(): expands into the plan's int32 coefficient buffers (returned); asynchronous."""

@@ -27,7 +27,7 @@ EXPORTS = [
     "aeaj_peer_alloc", "aeaj_peer_free", "aeaj_peer_export", "aeaj_peer_open", "aeaj_peer_close",
     "aeaj_plan_set_peers", "aeaj_copy_segments",
     "aeaj_encode_halo", "aeaj_decode_halo", "aeaj_set_fast_transfer",
-    "aeaj_deflate_caps", "aeaj_deflate_coefficients",
+    "aeaj_deflate_caps", "aeaj_deflate_coefficients", "aeaj_inflate_scratch_bytes", "aeaj_inflate_coefficients",
 ]
 
 
@@ -60,6 +60,11 @@ class PackedIO(C.Structure):
 
 class DeflateIO(C.Structure):
     _fields_ = [("out", C.c_void_p * 3), ("lengths", C.c_void_p), ("status", C.c_void_p)]
+
+
+class InflateIO(C.Structure):
+    _fields_ = [("inp", C.c_void_p), ("offsets", C.c_void_p), ("lengths", C.c_void_p), ("coef", C.c_void_p * 3),
+                ("status", C.c_void_p), ("out_bytes", C.c_void_p), ("segments", C.c_void_p)]
 
 
 class Segment(C.Structure):
@@ -136,6 +141,8 @@ def load():
         lib.aeaj_unpack_coefficients_host.argtypes = [vp, vp, C.c_int64, C.c_int64, vp]
         lib.aeaj_deflate_caps.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         lib.aeaj_deflate_coefficients.argtypes = [vp, C.POINTER(vp), vp, C.POINTER(DeflateIO), vp, vp]
+        lib.aeaj_inflate_scratch_bytes.argtypes = [vp, C.c_int64, C.POINTER(C.c_int64)]
+        lib.aeaj_inflate_coefficients.argtypes = [vp, C.POINTER(InflateIO), vp, C.c_int64, vp, vp]
         _lib = lib
         return lib
 

@@ -256,6 +256,30 @@ size_t deflate_chunk_scratch_bytes();
 int aeaj_deflate_init();
 int launch_deflate(const DeflatePlane* planes_host, DeflatePlane* planes_dev, int nplanes, int max_chunks, cudaStream_t st);
 
+// one plane's zlib stream -> its coefficient buffer (inflate.cu, inflate_core.h)
+struct InflatePlane {
+    const int64_t* offset;    // device: the stream's first byte in the input buffer
+    const int64_t* length;    // device: its bytes
+    const int32_t* n_coef;    // device: coefficients the stream must inflate to (4 bytes each)
+    uint8_t* out;             // the plane's coefficient buffer, as bytes
+    int64_t cap_bytes;
+    int32_t* status;          // device: IF_* of inflate_core.h
+    int64_t* out_bytes;       // device: bytes written
+    int32_t* segments;        // device: merged segments decoded independently
+};
+struct IfSeg;
+struct IfStream;
+struct InflateArgs {
+    const uint8_t* in;        // the input buffer
+    int64_t in_bytes;
+    int nplanes, cap_segs;    // candidate list: the planes' first segments, then up to cap_segs - nplanes sync points
+    int* counters;            // [0] sync points found, [1] / [2] next candidate of the speculative / output pass
+    IfStream* streams;        // [nplanes]
+    IfSeg* segs;              // [cap_segs]
+    int32_t* map;             // [in_bytes / 4 + 1]: input position >> 2 -> candidate index (-1: list full)
+};
+int launch_inflate(const InflatePlane* planes_host, InflatePlane* planes_dev, const InflateArgs& a, int sm_count, cudaStream_t st);
+
 // kernels' host launchers (defined in the .cu files)
 int aeaj_canny_init(aeaj_handle* h);
 int aeaj_dct_init(aeaj_handle* h);

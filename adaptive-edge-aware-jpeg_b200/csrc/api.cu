@@ -7,6 +7,7 @@
 #include <vector>
 #include "aeaj_internal.cuh"
 #include "deflate_core.h"
+#include "inflate_core.h"
 
 // ---------------------------------------------------------------------------------------------
 // errors
@@ -403,6 +404,9 @@ struct aeaj_plan {
     std::vector<DeflatePlane> df_planes, df_pushed;   // deflate descriptors, the same scheme
     DeflatePlane* df_planes_dev = nullptr;
     cudaStream_t df_pushed_stream = nullptr;
+    std::vector<InflatePlane> if_planes, if_pushed;   // inflate descriptors, the same scheme
+    InflatePlane* if_planes_dev = nullptr;
+    cudaStream_t if_pushed_stream = nullptr;
     // one image over several GPUs (peer.cu): the other ranks' workspaces / barrier flags, opened through CUDA IPC by the caller
     PeerSet peers = {1, 0, {0}};
     void* peer_ws[AEAJ_MAX_PEERS] = {nullptr};
@@ -544,7 +548,7 @@ extern "C" int aeaj_plan_create(aeaj_handle* h, int batch, int height, int width
 extern "C" int aeaj_plan_destroy(aeaj_plan* p) {
     if (!p) return 0;
     cudaSetDevice(p->h->device);
-    cudaFree(p->planes_dev); cudaFree(p->class_off_dev); cudaFree(p->outs_dev); cudaFree(p->qtab_dev); cudaFree(p->qtabf_dev); cudaFree(p->pack_planes_dev); cudaFree(p->peer_segs_dev); cudaFree(p->df_planes_dev);
+    cudaFree(p->planes_dev); cudaFree(p->class_off_dev); cudaFree(p->outs_dev); cudaFree(p->qtab_dev); cudaFree(p->qtabf_dev); cudaFree(p->pack_planes_dev); cudaFree(p->peer_segs_dev); cudaFree(p->df_planes_dev); cudaFree(p->if_planes_dev);
     delete p;
     return 0;
 }
@@ -941,6 +945,67 @@ extern "C" int aeaj_deflate_coefficients(aeaj_plan* p, const int32_t* const* coe
                       memcmp(p->df_pushed.data(), p->df_planes.data(), sizeof(DeflatePlane) * p->df_planes.size()) == 0;
     if (!same) { p->df_pushed = p->df_planes; p->df_pushed_stream = st; }
     return launch_deflate(same ? nullptr : p->df_planes.data(), p->df_planes_dev, p->nplanes, max_chunks, st);
+}
+
+// ---------------------------------------------------------------------------------------------
+// device inflate of the coefficient streams (inflate.cu)
+// ---------------------------------------------------------------------------------------------
+// scratch: counters | per-plane streams | candidate segments | position map; the list holds every sync point of real
+// streams (one per 64 KiB chunk of output at most a few bytes apart only for hostile input); beyond it, a plane decodes
+// the rest of its stream in one piece
+struct InflateLayout { int64_t cap_segs, streams, segs, map, total; };
+static InflateLayout inflate_layout(int nplanes, int64_t in_bytes) {
+    InflateLayout L;
+    L.cap_segs = std::min<int64_t>(nplanes + in_bytes / 16 + 64, 1 << 30);
+    L.streams = 256;
+    L.segs = L.streams + ((nplanes * (int64_t)sizeof(IfStream) + 255) & ~(int64_t)255);
+    L.map = L.segs + ((L.cap_segs * (int64_t)sizeof(IfSeg) + 255) & ~(int64_t)255);
+    L.total = L.map + (in_bytes / 4 + 1) * 4 + 256;
+    return L;
+}
+
+extern "C" int aeaj_inflate_scratch_bytes(const aeaj_plan* p, int64_t in_bytes, int64_t* scratch_bytes) {
+    AEAJ_REQUIRE(p && scratch_bytes && in_bytes >= 0, "aeaj_inflate_scratch_bytes: bad arguments");
+    *scratch_bytes = inflate_layout(p->nplanes, in_bytes).total;
+    return 0;
+}
+
+extern "C" int aeaj_inflate_coefficients(aeaj_plan* p, const aeaj_inflate_io* io, const int32_t* counts, int64_t in_bytes,
+                                         void* scratch, void* stream) {
+    AEAJ_REQUIRE(p && io && counts && scratch && in_bytes >= 0 && io->offsets && io->lengths && io->status && io->out_bytes &&
+                 io->segments && (io->in || in_bytes == 0), "aeaj_inflate_coefficients: bad arguments");
+    const cudaStream_t st = ST(stream);
+    const int B = p->info.batch;
+    if (!p->if_planes_dev) AEAJ_CUDA(cudaMalloc(&p->if_planes_dev, sizeof(InflatePlane) * p->nplanes));
+    p->if_planes.resize(p->nplanes);
+    for (int l = 0; l < 3; l++) {
+        AEAJ_REQUIRE(io->coef[l], "aeaj_inflate_coefficients: NULL buffer");
+        const int64_t cap = p->info.cap_coef[l];
+        for (int i = 0; i < B; i++) {
+            const size_t k = (size_t)i * 3 + l;
+            InflatePlane& P = p->if_planes[k];
+            P.offset = io->offsets + k;
+            P.length = io->lengths + k;
+            P.n_coef = counts + k * 4 + 2;
+            P.out = (uint8_t*)(io->coef[l] + (size_t)i * cap);
+            P.cap_bytes = 4 * cap;
+            P.status = io->status + k;
+            P.out_bytes = io->out_bytes + k;
+            P.segments = io->segments + k;
+        }
+    }
+    const InflateLayout L = inflate_layout(p->nplanes, in_bytes);
+    uint8_t* base = (uint8_t*)(((uintptr_t)scratch + 255) & ~(uintptr_t)255);
+    InflateArgs a;
+    a.in = io->in; a.in_bytes = in_bytes; a.nplanes = p->nplanes; a.cap_segs = (int)L.cap_segs;
+    a.counters = (int*)base;
+    a.streams = (IfStream*)(base + L.streams);
+    a.segs = (IfSeg*)(base + L.segs);
+    a.map = (int32_t*)(base + L.map);
+    const bool same = p->if_pushed_stream == st && p->if_pushed.size() == p->if_planes.size() &&
+                      memcmp(p->if_pushed.data(), p->if_planes.data(), sizeof(InflatePlane) * p->if_planes.size()) == 0;
+    if (!same) { p->if_pushed = p->if_planes; p->if_pushed_stream = st; }
+    return launch_inflate(same ? nullptr : p->if_planes.data(), p->if_planes_dev, a, p->h->sm_count, st);
 }
 
 extern "C" int aeaj_pack_coefficients_host(const int32_t* coef, int64_t n, uint32_t* mask, int16_t* vals, int64_t* nnz, int* overflow) {

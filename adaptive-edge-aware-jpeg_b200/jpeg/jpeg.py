@@ -4,7 +4,8 @@
 .ajpg container (jpeg.py:531-674); everything between the colour transform and the quantised
 coefficients -- and back -- runs on the GPU through libaeaj.so (aeaj_encode / aeaj_decode).
 Entropy coding (zigzag gather, state packing, zlib level 9) stays on the host, as in the reference -- unless
-``Jpeg(settings, deflate="device")`` selects the device coder, which writes valid zlib streams that are not zlib's bytes.
+``Jpeg(settings, deflate="device")`` selects the device coder and decoder: compress writes valid zlib streams that are not
+zlib's bytes, decompress inflates any .ajpg file's streams on the GPU.
 ``compress_batch`` / ``decompress_batch`` are additions for same-shape batches.
 """
 from __future__ import annotations
@@ -68,14 +69,30 @@ def _zigzag_stream(coef: np.ndarray, sizes: np.ndarray, zz_cache: dict, inverse:
     return out
 
 
+def _raise_inflate_status(status: np.ndarray) -> None:
+    """the first failed plane of aeaj_inflate_coefficients as the host path's exception: ValueError for a length mismatch
+    (as its size check), zlib.error for everything else"""
+    from aeaj.codec import INFLATE_ERRORS, INFLATE_LENGTH
+    for code in status.ravel():
+        if code == INFLATE_LENGTH:
+            raise ValueError(INFLATE_ERRORS[INFLATE_LENGTH])
+        if code:
+            raise zlib.error(f"Error while decompressing data on the device: {INFLATE_ERRORS.get(int(code), int(code))}")
+
+
 class Jpeg:
     """Adaptive-block JPEG codec (jpeg.py:177-800) backed by the B200 hot path."""
 
     def __init__(self, settings: JpegCompressionSettings, deflate: str = "host") -> None:
-        """deflate: "host" (default) codes the coefficient streams with zlib level 9 on the host, the reference's own bytes;
-        "device" deflates them on the GPU (aeaj_deflate_coefficients) and moves only the compressed bytes -- faster end to end
-        and about 15 % larger (DESIGN.md section 5), readable by every .ajpg decoder, the reference's included, but not
-        byte-identical to its files."""
+        """deflate: where the zlib layer of the coefficient streams runs, in both directions.
+        "host" (default): compress codes them with zlib level 9, the reference's own bytes; decompress uses zlib.decompress.
+        "device": compress deflates them on the GPU (aeaj_deflate_coefficients) and moves only the compressed bytes -- faster
+        end to end and about 15 % larger (DESIGN.md section 5), readable by every .ajpg decoder, the reference's included, but
+        not byte-identical to its files; decompress inflates them on the GPU (aeaj_inflate_coefficients), straight into the
+        buffers the decoder reads.  It reads any .ajpg file, the reference's zlib-9 files included, and gives the same images.
+        Errors: a corrupt zlib section raises zlib.error and a coefficient count that does not match the quadtree header raises
+        ValueError, as on the host -- with one difference: a stream that inflates past the expected length raises ValueError
+        even where zlib.decompress would have met a later error in it first."""
         if deflate not in ("host", "device"):
             raise ValueError("deflate must be 'host' or 'device'")
         self.deflate = deflate
@@ -174,15 +191,24 @@ class Jpeg:
         return self.decompress_batch([img_encoded], as_uint8=True)[0]
 
     def decompress_batch(self, streams: Sequence[bytes], as_uint8: bool = False) -> List[Image]:
-        parsed = [self._entropy_decode(b) for b in streams]
+        device = self.deflate == "device"
+        parsed = [self._entropy_decode(b, inflate=not device) for b in streams]
         out: List[Optional[Image]] = [None] * len(streams)
         groups = {}
         for i, p in enumerate(parsed):
             groups.setdefault((p["H"], p["W"], p["space"], p["quality"], p["blocks"]), []).append(i)
         codec = get_codec()
         for (H, W, space, q, b), idxs in groups.items():
-            coef, leaves, counts = codec.upload_for_decode([parsed[i]["layers"] for i in idxs], len(idxs), H, W, space, q, b)
+            layers = [parsed[i]["layers"] for i in idxs]
+            if device:
+                zbuf, offs, lens, leaves, counts = codec.upload_for_inflate(layers, len(idxs), H, W, space, q, b)
+                inf = codec.inflate(zbuf, offs, lens, counts, len(idxs), H, W, space, q, b)
+                coef = inf.coef
+            else:
+                coef, leaves, counts = codec.upload_for_decode(layers, len(idxs), H, W, space, q, b)
             rgb = codec.decode(coef, leaves, counts, len(idxs), H, W, space, q, b, zigzag=True, out="u8" if as_uint8 else "f32").cpu().numpy()
+            if device:
+                _raise_inflate_status(inf.status.cpu().numpy())
             codec.check_status(codec.last_decode_status, "decode")
             for k, i in enumerate(idxs):
                 out[i] = rgb[k] if as_uint8 else Image.from_array(rgb[k].reshape(-1, 3), (H, W, 3), parsed[i]["extension"])
@@ -227,7 +253,8 @@ class Jpeg:
             out.write(z)
         return out.getvalue()
 
-    def _entropy_decode(self, encoded_data: bytes) -> dict:
+    def _entropy_decode(self, encoded_data: bytes, inflate: bool = True) -> dict:
+        """the .ajpg framing; inflate=False leaves each layer's zlib bytes for the device (zlib, ncoef instead of coef)"""
         s = BytesIO(encoded_data)
         ml = int.from_bytes(s.read(4), byteorder="big")
         meta = json.loads(s.read(ml).decode("utf-8"))
@@ -245,6 +272,9 @@ class Jpeg:
             states = np.stack([(raw >> 6) & 3, (raw >> 4) & 3, (raw >> 2) & 3, raw & 3], axis=1).reshape(-1)[: nbits // 2]
             leaves, ncoef = native.states_to_leaves(states.astype(np.uint8), root, int(shapes[i][0]), int(shapes[i][1]), blocks)
             zl = int.from_bytes(s.read(4), byteorder="big")
+            if not inflate:
+                layers.append(dict(leaves=leaves, zlib=s.read(zl), ncoef=int(ncoef)))
+                continue
             coef = np.frombuffer(zlib.decompress(s.read(zl)), dtype=np.int32)
             if coef.size != ncoef:
                 raise ValueError("coefficient stream length does not match the quadtree header")

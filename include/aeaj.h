@@ -275,6 +275,37 @@ AEAJ_API int aeaj_deflate_caps(const aeaj_plan* p, int64_t* cap_out3, int64_t* s
 AEAJ_API int aeaj_deflate_coefficients(aeaj_plan* p, const int32_t* const* coef3, const int32_t* counts,
                                        const aeaj_deflate_io* io, void* scratch, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Device entropy decoder: inflate of the coefficient streams on the GPU, the counterpart of aeaj_deflate_coefficients and
+ * an alternative to the host's zlib.decompress (jpeg.py:659): only the compressed bytes cross PCIe, and the coefficients
+ * land in the buffers aeaj_decode reads.  Plane (b, l)'s zlib stream is in[offsets[b][l], + lengths[b][l]) (device arrays;
+ * ranges outside [0, in_bytes) are clamped to it; streams must not overlap); it must inflate to exactly
+ * 4 * counts[b][l][2] bytes (counts as aeaj_decode takes them, read on the device), written to coef[l] + b * cap_coef[l].
+ * Any zlib stream is read (RFC 1950 / 1951, as zlib's inflate accepts it: the reference's level-9 files included); it is
+ * decoded in parallel at its sync points (the non-final empty stored blocks of Z_SYNC_FLUSH / Z_FULL_FLUSH, which the
+ * device coder writes after every 64 KiB chunk) and one warp per plane where it has none.  Per plane on the device:
+ *   status: 0 ok, 1 header (FCHECK, method, window), 2 preset dictionary, 3 block type, 4 stored length, 5 code lengths,
+ *           6 invalid symbol, 7 distance too far back, 8 truncated, 9 Adler-32 mismatch, 10 length (the stream does not
+ *           inflate to exactly the expected bytes; decoding stops at the expected length);
+ *   out_bytes: bytes written (never beyond the expected length or the buffer);  segments: parts decoded independently.
+ * Nothing outside a stream's bytes is read and nothing outside [0, expected) of its plane is written, whatever the input.
+ * aeaj_inflate_scratch_bytes: the caller-owned device scratch for inputs of up to in_bytes (separate from the workspace).
+ * Asynchronous on `stream`, no host sync; after the first call on a plan, steady-state calls issue no host-to-device copy
+ * and can be captured in a CUDA graph.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct {
+    const uint8_t* in;       /* the zlib streams */
+    const int64_t* offsets;  /* [batch][3] */
+    const int64_t* lengths;  /* [batch][3] */
+    int32_t* coef[3];        /* [batch][cap_coef[l]] */
+    int32_t* status;         /* [batch][3] */
+    int64_t* out_bytes;      /* [batch][3] */
+    int32_t* segments;       /* [batch][3] */
+} aeaj_inflate_io;
+AEAJ_API int aeaj_inflate_scratch_bytes(const aeaj_plan* p, int64_t in_bytes, int64_t* scratch_bytes);
+AEAJ_API int aeaj_inflate_coefficients(aeaj_plan* p, const aeaj_inflate_io* io, const int32_t* counts, int64_t in_bytes,
+                                       void* scratch, void* stream);
+
 /* Stream layout (SURVEY 8f rank 1).  zigzag = 0 (default): each block of the coefficient stream is row-major,
  * i.e. the reference's img_quantized blocks.  zigzag = 1: each block is stored in the zigzag order of
  * Jpeg._zigzag_ordering (jpeg.py:726-766), i.e. the stream is byte-for-byte what _entropy_encode hands to zlib
