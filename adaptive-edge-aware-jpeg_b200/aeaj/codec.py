@@ -84,6 +84,31 @@ INFLATE_LENGTH = 10
 
 
 @dataclass
+class _HostStaging:
+    """Buffers of one stream slot of roundtrip_host_pipelined (one frame per job): pinned host memory for what crosses PCIe
+    in per-range copies, and the device-side input frame and arena."""
+    coef: List[torch.Tensor]       # 3 x int32 [cap_coef_l]     pinned
+    leaves: List[torch.Tensor]     # 3 x int32 [cap_leaves_l, 4]
+    states: List[torch.Tensor]     # 3 x uint8 [cap_states_l]
+    counts: torch.Tensor           # int32 [1, 3, 4]  of EncodedBatch.counts
+    pk_counts: torch.Tensor        # int32 [1, 3, 4]  of PackedBatch.counts
+    rgb_dev: Dict[torch.dtype, torch.Tensor] = field(default_factory=dict)   # device input frame [1,H,W,3] per pixel dtype used
+    arena_dev: Optional[torch.Tensor] = None       # a frame's packed streams, contiguous (device and pinned host)
+    arena_host: Optional[torch.Tensor] = None
+
+
+@dataclass
+class _Job:
+    """One frame in flight in roundtrip_host_pipelined."""
+    frame: int                     # index into host_in / host_out
+    slot: int                      # stream and plan instance
+    p: _Plan
+    enc: EncodedBatch
+    encoded: torch.cuda.Event      # phase A done: the counts are on the host
+    decoded: Optional[torch.cuda.Event] = None    # recorded after the job's last copy, when phase B is issued
+
+
+@dataclass
 class _Plan:
     ptr: C.c_void_p
     info: native.PlanInfo
@@ -92,7 +117,7 @@ class _Plan:
     rgb_out: torch.Tensor
     rgb8_out: Optional[torch.Tensor] = None
     qkey: Optional[tuple] = None
-    keep: list = field(default_factory=list)
+    staging: Optional[_HostStaging] = None
     dec_status: Optional[torch.Tensor] = None     # int32 [64]: [2] tensor-IDCT timeout flag, [3] leaves rejected by the device guard
     packed: Optional[PackedBatch] = None
     deflated: Optional[DeflatedBatch] = None
@@ -526,286 +551,160 @@ class DeviceCodec:
     # ------------------------------------------------------------------------------------------
     # host-buffer path (what a caller holding numpy / pinned host memory uses; bench.py e2e leg)
     # ------------------------------------------------------------------------------------------
-    def _host_staging(self, p: _Plan, with_rgb: bool = False):
-        if not p.keep:
-            B = p.info.batch
-            st = dict(
-                coef=[torch.empty((B, int(p.info.cap_coef[l])), dtype=torch.int32).pin_memory() for l in range(3)],
-                leaves=[torch.empty((B, int(p.info.cap_leaves[l]), 4), dtype=torch.int32).pin_memory() for l in range(3)],
-                states=[torch.empty((B, int(p.info.cap_states[l])), dtype=torch.uint8).pin_memory() for l in range(3)],
-                counts=torch.empty((B, 3, 4), dtype=torch.int32).pin_memory(),
-                pk_counts=torch.empty((B, 3, 4), dtype=torch.int32).pin_memory(),
-                mask=[torch.empty((B, int(p.info.cap_coef[l]) // 32 + 1), dtype=torch.int32).pin_memory() for l in range(3)],
-                vals=[torch.empty((B, int(p.info.cap_coef[l])), dtype=torch.int16).pin_memory() for l in range(3)],
-                rgb_dev=torch.empty((B, p.info.height, p.info.width, 3), dtype=torch.float32, device=p.rgb_out.device),
-                rgb8_dev=torch.empty((B, p.info.height, p.info.width, 3), dtype=torch.uint8, device=p.rgb_out.device))
-            p.keep.append(st)
-        st = p.keep[0]
-        if with_rgb and "rgb_out" not in st:
-            st["rgb_out"] = torch.empty((p.info.batch, p.info.height, p.info.width, 3), dtype=torch.float32).pin_memory()
-        return st
+    def _host_staging(self, p: _Plan) -> _HostStaging:
+        if p.staging is None:
+            info = p.info
+            p.staging = _HostStaging(
+                coef=[torch.empty(int(info.cap_coef[l]), dtype=torch.int32).pin_memory() for l in range(3)],
+                leaves=[torch.empty((int(info.cap_leaves[l]), 4), dtype=torch.int32).pin_memory() for l in range(3)],
+                states=[torch.empty(int(info.cap_states[l]), dtype=torch.uint8).pin_memory() for l in range(3)],
+                counts=torch.empty((1, 3, 4), dtype=torch.int32).pin_memory(),
+                pk_counts=torch.empty((1, 3, 4), dtype=torch.int32).pin_memory())
+        return p.staging
 
-    def _arena(self, p: _Plan, st: dict):
+    def _arena(self, p: _Plan):
         """one contiguous device + pinned-host buffer that holds a whole frame's packed streams (mask words, int16 values,
         leaves, states of the three layers), so that a frame travels in ONE copy per direction (aeaj_copy_segments)"""
-        if "arena_dev" not in st:
+        st = p.staging
+        if st.arena_dev is None:
             n = 0
             for l in range(3):
                 cc = int(p.info.cap_coef[l])
                 n += (cc // 32 + 1) * 4 + cc * 2 + int(p.info.cap_leaves[l]) * 16 + int(p.info.cap_states[l]) + 4 * 32
-            n = p.info.batch * n
-            st["arena_dev"] = torch.empty(n, dtype=torch.uint8, device=p.rgb_out.device)
-            st["arena_host"] = torch.empty(n, dtype=torch.uint8).pin_memory()
-            st["seg_table"] = torch.empty(64 * 24 * max(1, p.info.batch), dtype=torch.uint8, device=p.rgb_out.device)
-        return st["arena_dev"], st["arena_host"], st["seg_table"]
+            st.arena_dev = torch.empty(n, dtype=torch.uint8, device=p.rgb_out.device)
+            st.arena_host = torch.empty(n, dtype=torch.uint8).pin_memory()
+        return st.arena_dev, st.arena_host
 
-    def _copy_segments(self, segs, table: torch.Tensor):
+    def _copy_segments(self, segs):
+        """(src, dst, bytes) ranges in one launch; a frame has 12, within the 64 that travel in the kernel parameters"""
         arr = (native.Segment * len(segs))()
         for k, (src, dst, nb) in enumerate(segs):
             arr[k].src, arr[k].dst, arr[k].bytes = src, dst, nb
-        native.check(self.lib.aeaj_copy_segments(arr, len(segs), table.data_ptr(), _stream()), "aeaj_copy_segments")
+        native.check(self.lib.aeaj_copy_segments(arr, len(segs), None, _stream()), "aeaj_copy_segments")
 
-    def host_staging(self, B, H, W, space, brange, qrange):
-        return self._host_staging(self._plan(B, H, W, space, brange, qrange))
-
-    def encode_host(self, rgb_host: torch.Tensor, space, qrange, brange):
-        """rgb_host: pinned float32 CPU tensor [B,H,W,3].  H2D, encode, D2H of the used parts of the
-        coefficient / leaf / state buffers into pinned staging.  Returns (staging dict, counts ndarray, bytes h2d, bytes d2h)."""
-        B, H, W, _ = rgb_host.shape
-        p = self._plan(B, H, W, space, brange, qrange)
-        st = self._host_staging(p, with_rgb=True)
-        st["rgb_dev"].copy_(rgb_host, non_blocking=True)
-        enc = self.encode(st["rgb_dev"], space, qrange, brange)
-        st["counts"].copy_(enc.counts, non_blocking=True)
-        torch.cuda.current_stream().synchronize()
-        counts = st["counts"].numpy()
-        d2h = st["counts"].numel() * 4
-        for l in range(3):
-            for b in range(B):                              # contiguous per-image slices -> plain async memcpys
-                nl, ns, nc = (int(counts[b, l, k]) for k in range(3))
-                st["coef"][l][b, :nc].copy_(enc.coef[l][b, :nc], non_blocking=True)
-                st["leaves"][l][b, :nl].copy_(enc.leaves[l][b, :nl], non_blocking=True)
-                st["states"][l][b, :ns].copy_(enc.states[l][b, :ns], non_blocking=True)
-                d2h += nc * 4 + nl * 16 + ns
-        torch.cuda.current_stream().synchronize()
-        return st, counts, rgb_host.numel() * 4, d2h
-
-    def decode_host(self, st, counts: np.ndarray, B, H, W, space, qrange, brange):
-        """Inverse of encode_host: H2D of the used parts, decode, D2H of the RGB batch into pinned staging."""
-        p = self._plan(B, H, W, space, brange, qrange)
-        o = p.out
-        h2d = st["counts"].numel() * 4
-        for l in range(3):
-            for b in range(B):
-                nl, nc = int(counts[b, l, 0]), int(counts[b, l, 2])
-                o.coef[l][b, :nc].copy_(st["coef"][l][b, :nc], non_blocking=True)
-                o.leaves[l][b, :nl].copy_(st["leaves"][l][b, :nl], non_blocking=True)
-                h2d += nc * 4 + nl * 16
-        o.counts.copy_(st["counts"], non_blocking=True)
-        rgb = self.decode(o.coef, o.leaves, o.counts, B, H, W, space, qrange, brange)
-        st["rgb_out"].copy_(rgb, non_blocking=True)
-        torch.cuda.current_stream().synchronize()
-        return st["rgb_out"], h2d, st["rgb_out"].numel() * 4
-
-    def roundtrip_host_pipelined(self, host_in: torch.Tensor, host_out: torch.Tensor, space, qrange, brange, slots: int = 8, repeat: int = 1, lag: int = 3,
-                                 packed: bool = True, threads: int = 1, frames_per_job: int = 1, zero_copy: bool = False):
+    def roundtrip_host_pipelined(self, host_in: torch.Tensor, host_out: torch.Tensor, space, qrange, brange, slots: int = 8, repeat: int = 1,
+                                 lag: int = 3, packed: bool = True):
         """Host-buffer encode+decode of every frame of `host_in` (pinned float32 -- or uint8, the 8-bit image flow
-        Image.load -> compress ... decompress -> Image.save -- [F,H,W,3]) into `host_out` (float32 or uint8), `frames_per_job`
-        frames per job, jobs round-robin over `slots` CUDA streams so that the H2D and D2H copies of different jobs overlap
-        each other and the kernels (PCIe is full duplex; the step is copy-bound).  Per job, in stream order:
+        Image.load -> compress ... decompress -> Image.save -- [F,H,W,3]) into `host_out` (float32 or uint8), one frame per
+        job, jobs round-robin over `slots` CUDA streams so that the H2D and D2H copies of different jobs overlap each other
+        and the kernels (PCIe is full duplex; the step is copy-bound).  Per job, in stream order:
         H2D RGB -> aeaj_encode -> D2H counts -> [host waits for the counts] -> D2H of the job's streams ->
         H2D of the same bytes (what a host-side entropy decoder would hand back) -> aeaj_decode -> D2H RGB.
+        The host waits for a job's counts `lag` jobs later (at most slots - 1), so that the wait normally does not block.
         `repeat` > 1 streams the same F frames that many times back to back (a long-running ingest) without draining
         the pipeline in between.  packed=True moves the coefficient streams in their packed form (bit mask + int16 non-zeros,
-        aeaj_pack_coefficients after the encode, aeaj_unpack_coefficients before the decode; a plane whose overflow flag is
-        set travels as int32) and all of a job's streams as ONE copy per direction (aeaj_copy_segments).
-        zero_copy=True (packed only): the small transfers -- the counts and the arena of packed streams, ~4 MB per 4K frame -- are
-        written to / read from the pinned host buffers by the gather / scatter kernels themselves (pinned memory is mapped
-        into the device's address space), so the copy engines carry nothing but the two pixel transfers of every frame and
-        a copy that is ready is never queued behind one that still waits for a kernel.  Measured: no faster (0.85 vs 0.82 ms per
-        frame), so it is off by default -- the copy queues are not what keeps copies and kernels from overlapping fully.
+        aeaj_pack_coefficients after the encode, aeaj_unpack_coefficients before the decode) and all of a job's streams as ONE
+        copy per direction (aeaj_copy_segments); a job in which any plane overflows int16 travels as with packed=False:
+        raw int32 streams, one copy per range.
         Measured on B200 (tools/e2e_sweep.py, profiles/r2_e2e_sweep.txt): 0.77 ms per 4K frame against 0.60 ms for the same bytes as
-        bare copies (48 GB/s per direction); more slots, several frames per job (`frames_per_job`) or several host threads
-        (`threads`, each driving its own slots) do not change it -- the driving thread is blocked on the device half of the time
-        and the device work alone takes 0.42 ms per frame: copies and kernels do not overlap fully on this box (a bare
+        bare copies (48 GB/s per direction) and 0.42 ms for the device work alone; the driving thread is blocked on the device
+        (`pipeline_host_wait_s`) half of the time: copies and kernels do not overlap fully there (a bare
         H2D -> idle kernel -> D2H chain on 8 streams shows the same loss).  Returns (h2d_bytes, d2h_bytes) summed over all jobs."""
-        F0, H, W, _ = host_in.shape
-        G = max(1, frames_per_job)
-        if F0 % G != 0:
-            raise ValueError(f"frames_per_job ({G}) must divide the number of frames ({F0})")
-        J = (F0 // G) * repeat                                      # jobs
+        F, H, W, _ = host_in.shape
+        J = F * repeat
+        lag = min(lag, slots - 1)
         dev = torch.device("cuda", self.device)
         if not hasattr(self, "_streams") or len(self._streams) < slots:
             self._streams = [torch.cuda.Stream(device=dev) for _ in range(slots)]
-        threads = max(1, min(threads, slots, J))
-        self.pipeline_host_wait_s = 0.0                            # time the driving thread(s) spent blocked on the device (diagnostic)
-        for slot in range(min(slots, J)):                          # plans and staging are created by one thread, before the workers start
-            self._host_staging(self._plan(G, H, W, space, brange, qrange, instance=slot))
-        if threads == 1:
-            return self._pipeline_worker(list(range(J)), list(range(slots)), G, host_in, host_out, space, qrange, brange, min(lag, slots - 1), packed,
-                                         zero_copy)
-        import concurrent.futures as cf
-        per = slots // threads
-        work = [([j for j in range(J) if j % threads == t], list(range(t * per, (t + 1) * per))) for t in range(threads)]
-        with cf.ThreadPoolExecutor(max_workers=threads) as ex:
-            res = list(ex.map(lambda w: self._pipeline_worker(w[0], w[1], G, host_in, host_out, space, qrange, brange,
-                                                                   min(max(1, lag // threads + 1), per - 1), packed, zero_copy), work))
-        return sum(r[0] for r in res), sum(r[1] for r in res)
-
-    def _pipeline_worker(self, job_ids, slot_ids, G, host_in, host_out, space, qrange, brange, lag, packed, zero_copy=False):
-        """one host thread of roundtrip_host_pipelined: the jobs `job_ids` (job j = frames j G .. j G + G - 1 of the repeated
-        frame sequence), round-robin over its own `slot_ids`"""
-        torch.cuda.set_device(self.device)                         # the current device is per host thread
-        F0, H, W, _ = host_in.shape
-        nslots = len(slot_ids)
+        self.pipeline_host_wait_s = 0.0                            # time the host spent blocked on the device (diagnostic)
         h2d = d2h = 0
-        jobs = []
-        # phase A for every job: upload + encode + counts
-        for k, j in enumerate(job_ids):
-            slot = slot_ids[k % nslots]
-            stream = self._streams[slot]
-            f0 = (j * G) % F0
-            p = self._plan(G, H, W, space, brange, qrange, instance=slot)
+        jobs: List[_Job] = []
+        for k in range(J):
+            slot = k % slots
+            if k >= slots:
+                self._wait_decoded(jobs[k - slots])                # the slot's previous job must be done with its buffers
+            p = self._plan(1, H, W, space, brange, qrange, instance=slot)
             st = self._host_staging(p)
-            with torch.cuda.stream(stream):
-                if k >= nslots:
-                    self._finish_job(jobs[k - nslots])             # the slot's previous job must be done with its buffers
-                src = st["rgb8_dev"] if host_in.dtype == torch.uint8 else st["rgb_dev"]
-                src.copy_(host_in[f0:f0 + G], non_blocking=True)
+            src = st.rgb_dev.get(host_in.dtype)
+            if src is None:
+                src = st.rgb_dev[host_in.dtype] = torch.empty((1, H, W, 3), dtype=host_in.dtype, device=dev)
+            f = k % F
+            # phase A: upload + encode + counts
+            with torch.cuda.stream(self._streams[slot]):
+                src.copy_(host_in[f:f + 1], non_blocking=True)
                 enc = self.encode(src, space, qrange, brange, instance=slot)
-                if packed and zero_copy:
+                st.counts.copy_(enc.counts, non_blocking=True)
+                if packed:
                     pk = self.pack(enc, space, qrange, brange, instance=slot)
-                    _, _, table = self._arena(p, st)
-                    self._copy_segments([(enc.counts.data_ptr(), st["counts"].data_ptr(), st["counts"].numel() * 4),
-                                         (pk.counts.data_ptr(), st["pk_counts"].data_ptr(), st["pk_counts"].numel() * 4)], table)
-                else:
-                    st["counts"].copy_(enc.counts, non_blocking=True)
-                    if packed:
-                        pk = self.pack(enc, space, qrange, brange, instance=slot)
-                        st["pk_counts"].copy_(pk.counts, non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(stream)
-            jobs.append(dict(f=f0, G=G, slot=slot, p=p, st=st, enc=enc, ev=ev, done=False, phase_b=False, packed=packed, zero_copy=packed and zero_copy))
-            h2d += G * host_in[0].numel() * host_in.element_size()
+                    st.pk_counts.copy_(pk.counts, non_blocking=True)
+                encoded = torch.cuda.Event()
+                encoded.record()
+            jobs.append(_Job(f, slot, p, enc, encoded))
+            h2d += host_in[0].numel() * host_in.element_size()
             # phase B of a job is issued `lag` jobs after its phase A (its counts have landed by then), and a slot is
-            # reused only `nslots` jobs later, so neither host wait normally blocks
+            # reused only `slots` jobs later, so neither host wait normally blocks
             if k >= lag:
-                a, b_ = self._phase_b(jobs[k - lag], host_out, space, qrange, brange)
+                a, b_ = self._phase_b(jobs[k - lag], host_out, space, qrange, brange, packed)
                 h2d += a; d2h += b_
-        for jb in jobs:
-            if not jb["phase_b"]:
-                a, b_ = self._phase_b(jb, host_out, space, qrange, brange)
-                h2d += a; d2h += b_
-        for jb in jobs:
-            self._finish_job(jb)
+        for jb in jobs[max(0, J - lag):]:
+            a, b_ = self._phase_b(jb, host_out, space, qrange, brange, packed)
+            h2d += a; d2h += b_
+        for jb in jobs[max(0, J - slots):]:
+            self._wait_decoded(jb)
         return h2d, d2h
 
-    def _phase_b(self, job, host_out, space, qrange, brange):
-        p, st, enc, slot, G = job["p"], job["st"], job["enc"], job["slot"], job["G"]
-        stream = self._streams[slot]
+    def _phase_b(self, job: _Job, host_out, space, qrange, brange, packed: bool):
+        p, st, enc, slot = job.p, job.p.staging, job.enc, job.slot
         t0 = time.perf_counter()
-        job["ev"].synchronize()                                    # counts are on the host now
+        job.encoded.synchronize()                                  # counts are on the host now
         self.pipeline_host_wait_s += time.perf_counter() - t0
-        counts = st["counts"].numpy()
-        h2d = d2h = st["counts"].numel() * 4
+        counts = st.counts.numpy()[0]
+        pkc = st.pk_counts.numpy()[0]
+        h2d = d2h = st.counts.numel() * 4
         H, W = p.info.height, p.info.width
-        pk = p.packed if job.get("packed") else None
-        pkc = st["pk_counts"].numpy() if pk is not None else None
         out_kind = "u8" if host_out.dtype == torch.uint8 else "f32"
-        if pk is not None and not (pkc[:, :, 2] != 0).any():
-            # the normal case (no int16 overflow): gather the job's streams into one arena, ONE copy each way, scatter back
-            arena_dev, arena_host, table = self._arena(p, st)
-            zc = job.get("zero_copy", False)
-            base = arena_host.data_ptr() if zc else arena_dev.data_ptr()
-            off = 0
-            there, back = [], []
-            for b in range(G):
+        route_packed = packed and not pkc[:, 2].any()
+        if route_packed:
+            arena_dev, arena_host = self._arena(p)
+        with torch.cuda.stream(self._streams[slot]):
+            if route_packed:
+                # gather the job's packed streams into one arena, ONE copy each way, scatter back
+                pk = p.packed
+                off = 0
+                there, back = [], []
                 for l in range(3):
-                    nl, ns = int(counts[b, l, 0]), int(counts[b, l, 1])
-                    nnz, nw = int(pkc[b, l, 0]), int(pkc[b, l, 3])
-                    for t, nb, needed_back in ((pk.mask[l][b], nw * 4, True), (pk.vals[l][b], nnz * 2, True), (enc.leaves[l][b], nl * 16, True),
-                                               (enc.states[l][b], ns, False)):
-                        there.append((t.data_ptr(), base + off, nb))
+                    nl, ns = int(counts[l, 0]), int(counts[l, 1])
+                    nnz, nw = int(pkc[l, 0]), int(pkc[l, 3])
+                    for t, nb, needed_back in ((pk.mask[l][0], nw * 4, True), (pk.vals[l][0], nnz * 2, True), (enc.leaves[l][0], nl * 16, True),
+                                               (enc.states[l][0], ns, False)):
+                        there.append((t.data_ptr(), arena_dev.data_ptr() + off, nb))
                         if needed_back:
-                            back.append((base + off, t.data_ptr(), nb))
+                            back.append((arena_dev.data_ptr() + off, t.data_ptr(), nb))
                         off = (off + nb + 15) & ~15
-            with torch.cuda.stream(stream):
-                if zc:
-                    # the gather kernel writes the host arena itself, the scatter kernel reads it back (and the counts with it)
-                    back += [(st["counts"].data_ptr(), enc.counts.data_ptr(), st["counts"].numel() * 4),
-                             (st["pk_counts"].data_ptr(), pk.counts.data_ptr(), st["pk_counts"].numel() * 4)]
-                    self._copy_segments(there, table)                                   # -> the host-side entropy coder
-                    self._copy_segments(back, table)                                    # <- what the entropy decoder hands back
-                else:
-                    self._copy_segments(there, table)
-                    arena_host[:off].copy_(arena_dev[:off], non_blocking=True)          # -> the host-side entropy coder
-                    arena_dev[:off].copy_(arena_host[:off], non_blocking=True)          # <- what the entropy decoder hands back
-                    self._copy_segments(back, table)
-                    enc.counts.copy_(st["counts"], non_blocking=True)
-                    pk.counts.copy_(st["pk_counts"], non_blocking=True)
-                self.unpack(pk, G, H, W, space, qrange, brange, instance=slot)
-                rgb = self.decode(enc.coef, enc.leaves, enc.counts, G, H, W, space, qrange, brange, instance=slot, out=out_kind)
-                host_out[job["f"]:job["f"] + G].copy_(rgb, non_blocking=True)
-                job["ev2"] = torch.cuda.Event()
-                job["ev2"].record(stream)
-            job["phase_b"] = True
-            return h2d + off + 2 * st["counts"].numel() * 4, d2h + off + rgb.numel() * rgb.element_size()
-        # raw int32 streams (packed=False), or a plane whose coefficients do not fit int16: per-range copies
-        with torch.cuda.stream(stream):
-            use_pk = [[pk is not None and pkc[b, l, 2] == 0 for l in range(3)] for b in range(G)]
-            for b in range(G):
+                self._copy_segments(there)
+                arena_host[:off].copy_(arena_dev[:off], non_blocking=True)          # -> the host-side entropy coder
+                arena_dev[:off].copy_(arena_host[:off], non_blocking=True)          # <- what the entropy decoder hands back
+                self._copy_segments(back)
+                enc.counts.copy_(st.counts, non_blocking=True)
+                pk.counts.copy_(st.pk_counts, non_blocking=True)
+                self.unpack(pk, 1, H, W, space, qrange, brange, instance=slot)
+                h2d += off + 2 * st.counts.numel() * 4
+                d2h += off
+            else:
+                # raw int32 streams (packed=False, or a plane whose coefficients do not fit int16): per-range copies
                 for l in range(3):
-                    nl, ns, nc = (int(counts[b, l, k]) for k in range(3))
-                    if use_pk[b][l]:                                  # packed: mask words + int16 non-zeros
-                        nnz, nw = int(pkc[b, l, 0]), int(pkc[b, l, 3])
-                        st["mask"][l][b, :nw].copy_(pk.mask[l][b, :nw], non_blocking=True)
-                        st["vals"][l][b, :nnz].copy_(pk.vals[l][b, :nnz], non_blocking=True)
-                        d2h += nw * 4 + nnz * 2
-                    else:
-                        st["coef"][l][b, :nc].copy_(enc.coef[l][b, :nc], non_blocking=True)
-                        d2h += nc * 4
-                    st["leaves"][l][b, :nl].copy_(enc.leaves[l][b, :nl], non_blocking=True)
-                    st["states"][l][b, :ns].copy_(enc.states[l][b, :ns], non_blocking=True)
-                    d2h += nl * 16 + ns
-            any_packed = any(any(r) for r in use_pk)
-            for b in range(G):
+                    nl, ns, nc = (int(counts[l, i]) for i in range(3))
+                    st.coef[l][:nc].copy_(enc.coef[l][0, :nc], non_blocking=True)
+                    st.leaves[l][:nl].copy_(enc.leaves[l][0, :nl], non_blocking=True)
+                    st.states[l][:ns].copy_(enc.states[l][0, :ns], non_blocking=True)
+                    d2h += nc * 4 + nl * 16 + ns
                 for l in range(3):
-                    nl, nc = int(counts[b, l, 0]), int(counts[b, l, 2])
-                    if use_pk[b][l]:
-                        nnz, nw = int(pkc[b, l, 0]), int(pkc[b, l, 3])
-                        pk.mask[l][b, :nw].copy_(st["mask"][l][b, :nw], non_blocking=True)
-                        pk.vals[l][b, :nnz].copy_(st["vals"][l][b, :nnz], non_blocking=True)
-                        h2d += nw * 4 + nnz * 2
-                    else:
-                        enc.coef[l][b, :nc].copy_(st["coef"][l][b, :nc], non_blocking=True)
-                        h2d += nc * 4
-                    enc.leaves[l][b, :nl].copy_(st["leaves"][l][b, :nl], non_blocking=True)
-                    h2d += nl * 16
-            enc.counts.copy_(st["counts"], non_blocking=True)
-            if any_packed:
-                # mixed: keep the int32 planes aside, expand the packed ones around them
-                keep = {(b, l): enc.coef[l][b].clone() for b in range(G) for l in range(3) if not use_pk[b][l]}
-                pk.counts.copy_(st["pk_counts"], non_blocking=True)
-                h2d += st["pk_counts"].numel() * 4
-                self.unpack(pk, G, H, W, space, qrange, brange, instance=slot)
-                for (b, l), t in keep.items():
-                    enc.coef[l][b].copy_(t)
-            rgb = self.decode(enc.coef, enc.leaves, enc.counts, G, H, W, space, qrange, brange, instance=slot, out=out_kind)
-            host_out[job["f"]:job["f"] + G].copy_(rgb, non_blocking=True)
+                    nl, nc = int(counts[l, 0]), int(counts[l, 2])
+                    enc.coef[l][0, :nc].copy_(st.coef[l][:nc], non_blocking=True)
+                    enc.leaves[l][0, :nl].copy_(st.leaves[l][:nl], non_blocking=True)
+                    h2d += nc * 4 + nl * 16
+                enc.counts.copy_(st.counts, non_blocking=True)
+            rgb = self.decode(enc.coef, enc.leaves, enc.counts, 1, H, W, space, qrange, brange, instance=slot, out=out_kind)
+            host_out[job.frame:job.frame + 1].copy_(rgb, non_blocking=True)
             d2h += rgb.numel() * rgb.element_size()
-            job["ev2"] = torch.cuda.Event()
-            job["ev2"].record(stream)
-        job["phase_b"] = True
+            job.decoded = torch.cuda.Event()
+            job.decoded.record()
         return h2d, d2h
 
-    def _finish_job(self, job):
-        if not job["done"]:
-            if not job["phase_b"]:
-                raise RuntimeError("pipeline order error")
-            t0 = time.perf_counter()
-            job["ev2"].synchronize()
-            self.pipeline_host_wait_s += time.perf_counter() - t0
-            job["done"] = True
+    def _wait_decoded(self, job: _Job):
+        t0 = time.perf_counter()
+        job.decoded.synchronize()
+        self.pipeline_host_wait_s += time.perf_counter() - t0
 
     def decode_encoded(self, enc: EncodedBatch, space, qrange, brange, out: str = "f32"):
         B, H, W = enc.shape

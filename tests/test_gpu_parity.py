@@ -574,19 +574,18 @@ def test_tensor_core_dct_parity(codec):
     assert err[False] <= 3e-6 and err[True] <= 3e-6
 
 
-@pytest.mark.parametrize("zero_copy", [False, True])
-@pytest.mark.parametrize("slots,threads,lag,G", [(3, 1, 2, 1), (3, 2, 2, 1), (8, 2, 3, 2), (4, 4, 3, 1), (3, 1, 2, 3), (2, 1, 1, 6)])
-def test_host_pipelined_roundtrip_matches_device_path(codec, slots, threads, lag, G, zero_copy):
+@pytest.mark.parametrize("packed", [True, False])
+@pytest.mark.parametrize("slots,lag", [(3, 2), (8, 3), (4, 3), (2, 1), (2, 3), (1, 2)])
+def test_host_pipelined_roundtrip_matches_device_path(codec, slots, lag, packed):
     """the host-buffer API (bench.py's e2e leg) returns the same pixels as the device-resident path, whatever the number of
-    stream slots and of host threads driving them"""
+    stream slots (12 jobs: every slot is reused) and the lag, requested lags above slots - 1 included"""
     import torch
     H, W = 270, 480
     frames = np.stack([synth(H, W, seed=s) for s in range(6)])
     space, q, b = "YCbCr", (30, 95), (4, 64)
     host_in = torch.from_numpy(frames).pin_memory()
     host_out = torch.zeros_like(host_in).pin_memory()
-    h2d, d2h = codec.roundtrip_host_pipelined(host_in, host_out, space, q, b, slots=slots, repeat=2, lag=lag, threads=threads, frames_per_job=G,
-                                                  zero_copy=zero_copy)
+    h2d, d2h = codec.roundtrip_host_pipelined(host_in, host_out, space, q, b, slots=slots, repeat=2, lag=lag, packed=packed)
     dev = codec.decode_encoded(codec.encode(host_in.cuda(), space, q, b), space, q, b).cpu()
     assert torch.equal(dev, host_out)
     assert h2d > 2 * frames.nbytes and d2h > 2 * frames.nbytes
@@ -712,6 +711,94 @@ def test_packed_coefficient_streams(codec):
     h1, d1 = codec.roundtrip_host_pipelined(host_in, a, space, q, b, slots=3, repeat=2, lag=2, packed=True)
     h2, d2 = codec.roundtrip_host_pipelined(host_in, c, space, q, b, slots=3, repeat=2, lag=2, packed=False)
     assert torch.equal(a, c) and h1 < 0.7 * h2 and d1 < 0.7 * d2
+
+
+@pytest.fixture
+def overflow_frames(codec):
+    """codec.encode, wrapped: after the real call, the first coefficient of plane 0 becomes 65536 + k (k its value) in every
+    call whose index modulo `period` is in `frames` -- a plane that does not fit int16, whose int16 truncation is k"""
+    real = codec.encode
+    sel = dict(frames=set(), period=1, calls=0)
+
+    def encode(*args, **kw):
+        enc = real(*args, **kw)
+        if sel["calls"] % sel["period"] in sel["frames"]:
+            enc.coef[0][0, :1] += 65536
+        sel["calls"] += 1
+        return enc
+
+    codec.encode = encode
+    try:
+        yield sel
+    finally:
+        del codec.encode
+
+
+def test_host_pipelined_int16_overflow_travels_as_int32(codec, overflow_frames):
+    """a packed job in which a plane overflows int16 travels whole as raw int32 streams, the other jobs stay packed: the
+    pixels are those of packed=False, the bytes lie between an all-packed and an all-int32 run"""
+    import torch
+    H, W = 270, 480
+    space, q, b = "YCbCr", (30, 95), (4, 64)
+    F = 5
+    host_in = torch.from_numpy(np.stack([(synth(H, W, seed=s) * 255).astype(np.uint8) for s in range(F)])).pin_memory()
+    clean, mixed, raw = (torch.empty_like(host_in).pin_memory() for _ in range(3))
+
+    def run(out, packed):
+        overflow_frames["calls"] = 0
+        return codec.roundtrip_host_pipelined(host_in, out, space, q, b, slots=3, repeat=2, lag=2, packed=packed)
+
+    h_pk, d_pk = run(clean, True)
+    overflow_frames.update(frames={1, 3}, period=F)
+    h_mix, d_mix = run(mixed, True)
+    h_raw, d_raw = run(raw, False)
+    assert torch.equal(mixed, raw)
+    for f in range(F):                                         # the added 65536 reaches the pixels of the frames it was added to
+        assert torch.equal(mixed[f], clean[f]) == (f not in (1, 3)), f
+    assert h_pk < h_mix < h_raw and d_pk < d_mix < d_raw
+
+
+def test_copy_segments_device_table(codec):
+    """aeaj_copy_segments with more than the 64 ranges that travel in the kernel parameters: the table goes through the
+    caller's device scratch.  80 ranges of mixed sizes and alignments gathered into one arena and scattered back, bit for
+    bit; without the scratch table the call fails instead of launching."""
+    import ctypes as C
+    import torch
+    from aeaj import native
+    rng = np.random.default_rng(7)
+    sizes = [0, 0, 1, 1, 2, 3, 4, 7, 15, 16, 17, 31, 32, 33, 64, 100, 255, 256, 4096, 65539, 300_000] + [int(n) for n in rng.integers(1, 5000, 59)]
+    src_shift, arena_shift = (0, 4, 1, 8), (0, 4, 3)           # 16-byte, 4-byte and odd starts, in changing combinations
+    spos = apos = 0
+    ranges = []
+    for i, n in enumerate(sizes):
+        so, ao = spos + src_shift[i % 4], apos + arena_shift[i % 3]
+        ranges.append((so, ao, n))
+        spos, apos = (so + n + 31) & ~15, (ao + n + 31) & ~15
+    src_h = rng.integers(0, 256, spos, dtype=np.uint8)
+    src = torch.from_numpy(src_h).cuda()
+    dst = torch.zeros_like(src)
+    arena = torch.zeros(apos, dtype=torch.uint8, device="cuda")
+    table = torch.empty(len(ranges) * C.sizeof(native.Segment), dtype=torch.uint8, device="cuda")
+    stream = torch.cuda.current_stream().cuda_stream
+
+    def segs(pairs):
+        arr = (native.Segment * len(pairs))()
+        for k, (s, d, n) in enumerate(pairs):
+            arr[k].src, arr[k].dst, arr[k].bytes = s, d, n
+        return arr
+
+    gather = segs([(src.data_ptr() + so, arena.data_ptr() + ao, n) for so, ao, n in ranges] + [(None, None, 0)])
+    scatter = segs([(arena.data_ptr() + ao, dst.data_ptr() + so, n) for so, ao, n in ranges])
+    with pytest.raises(native.AeajError, match="more than 64 ranges"):
+        native.check(codec.lib.aeaj_copy_segments(gather, len(gather), None, stream), "aeaj_copy_segments")
+    native.check(codec.lib.aeaj_copy_segments(gather, len(gather), table.data_ptr(), stream), "aeaj_copy_segments")
+    native.check(codec.lib.aeaj_copy_segments(scatter, len(scatter), table.data_ptr(), stream), "aeaj_copy_segments")
+    want_arena, want_dst = np.zeros(apos, dtype=np.uint8), np.zeros(spos, dtype=np.uint8)
+    for so, ao, n in ranges:
+        want_arena[ao:ao + n] = src_h[so:so + n]
+        want_dst[so:so + n] = src_h[so:so + n]
+    assert np.array_equal(arena.cpu().numpy(), want_arena)
+    assert np.array_equal(dst.cpu().numpy(), want_dst)
 
 
 def test_cuda_graph_roundtrip_equals_eager(codec):

@@ -1,4 +1,4 @@
-"""measurement tool: the host-buffer pipeline (bench.py's e2e leg) over slots / lag / host threads, plus the pieces on their own:
+"""measurement tool: the host-buffer pipeline (bench.py's e2e leg) over slots / lag, plus the pieces on their own:
 pure copies through the same pinned buffers, and the device work of one frame.  usage: python tools/e2e_sweep.py [frames]"""
 import sys, time, torch, numpy as np
 sys.path.insert(0, 'adaptive-edge-aware-jpeg_b200'); sys.path.insert(0, 'tests')
@@ -23,9 +23,7 @@ def run(**kw):
     print(f"{kw}: {dt * 1e3 / F:.3f} ms/frame  {mp / dt:.0f} MP/s  {h2d / 4 / dt / 1e9:.1f} + {d2h / 4 / dt / 1e9:.1f} GB/s;  host blocked on the device "
           f"{c.pipeline_host_wait_s / 4 * 1e3 / F:.3f} ms/frame", flush=True)
 
-for kw in (dict(slots=8, lag=3, zero_copy=False), dict(slots=8, lag=3, zero_copy=True), dict(slots=12, lag=4, zero_copy=True),
-           dict(slots=6, lag=2, zero_copy=True), dict(slots=8, lag=3, zero_copy=True, threads=2), dict(slots=8, lag=3, zero_copy=False, frames_per_job=2),
-           dict(slots=8, lag=3, zero_copy=True, frames_per_job=2)):
+for kw in (dict(slots=8, lag=3), dict(slots=12, lag=4), dict(slots=6, lag=2), dict(slots=16, lag=6)):
     run(**kw)
 
 # pure copies of the same byte counts, both directions at once, 8 streams

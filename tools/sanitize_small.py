@@ -23,8 +23,8 @@ for space, (H, W), b, mask in (("YCbCr", (384, 512), (4, 128), 0xf), ("JzAzBz", 
 c.tensor_dct = 0xa
 fr = torch.from_numpy(np.stack([(synth(270, 480, s) * 255).astype(np.uint8) for s in range(4)])).pin_memory()
 out = torch.empty_like(fr).pin_memory()
-for zc in (False, True):
-    c.roundtrip_host_pipelined(fr, out, "YCbCr", q, (4, 64), slots=3, lag=2, frames_per_job=2, zero_copy=zc)
+for packed in (True, False):
+    c.roundtrip_host_pipelined(fr, out, "YCbCr", q, (4, 64), slots=3, lag=2, packed=packed)
 rgb = torch.from_numpy(synth(1024, 640, 21)).cuda()
 t = TiledCodec(c, emulate=2)
 enc = t.encode(rgb, 1024, 640, "ICtCp", q, (4, 128))
