@@ -10,8 +10,6 @@
 #include <string.h>
 #include "../../include/aeaj.h"
 
-#define AEAJ_MAX_PLANES_INLINE 0
-
 // ---------------------------------------------------------------------------------------------
 // error plumbing
 // ---------------------------------------------------------------------------------------------
@@ -158,11 +156,6 @@ struct aeaj_handle {
     int32_t* tc_izz_all_dev;
     float* dct_tc_tiles_dev;      // [size class 16..128][fwd, inv][Ah | Al]: block-diagonal DCT matrices for the tcgen05 path
     int* tc_err_dev;              // set by the tcgen05 kernel if a barrier wait timed out
-    // device scratch for single-plane stage calls
-    struct PlaneDesc* stage_plane_dev;
-    long long* stage_class_off_dev;   // [18]: offsets, capacities
-    int* stage_tile_base_dev;         // [1]
-    uint8_t** stage_outs_dev;         // [1]
 };
 
 // device-side description of every plane of a batch; lives in the plan's device memory
@@ -194,6 +187,7 @@ struct PlaneDesc {
     int zigzag;              // 1: coefficient streams are stored zigzag-ordered per block (the .ajpg layout)
     uint8_t* packed_states;  // optional: 2-bit MSB-first packing of `states` (jpeg.py:563-571)
     int64_t cap_leaves, cap_states, cap_coef;
+    uint8_t* tap_edge;       // optional: the final edge map as uint8 {0,1} [h][w] (encode taps, Canny stage calls)
 };
 
 struct ClassEntry { int x, y, plane, coef_off; };
@@ -235,7 +229,7 @@ struct PackPlane {
     int64_t cap_coef;         // capacity of the stream buffers
 };
 size_t aeaj_pack_scratch_ints(int64_t cap_coef);
-int launch_pack(const PackPlane* planes_host, PackPlane* planes_dev, int nplanes, int64_t max_cap_coef, int unpack, cudaStream_t st);
+int launch_pack(const PackPlane* planes_dev, int nplanes, int64_t max_cap_coef, int unpack, cudaStream_t st);
 
 // one plane's zlib stream (deflate.cu, deflate_core.h)
 struct DeflatePlane {
@@ -252,9 +246,8 @@ struct DeflatePlane {
     uint32_t* chunk_adler;    // scratch [chunks]
     int64_t* chunk_off;       // scratch [chunks]
 };
-size_t deflate_chunk_scratch_bytes();
 int aeaj_deflate_init();
-int launch_deflate(const DeflatePlane* planes_host, DeflatePlane* planes_dev, int nplanes, int max_chunks, cudaStream_t st);
+int launch_deflate(const DeflatePlane* planes_dev, int nplanes, int max_chunks, cudaStream_t st);
 
 // one plane's zlib stream -> its coefficient buffer (inflate.cu, inflate_core.h)
 struct InflatePlane {
@@ -278,7 +271,7 @@ struct InflateArgs {
     IfSeg* segs;              // [cap_segs]
     int32_t* map;             // [in_bytes / 4 + 1]: input position >> 2 -> candidate index (-1: list full)
 };
-int launch_inflate(const InflatePlane* planes_host, InflatePlane* planes_dev, const InflateArgs& a, int sm_count, cudaStream_t st);
+int launch_inflate(const InflatePlane* planes_dev, const InflateArgs& a, int sm_count, cudaStream_t st);
 
 // kernels' host launchers (defined in the .cu files)
 int aeaj_canny_init(aeaj_handle* h);
@@ -312,8 +305,7 @@ int hysteresis_tiles(PlaneDesc* planes_host, int nplanes, int* ring_cap);
 int hysteresis_ctrl_ints();
 int launch_hysteresis(aeaj_handle* h, const PlaneDesc* planes_dev, const PlaneDesc* planes_host, int nplanes, int ntiles, int ring_cap,
                       int* flags, int* ring, int* ctrl, int* status, cudaStream_t st);
-int launch_bitmap_to_u8(const PlaneDesc* planes_dev, const PlaneDesc* planes_host, int nplanes,
-                        uint8_t* const* outs_dev, cudaStream_t st);
+int launch_bitmap_to_u8(const PlaneDesc* planes_dev, const PlaneDesc* planes_host, int nplanes, cudaStream_t st);
 int launch_u8_to_bitmap(const uint8_t* edge, int h, int w, uint32_t* bits, cudaStream_t st);
 
 int launch_quadtree(const PlaneDesc* planes_dev, const PlaneDesc* planes_host, int nplanes, int min_size, int max_size,

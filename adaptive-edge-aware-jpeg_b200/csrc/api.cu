@@ -37,6 +37,36 @@ struct Bump {
     size_t used() const { return (off + 255) & ~(size_t)255; }
 };
 
+// device copy of a host descriptor array (one per kernel family of a plan).  push() uploads only when the bytes or the
+// stream differ from the last push: steady-state calls issue no host-to-device copy at all, which also makes them
+// capturable in a CUDA graph.  The stream is part of the check because the last upload is ordered on its own stream only.
+template <typename T> struct DescTable {
+    static_assert(std::is_trivially_copyable<T>::value, "descriptors are compared and uploaded as bytes");
+    T* dev = nullptr;
+    size_t cap = 0;
+    std::vector<T> pushed;                 // what `dev` holds
+    cudaStream_t stream = nullptr;         // the stream of that upload
+    DescTable() = default;
+    DescTable(const DescTable&) = delete;
+    DescTable& operator=(const DescTable&) = delete;
+    ~DescTable() { cudaFree(dev); }
+    // `out` receives the device array that holds `host` once `st` reaches this point
+    int push(const std::vector<T>& host, cudaStream_t st, T*& out) {
+        if (host.size() > cap) {
+            cudaFree(dev); dev = nullptr; cap = 0; pushed.clear();
+            AEAJ_CUDA(cudaMalloc(&dev, sizeof(T) * host.size()));
+            cap = host.size();
+        }
+        out = dev;
+        if (stream == st && pushed.size() == host.size() && memcmp(pushed.data(), host.data(), sizeof(T) * host.size()) == 0) return 0;
+        pushed.clear();                    // a failed upload leaves nothing that could be mistaken for the device contents
+        AEAJ_CUDA(cudaMemcpyAsync(dev, host.data(), sizeof(T) * host.size(), cudaMemcpyHostToDevice, st));
+        pushed = host; stream = st;
+        return 0;
+    }
+    void forget() { pushed.clear(); }      // the next push uploads
+};
+
 static int64_t cap_leaves_of(int h, int w, int mn) { return (int64_t)aeaj_cdiv(h, mn) * aeaj_cdiv(w, mn); }
 static int64_t cap_states_of(int h, int w, int mn, int root) {
     int64_t n = 1;
@@ -77,7 +107,11 @@ static void carve_plane_scratch(Bump& b, PlaneDesc& P, bool canny, bool qt) {
     }
 }
 
-struct ClassGeom { int64_t off[9], cap[9], total; };
+struct ClassGeom {
+    int64_t off[9], cap[9], total;
+    // the class-offset table the quadtree / bucketing kernels read: offsets, then capacities
+    void table(long long (&t)[18]) const { for (int k = 0; k < 9; k++) { t[k] = off[k]; t[9 + k] = cap[k]; } }
+};
 static void class_geom(const PlaneDesc* P, int nplanes, int lg_min, int lg_max, ClassGeom& g) {
     g.total = 0;
     for (int k = 0; k < 9; k++) { g.off[k] = 0; g.cap[k] = 0; }
@@ -123,11 +157,6 @@ extern "C" int aeaj_create(int device, aeaj_handle** out) {
     rc = aeaj_deflate_init();
     if (rc) { free(h); return rc; }
     AEAJ_CUDA(cudaMalloc(&h->srgb_lut_dev, 256 * sizeof(float)));
-    AEAJ_CUDA(cudaMalloc(&h->stage_plane_dev, sizeof(PlaneDesc)));
-    AEAJ_CUDA(cudaMalloc(&h->stage_class_off_dev, 18 * sizeof(long long)));
-    AEAJ_CUDA(cudaMalloc(&h->stage_tile_base_dev, sizeof(int)));
-    AEAJ_CUDA(cudaMalloc(&h->stage_outs_dev, sizeof(uint8_t*)));
-    AEAJ_CUDA(cudaMemset(h->stage_tile_base_dev, 0, sizeof(int)));
     *out = h;
     return 0;
 }
@@ -135,8 +164,7 @@ extern "C" int aeaj_create(int device, aeaj_handle** out) {
 extern "C" int aeaj_destroy(aeaj_handle* h) {
     if (!h) return 0;
     cudaSetDevice(h->device);
-    cudaFree(h->pq_tabs_dev); cudaFree(h->srgb_lut_dev); cudaFree(h->dct_all_dev); cudaFree(h->dct_half_all_dev); cudaFree(h->zz_all_dev); cudaFree(h->izz256_dev); cudaFree(h->dct_tc_tiles_dev); cudaFree(h->tc_izz_all_dev); cudaFree(h->tc_err_dev); cudaFree(h->stage_plane_dev);
-    cudaFree(h->stage_class_off_dev); cudaFree(h->stage_tile_base_dev); cudaFree(h->stage_outs_dev);
+    cudaFree(h->pq_tabs_dev); cudaFree(h->srgb_lut_dev); cudaFree(h->dct_all_dev); cudaFree(h->dct_half_all_dev); cudaFree(h->zz_all_dev); cudaFree(h->izz256_dev); cudaFree(h->dct_tc_tiles_dev); cudaFree(h->tc_izz_all_dev); cudaFree(h->tc_err_dev);
     free(h);
     return 0;
 }
@@ -208,8 +236,11 @@ extern "C" int aeaj_cast_u8(aeaj_handle* h, const float* layer, uint8_t* out, si
 }
 
 // ---- single-plane stage workspace -------------------------------------------------------------
+// The call's descriptor and class-offset table live in the workspace too, so that calls on separate workspaces are independent.
 struct StageWs {
     PlaneDesc P;
+    PlaneDesc* desc;                      // device copy of P
+    long long* class_off;                 // device ClassGeom::table (quadtree / DCT calls)
     uint8_t* u8a; uint8_t* u8b;
     int* flags; int* ring; int* ctrl; int* status;
     ClassEntry* class_lists; int* class_counts;
@@ -231,9 +262,11 @@ static void stage_ws(void* ws, int h, int w, int mn, int mx, StageWs& S) {
     S.ctrl = b.take<int>(hysteresis_ctrl_ints());
     S.status = b.take<int>(4);
     S.class_counts = b.take<int>(16);
+    S.desc = b.take<PlaneDesc>(1);
     if (mx > 0) {
         class_geom(&S.P, 1, ilog2i(mn), ilog2i(mx), S.cg);
         S.class_lists = b.take<ClassEntry>((size_t)S.cg.total);
+        S.class_off = b.take<long long>(18);
         if (mx >= 256) S.scratch256 = b.take<float>(aeaj_dct256_scratch_floats());
     }
     S.bytes = b.used();
@@ -244,38 +277,43 @@ extern "C" size_t aeaj_stage_workspace_bytes(int h, int w, int min_size, int max
     stage_ws(nullptr, h, w, min_size, max_size, S);
     return S.bytes + 256;
 }
-static int push_stage_plane(aeaj_handle* h, const PlaneDesc& P, cudaStream_t st) {
-    AEAJ_CUDA(cudaMemcpyAsync(h->stage_plane_dev, &P, sizeof(PlaneDesc), cudaMemcpyHostToDevice, st));
+// once per call, after S.P is complete
+static int push_stage(const StageWs& S, cudaStream_t st) {
+    AEAJ_CUDA(cudaMemcpyAsync(S.desc, &S.P, sizeof(PlaneDesc), cudaMemcpyHostToDevice, st));
+    if (S.class_off) {
+        long long t[18]; S.cg.table(t);
+        AEAJ_CUDA(cudaMemcpyAsync(S.class_off, t, sizeof t, cudaMemcpyHostToDevice, st));
+    }
     return 0;
 }
 
-static int run_clahe(aeaj_handle* hd, StageWs& S, cudaStream_t st) {
+static int run_clahe(StageWs& S, cudaStream_t st) {
     AEAJ_CUDA(cudaMemsetAsync(S.P.clahe_hist, 0, 16 * 256 * sizeof(uint32_t), st));
-    int rc = launch_clahe_hist(hd->stage_plane_dev, &S.P, 1, st); if (rc) return rc;
-    return launch_clahe_lut(hd->stage_plane_dev, 1, PeerSet{1, 0, {0}}, st);
+    int rc = launch_clahe_hist(S.desc, &S.P, 1, st); if (rc) return rc;
+    return launch_clahe_lut(S.desc, 1, PeerSet{1, 0, {0}}, st);
 }
 
 extern "C" int aeaj_clahe(aeaj_handle* hd, const uint8_t* src, int h, int w, uint8_t* dst, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && src && dst && ws && h > 0 && w > 0, "aeaj_clahe: bad arguments");
     StageWs S; stage_ws(ws, h, w, 0, 0, S);
     S.P.u8a = (uint8_t*)src; S.P.u8b = dst;
-    int rc = push_stage_plane(hd, S.P, ST(stream)); if (rc) return rc;
-    rc = run_clahe(hd, S, ST(stream)); if (rc) return rc;
-    return launch_prefilter(hd->stage_plane_dev, &S.P, 1, 1, 0, ST(stream));
+    int rc = push_stage(S, ST(stream)); if (rc) return rc;
+    rc = run_clahe(S, ST(stream)); if (rc) return rc;
+    return launch_prefilter(S.desc, &S.P, 1, 1, 0, ST(stream));
 }
-static int prefilter_only(aeaj_handle* hd, const uint8_t* src, int h, int w, uint8_t* dst, void* ws, void* stream, int stages) {
+static int prefilter_only(const uint8_t* src, int h, int w, uint8_t* dst, void* ws, void* stream, int stages) {
     StageWs S; stage_ws(ws, h, w, 0, 0, S);
     S.P.u8a = (uint8_t*)src; S.P.u8b = dst;
-    int rc = push_stage_plane(hd, S.P, ST(stream)); if (rc) return rc;
-    return launch_prefilter(hd->stage_plane_dev, &S.P, 1, stages, 0, ST(stream));
+    int rc = push_stage(S, ST(stream)); if (rc) return rc;
+    return launch_prefilter(S.desc, &S.P, 1, stages, 0, ST(stream));
 }
 extern "C" int aeaj_gauss3(aeaj_handle* hd, const uint8_t* src, int h, int w, uint8_t* dst, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && src && dst && ws && h > 0 && w > 0, "aeaj_gauss3: bad arguments");
-    return prefilter_only(hd, src, h, w, dst, ws, stream, 2);
+    return prefilter_only(src, h, w, dst, ws, stream, 2);
 }
 extern "C" int aeaj_bilateral5(aeaj_handle* hd, const uint8_t* src, int h, int w, uint8_t* dst, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && src && dst && ws && h > 0 && w > 0, "aeaj_bilateral5: bad arguments");
-    return prefilter_only(hd, src, h, w, dst, ws, stream, 4);
+    return prefilter_only(src, h, w, dst, ws, stream, 4);
 }
 extern "C" int aeaj_percentile_thresholds(aeaj_handle* hd, const uint8_t* src, int h, int w, double* thr, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && src && thr && ws && h > 0 && w > 0, "aeaj_percentile_thresholds: bad arguments");
@@ -283,42 +321,39 @@ extern "C" int aeaj_percentile_thresholds(aeaj_handle* hd, const uint8_t* src, i
     S.P.thr_d = thr;
     cudaStream_t st = ST(stream);
     AEAJ_CUDA(cudaMemsetAsync(S.P.hist, 0, 256 * sizeof(uint32_t), st));
-    int rc = push_stage_plane(hd, S.P, st); if (rc) return rc;
+    int rc = push_stage(S, st); if (rc) return rc;
     rc = launch_hist_u8(src, (size_t)h * w, S.P.hist, st); if (rc) return rc;
-    return launch_thresholds(hd->stage_plane_dev, 1, PeerSet{1, 0, {0}}, st);
+    return launch_thresholds(S.desc, 1, PeerSet{1, 0, {0}}, st);
 }
 
-static int run_nms_hysteresis(aeaj_handle* hd, StageWs& S, uint8_t* edge, cudaStream_t st) {
-    int rc = launch_canny_nms(hd->stage_plane_dev, &S.P, 1, st); if (rc) return rc;
-    rc = launch_hysteresis(hd, hd->stage_plane_dev, &S.P, 1, S.ntiles, S.ring_cap, S.flags, S.ring, S.ctrl, S.status, st);
+// the descriptor's tap_edge receives the edge map
+static int run_nms_hysteresis(aeaj_handle* hd, StageWs& S, cudaStream_t st) {
+    int rc = launch_canny_nms(S.desc, &S.P, 1, st); if (rc) return rc;
+    rc = launch_hysteresis(hd, S.desc, &S.P, 1, S.ntiles, S.ring_cap, S.flags, S.ring, S.ctrl, S.status, st);
     if (rc) return rc;
-    if (edge) {
-        AEAJ_CUDA(cudaMemcpyAsync(hd->stage_outs_dev, &edge, sizeof(uint8_t*), cudaMemcpyHostToDevice, st));
-        rc = launch_bitmap_to_u8(hd->stage_plane_dev, &S.P, 1, hd->stage_outs_dev, st);
-    }
-    return rc;
+    return launch_bitmap_to_u8(S.desc, &S.P, 1, st);
 }
 extern "C" int aeaj_canny_u8(aeaj_handle* hd, const uint8_t* src, int h, int w, const double* thr, uint8_t* edge, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && src && thr && edge && ws && h > 0 && w > 0, "aeaj_canny_u8: bad arguments");
     StageWs S; stage_ws(ws, h, w, 0, 0, S);
-    S.P.u8b = (uint8_t*)src;
+    S.P.u8b = (uint8_t*)src; S.P.tap_edge = edge;
     cudaStream_t st = ST(stream);
-    int rc = push_stage_plane(hd, S.P, st); if (rc) return rc;
+    int rc = push_stage(S, st); if (rc) return rc;
     rc = launch_thresholds_from_double(thr, S.P.thr, st); if (rc) return rc;
-    return run_nms_hysteresis(hd, S, edge, st);
+    return run_nms_hysteresis(hd, S, st);
 }
 extern "C" int aeaj_canny(aeaj_handle* hd, const float* layer, int h, int w, uint8_t* edge, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && layer && edge && ws && h > 0 && w > 0, "aeaj_canny: bad arguments");
     StageWs S; stage_ws(ws, h, w, 0, 0, S);
-    S.P.u8a = S.u8a; S.P.u8b = S.u8b;
+    S.P.u8a = S.u8a; S.P.u8b = S.u8b; S.P.tap_edge = edge;
     cudaStream_t st = ST(stream);
-    int rc = push_stage_plane(hd, S.P, st); if (rc) return rc;
+    int rc = push_stage(S, st); if (rc) return rc;
     rc = launch_cast_u8(layer, S.u8a, (size_t)h * w, st); if (rc) return rc;
-    rc = run_clahe(hd, S, st); if (rc) return rc;
+    rc = run_clahe(S, st); if (rc) return rc;
     AEAJ_CUDA(cudaMemsetAsync(S.P.hist, 0, 256 * sizeof(uint32_t), st));
-    rc = launch_prefilter(hd->stage_plane_dev, &S.P, 1, 7, 1, st); if (rc) return rc;
-    rc = launch_thresholds(hd->stage_plane_dev, 1, PeerSet{1, 0, {0}}, st); if (rc) return rc;
-    return run_nms_hysteresis(hd, S, edge, st);
+    rc = launch_prefilter(S.desc, &S.P, 1, 7, 1, st); if (rc) return rc;
+    rc = launch_thresholds(S.desc, 1, PeerSet{1, 0, {0}}, st); if (rc) return rc;
+    return run_nms_hysteresis(hd, S, st);
 }
 
 extern "C" int aeaj_quadtree_caps(int h, int w, int mn, int mx, int64_t* cl, int64_t* cs, int64_t* cc, int* root) {
@@ -341,12 +376,10 @@ extern "C" int aeaj_quadtree(aeaj_handle* hd, const uint8_t* edge, int h, int w,
     StageWs S; stage_ws(ws, h, w, mn, mx, S);
     S.P.leaves = leaves; S.P.states = states; S.P.counts = counts;
     cudaStream_t st = ST(stream);
-    rc = push_stage_plane(hd, S.P, st); if (rc) return rc;
-    long long off[18]; for (int k = 0; k < 9; k++) { off[k] = S.cg.off[k]; off[9 + k] = S.cg.cap[k]; }
-    AEAJ_CUDA(cudaMemcpyAsync(hd->stage_class_off_dev, off, sizeof off, cudaMemcpyHostToDevice, st));
+    rc = push_stage(S, st); if (rc) return rc;
     AEAJ_CUDA(cudaMemsetAsync(S.class_counts, 0, 16 * sizeof(int), st));
     rc = launch_u8_to_bitmap(edge, h, w, S.P.strong, st); if (rc) return rc;
-    return launch_quadtree(hd->stage_plane_dev, &S.P, 1, mn, mx, S.class_lists, S.class_counts, hd->stage_class_off_dev, st, nullptr);
+    return launch_quadtree(S.desc, &S.P, 1, mn, mx, S.class_lists, S.class_counts, S.class_off, st, nullptr);
 }
 
 static int stage_blocks(aeaj_handle* hd, bool inverse, float* layer, int h, int w, float mid, float scale, const int32_t* leaves,
@@ -356,15 +389,12 @@ static int stage_blocks(aeaj_handle* hd, bool inverse, float* layer, int h, int 
     S.P.layer_f32 = layer; S.P.mid = mid; S.P.scale = scale;
     S.P.leaves = (int32_t*)leaves; S.P.counts = (int32_t*)counts; S.P.coef = coef;
     for (int k = 0; k < 9; k++) S.P.qtab[k] = qtab[k];
-    rc = push_stage_plane(hd, S.P, st); if (rc) return rc;
-    long long off[18]; for (int k = 0; k < 9; k++) { off[k] = S.cg.off[k]; off[9 + k] = S.cg.cap[k]; }
-    AEAJ_CUDA(cudaMemcpyAsync(hd->stage_class_off_dev, off, sizeof off, cudaMemcpyHostToDevice, st));
-    AEAJ_CUDA(cudaMemsetAsync(S.class_counts, 0, 16 * sizeof(int), st));
     S.P.cap_leaves = INT32_MAX;                        // the stage API trusts counts[0] (the caller sized the leaf list)
-    rc = push_stage_plane(hd, S.P, st); if (rc) return rc;
-    rc = launch_bucket_leaves(hd->stage_plane_dev, &S.P, 1, S.class_lists, S.class_counts, hd->stage_class_off_dev, ilog2i(mn), ilog2i(mx), st); if (rc) return rc;
-    if (inverse) return launch_dequant_idct(hd, hd->stage_plane_dev, S.class_lists, S.class_counts, S.cg.off, S.cg.cap, ilog2i(mn), ilog2i(mx), st, nullptr, nullptr, nullptr, 0, S.scratch256);
-    return launch_dct_quant(hd, hd->stage_plane_dev, S.class_lists, S.class_counts, S.cg.off, S.cg.cap, ilog2i(mn), ilog2i(mx), st, nullptr, nullptr, nullptr, 0, S.scratch256);
+    rc = push_stage(S, st); if (rc) return rc;
+    AEAJ_CUDA(cudaMemsetAsync(S.class_counts, 0, 16 * sizeof(int), st));
+    rc = launch_bucket_leaves(S.desc, &S.P, 1, S.class_lists, S.class_counts, S.class_off, ilog2i(mn), ilog2i(mx), st); if (rc) return rc;
+    if (inverse) return launch_dequant_idct(hd, S.desc, S.class_lists, S.class_counts, S.cg.off, S.cg.cap, ilog2i(mn), ilog2i(mx), st, nullptr, nullptr, nullptr, 0, S.scratch256);
+    return launch_dct_quant(hd, S.desc, S.class_lists, S.class_counts, S.cg.off, S.cg.cap, ilog2i(mn), ilog2i(mx), st, nullptr, nullptr, nullptr, 0, S.scratch256);
 }
 extern "C" int aeaj_dct_quant(aeaj_handle* hd, const float* layer, int h, int w, float mid, float scale, const int32_t* leaves,
                               const int32_t* counts, int mn, int mx, const int32_t* const* qtab, int32_t* coef, void* ws, void* stream) {
@@ -385,10 +415,7 @@ struct aeaj_plan {
     aeaj_plan_info info;
     int nplanes, lg_min, lg_max;
     std::vector<PlaneDesc> planes;       // host copy, index b*3 + l
-    std::vector<PlaneDesc> planes_pushed; // what planes_dev holds (the upload is skipped while nothing changed: steady-state
-                                         // calls issue no host-to-device copy at all, which also makes them CUDA-graph capturable)
-    PlaneDesc* planes_dev;
-    cudaStream_t pushed_stream = 0;
+    DescTable<PlaneDesc> planes_tab;
     int ntiles, ring_cap;
     long long* class_off_dev;
     ClassGeom cg;
@@ -396,17 +423,12 @@ struct aeaj_plan {
     float* qtabf_dev;                    // the same entries as float
     const int32_t* qtab_ptr[2][9];       // device pointers per table (0 luma, 1 chroma) and log2 size
     const float* qtabf_ptr[2][9];
-    uint8_t** outs_dev;                  // tap pointers [nplanes]
     std::vector<PackPlane> pack_planes;  // host copy of the packing descriptors
-    PackPlane* pack_planes_dev;          // [2][nplanes]: the pack and the unpack flavour of the table (they differ in n_coef)
-    std::vector<PackPlane> pack_pushed[2];   // what the device tables hold (upload skipped when unchanged: no per-call pageable copy,
-    cudaStream_t pack_pushed_stream[2] = {nullptr, nullptr};   // which may synchronise the stream and is not capturable)
-    std::vector<DeflatePlane> df_planes, df_pushed;   // deflate descriptors, the same scheme
-    DeflatePlane* df_planes_dev = nullptr;
-    cudaStream_t df_pushed_stream = nullptr;
-    std::vector<InflatePlane> if_planes, if_pushed;   // inflate descriptors, the same scheme
-    InflatePlane* if_planes_dev = nullptr;
-    cudaStream_t if_pushed_stream = nullptr;
+    DescTable<PackPlane> pack_tab, unpack_tab;   // separate tables (they differ in n_coef): alternating calls upload nothing
+    std::vector<DeflatePlane> df_planes;
+    DescTable<DeflatePlane> deflate_tab;
+    std::vector<InflatePlane> if_planes;
+    DescTable<InflatePlane> inflate_tab;
     // one image over several GPUs (peer.cu): the other ranks' workspaces / barrier flags, opened through CUDA IPC by the caller
     PeerSet peers = {1, 0, {0}};
     void* peer_ws[AEAJ_MAX_PEERS] = {nullptr};
@@ -442,8 +464,10 @@ static int sub_ratio(int space, int& rh, int& rw) {
     return AEAJ_EINVAL;
 }
 
-// carve the plan workspace; with ws == nullptr only sizes are computed
-static size_t plan_carve(aeaj_plan* p, void* ws) {
+struct PlanAux { float* full_c1; float* full_c2; int* flags; int* ring; int* ctrl; int* class_counts; ClassEntry* class_lists; float* scratch256;
+                 int* pack_sums[3]; };
+// carve the plan workspace: the plane pointers of p->planes and the call's buffers A; with ws == nullptr only the size
+static size_t plan_carve(aeaj_plan* p, void* ws, PlanAux& A) {
     Bump b(ws);
     const int B = p->info.batch;
     for (int l = 0; l < 3; l++) {
@@ -472,13 +496,6 @@ static size_t plan_carve(aeaj_plan* p, void* ws) {
         size_t ntb = (size_t)P.ntx * P.nty;
         P.tb_tot = b.take<int2>(ntb); P.tb_coef = b.take<int>(ntb); P.tb_base = b.take<int4>(ntb);
     }
-    return b.off;
-}
-
-struct PlanAux { float* full_c1; float* full_c2; int* flags; int* ring; int* ctrl; int* class_counts; ClassEntry* class_lists; float* scratch256;
-                 int* pack_sums[3]; };
-static size_t plan_carve_aux(aeaj_plan* p, void* ws, size_t start, PlanAux& A) {
-    Bump b(ws); b.off = start;
     const size_t HW = (size_t)p->info.height * p->info.width;
     if (p->need_full_chroma) { A.full_c1 = b.take<float>(HW * p->info.batch); A.full_c2 = b.take<float>(HW * p->info.batch); }
     else { A.full_c1 = A.full_c2 = nullptr; }
@@ -527,15 +544,11 @@ extern "C" int aeaj_plan_create(aeaj_handle* h, int batch, int height, int width
     p->need_full_chroma = !((ch * 2 == height && cw * 2 == width && (width % 4) == 0) || (ch == height && cw * 4 == width));
     class_geom(p->planes.data(), p->nplanes, p->lg_min, p->lg_max, p->cg);
     p->ntiles = hysteresis_tiles(p->planes.data(), p->nplanes, &p->ring_cap);
-    size_t s1 = plan_carve(p, nullptr);
     PlanAux A;
-    p->info.workspace_bytes = (int64_t)plan_carve_aux(p, nullptr, s1, A) + 256;
-    AEAJ_CUDA(cudaMalloc(&p->planes_dev, sizeof(PlaneDesc) * p->nplanes));
+    p->info.workspace_bytes = (int64_t)plan_carve(p, nullptr, A) + 256;
     AEAJ_CUDA(cudaMalloc(&p->class_off_dev, sizeof(long long) * 18));
-    AEAJ_CUDA(cudaMalloc(&p->outs_dev, sizeof(uint8_t*) * p->nplanes));
     p->pack_planes.resize(p->nplanes);
-    AEAJ_CUDA(cudaMalloc(&p->pack_planes_dev, sizeof(PackPlane) * p->nplanes * 2));
-    long long off[18]; for (int k = 0; k < 9; k++) { off[k] = p->cg.off[k]; off[9 + k] = p->cg.cap[k]; }
+    long long off[18]; p->cg.table(off);
     AEAJ_CUDA(cudaMemcpy(p->class_off_dev, off, sizeof off, cudaMemcpyHostToDevice));
     p->qtab_dev = nullptr; p->qtabf_dev = nullptr; p->qtab_entries = 0;
     memset(p->qtab_ptr, 0, sizeof p->qtab_ptr);
@@ -548,8 +561,8 @@ extern "C" int aeaj_plan_create(aeaj_handle* h, int batch, int height, int width
 extern "C" int aeaj_plan_destroy(aeaj_plan* p) {
     if (!p) return 0;
     cudaSetDevice(p->h->device);
-    cudaFree(p->planes_dev); cudaFree(p->class_off_dev); cudaFree(p->outs_dev); cudaFree(p->qtab_dev); cudaFree(p->qtabf_dev); cudaFree(p->pack_planes_dev); cudaFree(p->peer_segs_dev); cudaFree(p->df_planes_dev); cudaFree(p->if_planes_dev);
-    delete p;
+    cudaFree(p->class_off_dev); cudaFree(p->qtab_dev); cudaFree(p->qtabf_dev); cudaFree(p->peer_segs_dev);
+    delete p;                            // the descriptor tables free their device arrays
     return 0;
 }
 extern "C" int aeaj_plan_get_info(const aeaj_plan* p, aeaj_plan_info* info) {
@@ -645,17 +658,12 @@ extern "C" int aeaj_plan_set_qtables(aeaj_plan* p, const int32_t* tables, size_t
     return 0;
 }
 
-static int plan_push_planes(aeaj_plan* p, cudaStream_t st) {
+static int plan_push_planes(aeaj_plan* p, cudaStream_t st, PlaneDesc*& planes_dev) {
     for (auto& P : p->planes) {
         P.zigzag = p->zigzag;
         for (int k = 0; k < 9; k++) P.zz[k] = p->h->zz_dev[k];
     }
-    if (p->pushed_stream == st && p->planes_pushed.size() == p->planes.size() &&
-        memcmp(p->planes_pushed.data(), p->planes.data(), sizeof(PlaneDesc) * p->planes.size()) == 0) return 0;
-    AEAJ_CUDA(cudaMemcpyAsync(p->planes_dev, p->planes.data(), sizeof(PlaneDesc) * p->nplanes, cudaMemcpyHostToDevice, st));
-    p->planes_pushed = p->planes;
-    p->pushed_stream = st;
-    return 0;
+    return p->planes_tab.push(p->planes, st, planes_dev);
 }
 
 // full-res luma rows [band0, band1) -> rows of every layer (chroma rows scale with the subsampling ratio)
@@ -703,10 +711,8 @@ static int encode_impl(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, 
     aeaj_handle* h = p->h;
     const int B = p->info.batch, NP = p->nplanes;
     int launches = 0;
-    size_t s1 = plan_carve(p, workspace);
     PlanAux A;
-    plan_carve_aux(p, workspace, s1, A);
-    std::vector<uint8_t*> outs(NP, nullptr);
+    plan_carve(p, workspace, A);
     bool any_tap_edge = false;
     for (int l = 0; l < 3; l++) {
         AEAJ_REQUIRE(io->coef[l] && io->leaves[l] && io->states[l], "aeaj_encode: NULL output buffer");
@@ -717,11 +723,13 @@ static int encode_impl(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, 
             P.states = io->states[l] + (size_t)i * p->info.cap_states[l];
             P.counts = io->counts + ((size_t)i * 3 + l) * 4;
             P.packed_states = io->packed_states[l] ? io->packed_states[l] + (size_t)i * ((p->info.cap_states[l] + 3) / 4) : nullptr;
-            if (io->tap_edges[l]) { outs[i * 3 + l] = io->tap_edges[l] + (size_t)i * P.h * P.w; any_tap_edge = true; }
+            P.tap_edge = io->tap_edges[l] ? io->tap_edges[l] + (size_t)i * P.h * P.w : nullptr;
         }
+        any_tap_edge |= io->tap_edges[l] != nullptr;
     }
     int rc = set_band(p, band0, band1); if (rc) return rc;
-    rc = plan_push_planes(p, st); if (rc) return rc;
+    PlaneDesc* Pd;
+    rc = plan_push_planes(p, st, Pd); if (rc) return rc;
     p->ev_n = 0; p->ev_stream = st; p->mark("start");
     // a whole-image call on a plan that is one rank of a halo-split is a plain single-GPU call: no partial histograms to sum
     const bool whole = band0 == 0 && (band1 < 0 || band1 == p->info.height);
@@ -734,38 +742,37 @@ static int encode_impl(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, 
         if (peers.world > 1)                               // sharded quadtree: this rank fills only its band's leaf slots; the others read as absent
             for (int l = 0; l < 3; l++) AEAJ_CUDA(cudaMemsetAsync(io->leaves[l], 0, sizeof(int32_t) * 4 * (size_t)p->info.cap_leaves[l], st));
         // colour + chroma subsampling + u8 cast
-        rc = launch_color_forward_planar(h, p->info.space, io->rgb, io->rgb ? nullptr : io->rgb_u8, B, p->info.height, p->info.width, p->planes_dev, p->planes.data(),
+        rc = launch_color_forward_planar(h, p->info.space, io->rgb, io->rgb ? nullptr : io->rgb_u8, B, p->info.height, p->info.width, Pd, p->planes.data(),
                                          A.full_c1, A.full_c2, st, &launches, band0, band1);
         if (rc) return rc;
         p->mark("color_forward_planar");
     }
     // Canny pipeline on all planes of the batch at once
     if (phases & (1u << AEAJ_PHASE_CLAHE_HIST)) {
-        rc = launch_clahe_hist(p->planes_dev, p->planes.data(), NP, st); if (rc) return rc;
+        rc = launch_clahe_hist(Pd, p->planes.data(), NP, st); if (rc) return rc;
         launches++;
         p->mark("clahe_hist");
     }
     if (phases & (1u << AEAJ_PHASE_PREFILTER)) {
-        rc = launch_clahe_lut(p->planes_dev, NP, peers, st); if (rc) return rc;
+        rc = launch_clahe_lut(Pd, NP, peers, st); if (rc) return rc;
         p->mark("clahe_lut");
-        rc = launch_prefilter(p->planes_dev, p->planes.data(), NP, 7, 1, st); if (rc) return rc;
+        rc = launch_prefilter(Pd, p->planes.data(), NP, 7, 1, st); if (rc) return rc;
         p->mark("prefilter");
         launches += 2;
     }
     if (phases & (1u << AEAJ_PHASE_NMS)) {
-        rc = launch_thresholds(p->planes_dev, NP, peers, st); if (rc) return rc;
+        rc = launch_thresholds(Pd, NP, peers, st); if (rc) return rc;
         p->mark("thresholds");
-        rc = launch_canny_nms(p->planes_dev, p->planes.data(), NP, st); if (rc) return rc;
+        rc = launch_canny_nms(Pd, p->planes.data(), NP, st); if (rc) return rc;
         p->mark("canny_nms");
         launches += 2;
     }
     if (phases & (1u << AEAJ_PHASE_HYST)) {
-        rc = launch_hysteresis(h, p->planes_dev, p->planes.data(), NP, p->ntiles, p->ring_cap, A.flags, A.ring, A.ctrl, io->status, st); if (rc) return rc;
+        rc = launch_hysteresis(h, Pd, p->planes.data(), NP, p->ntiles, p->ring_cap, A.flags, A.ring, A.ctrl, io->status, st); if (rc) return rc;
         p->mark("hysteresis");
         launches += 1;
         if (any_tap_edge) {
-            AEAJ_CUDA(cudaMemcpyAsync(p->outs_dev, outs.data(), sizeof(uint8_t*) * NP, cudaMemcpyHostToDevice, st));
-            rc = launch_bitmap_to_u8(p->planes_dev, p->planes.data(), NP, p->outs_dev, st); if (rc) return rc;
+            rc = launch_bitmap_to_u8(Pd, p->planes.data(), NP, st); if (rc) return rc;
             launches++;
         }
         for (int l = 0; l < 3; l++)
@@ -776,17 +783,17 @@ static int encode_impl(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, 
     // quadtree: per-top-block counts (band), scan over all top blocks (needs every band's counts), emit (band)
     const int qt_parts = ((phases & (1u << AEAJ_PHASE_QT_COUNT)) ? 1 : 0) | ((phases & (1u << AEAJ_PHASE_QT_EMIT)) ? 6 : 0);
     if (qt_parts) {
-        rc = launch_quadtree(p->planes_dev, p->planes.data(), NP, p->info.block_min, p->info.block_max, A.class_lists, A.class_counts,
+        rc = launch_quadtree(Pd, p->planes.data(), NP, p->info.block_min, p->info.block_max, A.class_lists, A.class_counts,
                              p->class_off_dev, st, &launches, qt_parts);
         if (rc) return rc;
         if ((qt_parts & 4) && (io->packed_states[0] || io->packed_states[1] || io->packed_states[2])) {
-            rc = launch_pack_states(p->planes_dev, p->planes.data(), NP, st); if (rc) return rc;
+            rc = launch_pack_states(Pd, p->planes.data(), NP, st); if (rc) return rc;
             launches++;
         }
         p->mark("quadtree");
     }
     if (phases & (1u << AEAJ_PHASE_DCT)) {
-        rc = launch_dct_quant(h, p->planes_dev, A.class_lists, A.class_counts, p->cg.off, p->cg.cap, p->lg_min, p->lg_max, st, &launches,
+        rc = launch_dct_quant(h, Pd, A.class_lists, A.class_counts, p->cg.off, p->cg.cap, p->lg_min, p->lg_max, st, &launches,
                               plan_mark_cb, p, p->tensor_dct, A.scratch256);
         if (rc) return rc;
         if (io->status) AEAJ_CUDA(cudaMemcpyAsync(io->status + 2, h->tc_err_dev, sizeof(int), cudaMemcpyDeviceToDevice, st));
@@ -805,9 +812,8 @@ static int decode_impl(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, 
     aeaj_handle* h = p->h;
     const int B = p->info.batch, NP = p->nplanes;
     int launches = 0;
-    size_t s1 = plan_carve(p, workspace);
     PlanAux A;
-    plan_carve_aux(p, workspace, s1, A);
+    plan_carve(p, workspace, A);
     for (int l = 0; l < 3; l++) {
         AEAJ_REQUIRE(io->coef[l] && io->leaves[l], "aeaj_decode: NULL input buffer");
         for (int i = 0; i < B; i++) {
@@ -816,18 +822,20 @@ static int decode_impl(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, 
             P.leaves = (int32_t*)io->leaves[l] + (size_t)i * p->info.cap_leaves[l] * 4;
             P.counts = (int32_t*)io->counts + ((size_t)i * 3 + l) * 4;
             P.packed_states = nullptr;
+            P.tap_edge = nullptr;
         }
     }
     int rc = set_band(p, band0, band1); if (rc) return rc;
-    rc = plan_push_planes(p, st); if (rc) return rc;
+    PlaneDesc* Pd;
+    rc = plan_push_planes(p, st, Pd); if (rc) return rc;
     p->ev_n = 0; p->ev_stream = st; p->mark("start");
     if (phases & (1u << AEAJ_DPHASE_IDCT)) {
         AEAJ_CUDA(cudaMemsetAsync(A.class_counts, 0, 16 * sizeof(int), st));
-        rc = launch_bucket_leaves(p->planes_dev, p->planes.data(), NP, A.class_lists, A.class_counts, p->class_off_dev, p->lg_min, p->lg_max, st);
+        rc = launch_bucket_leaves(Pd, p->planes.data(), NP, A.class_lists, A.class_counts, p->class_off_dev, p->lg_min, p->lg_max, st);
         if (rc) return rc;
         launches++;
         p->mark("bucket_leaves");
-        rc = launch_dequant_idct(h, p->planes_dev, A.class_lists, A.class_counts, p->cg.off, p->cg.cap, p->lg_min, p->lg_max, st, &launches,
+        rc = launch_dequant_idct(h, Pd, A.class_lists, A.class_counts, p->cg.off, p->cg.cap, p->lg_min, p->lg_max, st, &launches,
                                  plan_mark_cb, p, p->tensor_dct, A.scratch256);
         if (rc) return rc;
         if (io->status) {
@@ -858,9 +866,8 @@ extern "C" int aeaj_decode(aeaj_plan* p, const aeaj_decode_io* io, void* workspa
 static int pack_impl(aeaj_plan* p, const int32_t* const* coef3, const int32_t* counts, const aeaj_packed_io* pk, void* workspace, cudaStream_t st, int unpack) {
     AEAJ_REQUIRE(p && coef3 && pk && pk->counts && workspace && (unpack || counts), "aeaj_(un)pack_coefficients: bad arguments");
     const int B = p->info.batch;
-    size_t s1 = plan_carve(p, workspace);
     PlanAux A;
-    plan_carve_aux(p, workspace, s1, A);
+    plan_carve(p, workspace, A);
     int64_t max_cap = 1;
     for (int l = 0; l < 3; l++) {
         AEAJ_REQUIRE(coef3[l] && pk->mask[l] && pk->vals[l], "aeaj_(un)pack_coefficients: NULL buffer");
@@ -879,12 +886,9 @@ static int pack_impl(aeaj_plan* p, const int32_t* const* coef3, const int32_t* c
         }
     }
     if (!unpack) AEAJ_CUDA(cudaMemsetAsync(pk->counts, 0, sizeof(int32_t) * 12 * (size_t)B, st));
-    const int k = unpack ? 1 : 0;
-    PackPlane* table = p->pack_planes_dev + (size_t)k * p->nplanes;
-    const bool same = p->pack_pushed_stream[k] == st && p->pack_pushed[k].size() == p->pack_planes.size() &&
-                      memcmp(p->pack_pushed[k].data(), p->pack_planes.data(), sizeof(PackPlane) * p->pack_planes.size()) == 0;
-    if (!same) { p->pack_pushed[k] = p->pack_planes; p->pack_pushed_stream[k] = st; }
-    return launch_pack(same ? nullptr : p->pack_planes.data(), table, p->nplanes, max_cap, unpack, st);
+    PackPlane* table;
+    int rc = (unpack ? p->unpack_tab : p->pack_tab).push(p->pack_planes, st, table); if (rc) return rc;
+    return launch_pack(table, p->nplanes, max_cap, unpack, st);
 }
 extern "C" int aeaj_pack_coefficients(aeaj_plan* p, const int32_t* const* coef3, const int32_t* counts, const aeaj_packed_io* out,
                                       void* workspace, void* stream) {
@@ -899,14 +903,29 @@ extern "C" int aeaj_unpack_coefficients(aeaj_plan* p, const aeaj_packed_io* in, 
 static int64_t deflate_chunks_cap(const aeaj_plan* p, int l) { return df_chunks(4 * p->info.cap_coef[l]); }
 static int64_t deflate_cap_out(const aeaj_plan* p, int l) { return (df_stream_bound(4 * p->info.cap_coef[l]) + 15) & ~(int64_t)15; }
 
+// the deflate scratch, per layer, per image: output slots | tokens | chunk offsets | lengths | Adler-32 sums.  Sets the scratch
+// pointers of planes[nplanes] (nullptr: size only) and returns the bytes the caller provides.
+static size_t deflate_carve(const aeaj_plan* p, void* scratch, DeflatePlane* planes) {
+    Bump b(scratch ? (void*)(((uintptr_t)scratch + 255) & ~(uintptr_t)255) : nullptr);
+    for (int l = 0; l < 3; l++) {
+        const int64_t nch = deflate_chunks_cap(p, l);
+        for (int i = 0; i < p->info.batch; i++) {
+            DeflatePlane size_only;
+            DeflatePlane& P = planes ? planes[i * 3 + l] : size_only;
+            P.slots = b.take<uint8_t>(nch * DF_CHUNK_BOUND);
+            P.tok = b.take<uint16_t>(nch * DF_CHUNK);
+            P.chunk_off = b.take<int64_t>(nch);
+            P.chunk_len = b.take<int32_t>(nch);
+            P.chunk_adler = b.take<uint32_t>(nch);
+        }
+    }
+    return b.used() + 256;
+}
+
 extern "C" int aeaj_deflate_caps(const aeaj_plan* p, int64_t* cap_out3, int64_t* scratch_bytes) {
     AEAJ_REQUIRE(p && cap_out3 && scratch_bytes, "aeaj_deflate_caps: bad arguments");
-    int64_t s = 0;
-    for (int l = 0; l < 3; l++) {
-        cap_out3[l] = deflate_cap_out(p, l);
-        s += p->info.batch * deflate_chunks_cap(p, l) * (int64_t)deflate_chunk_scratch_bytes();
-    }
-    *scratch_bytes = s + 256;
+    for (int l = 0; l < 3; l++) cap_out3[l] = deflate_cap_out(p, l);
+    *scratch_bytes = (int64_t)deflate_carve(p, nullptr, nullptr);
     return 0;
 }
 
@@ -915,10 +934,8 @@ extern "C" int aeaj_deflate_coefficients(aeaj_plan* p, const int32_t* const* coe
     AEAJ_REQUIRE(p && coef3 && counts && io && io->lengths && scratch, "aeaj_deflate_coefficients: bad arguments");
     const cudaStream_t st = ST(stream);
     const int B = p->info.batch;
-    if (!p->df_planes_dev) AEAJ_CUDA(cudaMalloc(&p->df_planes_dev, sizeof(DeflatePlane) * p->nplanes));
     p->df_planes.resize(p->nplanes);
-    // scratch: per layer, per image, per chunk: output slot | tokens | length, Adler-32, offset
-    uint8_t* base = (uint8_t*)(((uintptr_t)scratch + 255) & ~(uintptr_t)255);
+    deflate_carve(p, scratch, p->df_planes.data());
     int max_chunks = 1;
     for (int l = 0; l < 3; l++) {
         AEAJ_REQUIRE(coef3[l] && io->out[l], "aeaj_deflate_coefficients: NULL buffer");
@@ -933,18 +950,12 @@ extern "C" int aeaj_deflate_coefficients(aeaj_plan* p, const int32_t* const* coe
             P.cap_out = cap_out;
             P.length = io->lengths + (size_t)i * 3 + l;
             P.status = io->status;
-            P.slots = base; base += nch * DF_CHUNK_BOUND;
-            P.tok = (uint16_t*)base; base += nch * DF_CHUNK * 2;
-            P.chunk_off = (int64_t*)base; base += nch * 8;
-            P.chunk_len = (int32_t*)base; base += nch * 4;
-            P.chunk_adler = (uint32_t*)base; base += nch * 4;
         }
     }
     if (io->status) AEAJ_CUDA(cudaMemsetAsync(io->status, 0, 4 * sizeof(int32_t), st));
-    const bool same = p->df_pushed_stream == st && p->df_pushed.size() == p->df_planes.size() &&
-                      memcmp(p->df_pushed.data(), p->df_planes.data(), sizeof(DeflatePlane) * p->df_planes.size()) == 0;
-    if (!same) { p->df_pushed = p->df_planes; p->df_pushed_stream = st; }
-    return launch_deflate(same ? nullptr : p->df_planes.data(), p->df_planes_dev, p->nplanes, max_chunks, st);
+    DeflatePlane* table;
+    int rc = p->deflate_tab.push(p->df_planes, st, table); if (rc) return rc;
+    return launch_deflate(table, p->nplanes, max_chunks, st);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -976,7 +987,6 @@ extern "C" int aeaj_inflate_coefficients(aeaj_plan* p, const aeaj_inflate_io* io
                  io->segments && (io->in || in_bytes == 0), "aeaj_inflate_coefficients: bad arguments");
     const cudaStream_t st = ST(stream);
     const int B = p->info.batch;
-    if (!p->if_planes_dev) AEAJ_CUDA(cudaMalloc(&p->if_planes_dev, sizeof(InflatePlane) * p->nplanes));
     p->if_planes.resize(p->nplanes);
     for (int l = 0; l < 3; l++) {
         AEAJ_REQUIRE(io->coef[l], "aeaj_inflate_coefficients: NULL buffer");
@@ -1002,10 +1012,9 @@ extern "C" int aeaj_inflate_coefficients(aeaj_plan* p, const aeaj_inflate_io* io
     a.streams = (IfStream*)(base + L.streams);
     a.segs = (IfSeg*)(base + L.segs);
     a.map = (int32_t*)(base + L.map);
-    const bool same = p->if_pushed_stream == st && p->if_pushed.size() == p->if_planes.size() &&
-                      memcmp(p->if_pushed.data(), p->if_planes.data(), sizeof(InflatePlane) * p->if_planes.size()) == 0;
-    if (!same) { p->if_pushed = p->if_planes; p->if_pushed_stream = st; }
-    return launch_inflate(same ? nullptr : p->if_planes.data(), p->if_planes_dev, a, p->h->sm_count, st);
+    InflatePlane* table;
+    int rc = p->inflate_tab.push(p->if_planes, st, table); if (rc) return rc;
+    return launch_inflate(table, a, p->h->sm_count, st);
 }
 
 extern "C" int aeaj_pack_coefficients_host(const int32_t* coef, int64_t n, uint32_t* mask, int16_t* vals, int64_t* nnz, int* overflow) {
@@ -1081,7 +1090,7 @@ extern "C" int aeaj_plan_set_peers(aeaj_plan* p, int rank, int world, void* cons
         AEAJ_REQUIRE(p->peer_ws[r] && p->peer_flags[r], "aeaj_plan_set_peers: NULL peer pointer");
         p->peers.delta[r] = (long long)((const char*)p->peer_ws[r] - (const char*)p->peer_ws[rank]);
     }
-    p->planes_pushed.clear();
+    p->planes_tab.forget();
     if (world > 1 && !p->peer_segs_dev) {
         AEAJ_CUDA(cudaSetDevice(p->h->device));
         AEAJ_CUDA(cudaMalloc(&p->peer_segs_dev, sizeof(PeerSeg) * 64 * 2));
@@ -1104,7 +1113,8 @@ static int peer_barrier(aeaj_plan* p, cudaStream_t st) {
 static int peer_gather(aeaj_plan* p, int what, void* workspace, cudaStream_t st) {
     const int world = p->peers.world, rank = p->peers.rank;
     if (world <= 1) return 0;
-    plan_carve(p, workspace);
+    PlanAux A;
+    plan_carve(p, workspace, A);
     const int H = p->info.height;
     std::vector<PeerSeg> segs;
     long long maxb = 0;

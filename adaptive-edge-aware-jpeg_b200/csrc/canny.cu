@@ -801,9 +801,9 @@ __global__ void __launch_bounds__(HY_THREADS) k_hysteresis(const PlaneDesc* __re
 }
 
 // final strong bitmap -> uint8 {0,1} map (API / taps) and the reverse (stage API)
-__global__ void __launch_bounds__(256) k_bitmap_to_u8(const PlaneDesc* __restrict__ planes, uint8_t* const* __restrict__ outs) {
+__global__ void __launch_bounds__(256) k_bitmap_to_u8(const PlaneDesc* __restrict__ planes) {
     const PlaneDesc& P = planes[blockIdx.z];
-    uint8_t* out = outs[blockIdx.z];
+    uint8_t* out = P.tap_edge;
     int x = blockIdx.x * 256 + threadIdx.x, y = blockIdx.y;
     if (!out || y >= P.h || x >= P.w) return;
     out[(size_t)y * P.w + x] = (P.strong[(size_t)y * P.wpr + (x >> 5)] >> (x & 31)) & 1u;
@@ -918,9 +918,9 @@ int launch_hysteresis(aeaj_handle* h, const PlaneDesc* planes_dev, const PlaneDe
     return 0;
 }
 
-int launch_bitmap_to_u8(const PlaneDesc* planes_dev, const PlaneDesc* P, int nplanes, uint8_t* const* outs_dev, cudaStream_t st) {
+int launch_bitmap_to_u8(const PlaneDesc* planes_dev, const PlaneDesc* P, int nplanes, cudaStream_t st) {
     dim3 grd(aeaj_cdiv(max_dim(P, nplanes, true), 256), max_dim(P, nplanes, false), nplanes);
-    k_bitmap_to_u8<<<grd, 256, 0, st>>>(planes_dev, outs_dev);
+    k_bitmap_to_u8<<<grd, 256, 0, st>>>(planes_dev);
     AEAJ_LAUNCH_CHECK();
     return 0;
 }

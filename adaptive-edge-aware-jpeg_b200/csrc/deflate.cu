@@ -171,11 +171,7 @@ int aeaj_deflate_init() {
     return 0;
 }
 
-size_t deflate_chunk_scratch_bytes() { return (size_t)DF_CHUNK_BOUND + 2 * (size_t)DF_CHUNK + 16; }
-
-int launch_deflate(const DeflatePlane* planes_host, DeflatePlane* planes_dev, int nplanes, int max_chunks, cudaStream_t st) {
-    if (planes_host)                                                   // nullptr: the device table already holds these descriptors
-        AEAJ_CUDA(cudaMemcpyAsync(planes_dev, planes_host, sizeof(DeflatePlane) * nplanes, cudaMemcpyHostToDevice, st));
+int launch_deflate(const DeflatePlane* planes_dev, int nplanes, int max_chunks, cudaStream_t st) {
     k_deflate_chunks<<<dim3(max_chunks, nplanes), DF_THREADS, sizeof(DfSmem), st>>>(planes_dev);
     AEAJ_LAUNCH_CHECK();
     k_deflate_finish<<<nplanes, 32, 0, st>>>(planes_dev);

@@ -186,9 +186,7 @@ __global__ void k_inflate_finish(const InflatePlane* __restrict__ planes, Inflat
 
 }  // namespace
 
-int launch_inflate(const InflatePlane* planes_host, InflatePlane* planes_dev, const InflateArgs& a, int sm_count, cudaStream_t st) {
-    if (planes_host)                                                   // nullptr: the device table already holds these descriptors
-        AEAJ_CUDA(cudaMemcpyAsync(planes_dev, planes_host, sizeof(InflatePlane) * a.nplanes, cudaMemcpyHostToDevice, st));
+int launch_inflate(const InflatePlane* planes_dev, const InflateArgs& a, int sm_count, cudaStream_t st) {
     AEAJ_CUDA(cudaMemsetAsync(a.counters, 0, 4 * sizeof(int), st));
     const int64_t tiles = (a.in_bytes + 256 * 16 - 1) / (256 * 16);
     k_inflate_scan<<<dim3((unsigned)std::max<int64_t>(1, std::min<int64_t>(tiles, 1024)), a.nplanes), 256, 0, st>>>(planes_dev, a);

@@ -159,9 +159,7 @@ __global__ void __launch_bounds__(PK_THREADS) k_unpack_emit(const PackPlane* __r
 
 size_t aeaj_pack_scratch_ints(int64_t cap_coef) { return (size_t)(cap_coef / PK_CHUNK + 2); }
 
-int launch_pack(const PackPlane* planes_host, PackPlane* planes_dev, int nplanes, int64_t max_cap_coef, int unpack, cudaStream_t st) {
-    if (planes_host)                                                   // nullptr: the device table already holds these descriptors
-        AEAJ_CUDA(cudaMemcpyAsync(planes_dev, planes_host, sizeof(PackPlane) * nplanes, cudaMemcpyHostToDevice, st));
+int launch_pack(const PackPlane* planes_dev, int nplanes, int64_t max_cap_coef, int unpack, cudaStream_t st) {
     const unsigned chunks = (unsigned)std::max<int64_t>(1, (max_cap_coef + PK_CHUNK - 1) / PK_CHUNK);
     dim3 grd(chunks, nplanes);
     if (!unpack) {

@@ -89,7 +89,8 @@ AEAJ_API int aeaj_downsample_area(aeaj_handle* h, const float* src, int H, int W
 AEAJ_API int aeaj_resize_linear(aeaj_handle* h, const float* src, int sh, int sw, float* dst, int H, int W, void* stream);
 
 /* Device scratch for ANY single-plane stage call below on an (h,w) plane with the given block range
- * (upper bound over all stages; pass min_size = max_size = 0 if no quadtree/DCT call is made). */
+ * (upper bound over all stages; pass min_size = max_size = 0 if no quadtree/DCT call is made).
+ * The workspace also holds the call's descriptors: two stage calls in flight at once need two workspaces, not two handles. */
 AEAJ_API size_t aeaj_stage_workspace_bytes(int h, int w, int min_size, int max_size);
 
 /* EdgeDetection.canny stages (edge_detection.py:70-86), one (h,w) plane each. */

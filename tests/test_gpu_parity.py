@@ -211,6 +211,58 @@ def test_dct_quant_and_inverse(st, brange):
         assert np.abs(rec - ref).max() <= 2e-6            # f32 IDCT vs f64-accumulated oracle, values in [0,1]
 
 
+def test_two_stage_calls_in_flight():
+    """A stage call keeps its descriptors in its workspace: two aeaj_dct_quant calls on one handle, two workspaces and two
+    streams, the first held back so that they overlap, give what each gives alone."""
+    import ctypes as C
+    import torch
+    from aeaj import native
+    lib, hd = native.load(), native.handle(0)
+    H, W, brange = 200, 328, (4, 128)
+    space = "YCbCr"
+    layers = [np.ascontiguousarray(O.color_forward(space, synth(H, W, seed=s).reshape(-1, 3)).reshape(H, W, 3)[..., 0], dtype=np.float32)
+              for s in (31, 32)]
+    leaves, _, _ = O.quadtree(O.canny(layers[0]), brange[1], brange[0])       # one leaf list: the calls differ in their pixels only
+    off = np.concatenate([[0], np.cumsum(leaves[:, 2].astype(np.int64) ** 2)])[:-1]
+    n_coef = int((leaves[:, 2].astype(np.int64) ** 2).sum())
+    lv = torch.from_numpy(np.ascontiguousarray(np.concatenate([leaves, off[:, None].astype(np.int32)], axis=1))).cuda()
+    counts = torch.tensor([len(leaves), 0, n_coef, 0], dtype=torch.int32, device="cuda")
+    tabs = O.qtables(space, (30, 95), brange)[0]
+    tab_t = {s: torch.from_numpy(np.ascontiguousarray(m, dtype=np.int32)).cuda() for s, m in tabs.items()}
+    qtab = (C.c_void_p * 9)()
+    for s, t in tab_t.items():
+        qtab[int(np.log2(s))] = t.data_ptr()
+    mid, sc = O.NORM[space]
+    src = [torch.from_numpy(l).cuda() for l in layers]
+    ws = [torch.empty(int(lib.aeaj_stage_workspace_bytes(H, W, *brange)), dtype=torch.uint8, device="cuda") for _ in range(2)]
+    out = [torch.empty(n_coef, dtype=torch.int32, device="cuda") for _ in range(2)]
+
+    def call(k, stream):
+        native.check(lib.aeaj_dct_quant(hd, src[k].data_ptr(), H, W, float(mid[0]), float(sc[0]), lv.data_ptr(), counts.data_ptr(),
+                                        brange[0], brange[1], qtab, out[k].data_ptr(), ws[k].data_ptr(), stream.cuda_stream), "aeaj_dct_quant")
+
+    alone = []
+    for k in range(2):
+        out[k].fill_(-1)
+        call(k, torch.cuda.current_stream())
+        torch.cuda.synchronize()
+        alone.append(out[k].clone())
+    assert not torch.equal(alone[0], alone[1])
+    streams = [torch.cuda.Stream() for _ in range(2)]
+    for s in streams:
+        s.wait_stream(torch.cuda.current_stream())
+    for o in out:
+        o.fill_(-1)
+    torch.cuda.synchronize()
+    with torch.cuda.stream(streams[0]):
+        torch.cuda._sleep(50_000_000)                      # the first call starts after the second one is enqueued and running
+    call(0, streams[0])
+    call(1, streams[1])
+    torch.cuda.synchronize()
+    for k in range(2):
+        assert torch.equal(out[k], alone[k]), k
+
+
 # ------------------------------------------------------------------------------------------------
 # fused batch path + reference-facing shim
 # ------------------------------------------------------------------------------------------------
@@ -818,6 +870,45 @@ def test_cuda_graph_roundtrip_equals_eager(codec):
     g.replay()
     torch.cuda.synchronize()
     assert torch.equal(res, codec.decode_encoded(codec.encode(rgb, space, q, b), space, q, b))
+
+
+def test_cuda_graph_of_pack_and_unpack(codec):
+    """steady-state pack / unpack issue no host-to-device copy either (the two keep separate descriptor tables): encode, pack,
+    unpack and decode captured in one CUDA graph give the bits of the eager calls"""
+    import torch
+    H, W = 272, 480
+    space, q, b = "YCbCr", (30, 95), (4, 128)
+    rgb = torch.from_numpy(synth(H, W, seed=23)).cuda().unsqueeze(0)
+
+    def run():
+        enc = codec.encode(rgb, space, q, b, instance=2200)
+        pk = codec.pack(enc, space, q, b, instance=2200)
+        coef = codec.unpack(pk, 1, H, W, space, q, b, instance=2200)
+        return enc, pk, coef, codec.decode(coef, enc.leaves, enc.counts, 1, H, W, space, q, b, instance=2200)
+
+    def used(enc, pk, coef, res):                         # the parts of the buffers the calls write
+        c, pc = enc.counts.cpu().numpy(), pk.counts.cpu().numpy()
+        out = [enc.counts.clone(), pk.counts.clone(), res.clone()]
+        for l in range(3):
+            nnz, _, _, nw = (int(x) for x in pc[0, l])
+            out += [pk.mask[l][0, :nw].clone(), pk.vals[l][0, :nnz].clone(), coef[l][0, :int(c[0, l, 2])].clone()]
+        return out
+
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):
+        eager = run()
+    torch.cuda.synchronize()
+    eager = used(*eager)
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g, stream=side):
+        enc, pk, coef, res = run()
+    for t in [enc.counts, pk.counts, res] + pk.mask + pk.vals + coef:
+        t.zero_()
+    g.replay()
+    torch.cuda.synchronize()
+    got = used(enc, pk, coef, res)
+    assert all(torch.equal(a, e) for a, e in zip(got, eager))
 
 
 def test_two_stream_roundtrip_equals_single_stream(codec):
