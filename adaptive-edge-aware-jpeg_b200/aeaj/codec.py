@@ -109,6 +109,18 @@ class _Job:
 
 
 @dataclass
+class _Scaled:
+    """A plan's buffers for decode(..., scale=k), k > 1 (aeaj_decode_scaled)."""
+    out_h: int
+    out_w: int
+    layer_h: Tuple[int, int, int]  # the final scaled layers
+    layer_w: Tuple[int, int, int]
+    scratch: torch.Tensor          # the scaled layers of the call
+    rgb_out: torch.Tensor          # float32 [B, out_h, out_w, 3]
+    rgb8_out: Optional[torch.Tensor] = None
+
+
+@dataclass
 class _Plan:
     ptr: C.c_void_p
     info: native.PlanInfo
@@ -124,6 +136,7 @@ class _Plan:
     deflate_scratch: Optional[torch.Tensor] = None
     inflated: Optional[InflatedBatch] = None
     inflate_scratch: Optional[torch.Tensor] = None
+    scaled: Dict[int, _Scaled] = field(default_factory=dict)
     nbytes: int = 0
 
 
@@ -269,14 +282,20 @@ class DeviceCodec:
         return o
 
     def decode(self, coef, leaves, counts, B, H, W, space: str, qrange, brange, taps: bool = False, instance: int = 0,
-               zigzag: bool = False, out: str = "f32"):
+               zigzag: bool = False, out: str = "f32", scale: int = 1):
         """coef/leaves: 3 device tensors laid out like EncodedBatch; counts int32 [B,3,4]. Returns rgb [B,H,W,3].
         zigzag=True: the coefficient blocks are in the .ajpg zigzag order.
         out: "f32" (Image.data), "u8" (Image.get_uint8(), (data * 255).astype(uint8), written by the same kernel) or "both"
-        (returns the pair)."""
+        (returns the pair).
+        scale: 2, 4 or 8 decode at 1/scale of the size, straight from the coefficients (aeaj_decode_scaled, include/aeaj.h) and
+        return rgb [B, ceil(H/scale), ceil(W/scale), 3] (taps: the scaled layers); 1 is the full-size decode."""
         if out not in ("f32", "u8", "both"):
             raise ValueError("out must be 'f32', 'u8' or 'both'")
+        if scale not in (1, 2, 4, 8):
+            raise ValueError("scale must be 1, 2, 4 or 8")
         p = self._plan(B, H, W, space, brange, qrange, instance)
+        if scale != 1:
+            return self._decode_scaled(p, coef, leaves, counts, B, taps, zigzag, out, scale)
         native.check(self.lib.aeaj_plan_set_stream_layout(p.ptr, int(zigzag)), "aeaj_plan_set_stream_layout")
         native.check(self.lib.aeaj_plan_set_tensor_dct(p.ptr, self._tensor_mask()), "aeaj_plan_set_tensor_dct")
         io = native.DecodeIO()
@@ -302,6 +321,51 @@ class DeviceCodec:
         native.check(self.lib.aeaj_decode(p.ptr, C.byref(io), p.workspace.data_ptr(), _stream()), "aeaj_decode")
         self.last_launches = self.lib.aeaj_plan_last_launches(p.ptr)
         res = p.rgb_out if out == "f32" else (p.rgb8_out if out == "u8" else (p.rgb_out, p.rgb8_out))
+        return (res, tl) if taps else res
+
+    def _scaled(self, p: _Plan, scale: int) -> _Scaled:
+        sc = p.scaled.get(scale)
+        if sc is None:
+            oh, ow, scratch = C.c_int(), C.c_int(), C.c_int64()
+            lh, lw = (C.c_int * 3)(), (C.c_int * 3)()
+            native.check(self.lib.aeaj_decode_scaled_geometry(p.ptr, scale, C.byref(oh), C.byref(ow), lh, lw, C.byref(scratch)),
+                         "aeaj_decode_scaled_geometry")
+            dev = p.rgb_out.device
+            sc = _Scaled(oh.value, ow.value, tuple(lh), tuple(lw), torch.empty(int(scratch.value), dtype=torch.uint8, device=dev),
+                         torch.empty((p.info.batch, oh.value, ow.value, 3), dtype=torch.float32, device=dev))
+            p.scaled[scale] = sc
+            p.nbytes += sc.scratch.numel() + sc.rgb_out.numel() * 4
+            self._evict(keep=next(k for k, v in self._plans.items() if v is p))
+        return sc
+
+    def _decode_scaled(self, p: _Plan, coef, leaves, counts, B, taps, zigzag, out, scale):
+        sc = self._scaled(p, scale)
+        native.check(self.lib.aeaj_plan_set_stream_layout(p.ptr, int(zigzag)), "aeaj_plan_set_stream_layout")
+        io = native.DecodeIO()
+        for l in range(3):
+            if coef[l].shape[1] != p.info.cap_coef[l] or leaves[l].shape[1] != p.info.cap_leaves[l]:
+                raise ValueError("decode buffers must use the plan's capacities")
+            io.coef[l] = coef[l].data_ptr()
+            io.leaves[l] = leaves[l].data_ptr()
+        io.counts = counts.data_ptr()
+        if out != "u8":
+            io.rgb = sc.rgb_out.data_ptr()
+        if out != "f32":
+            if sc.rgb8_out is None:
+                sc.rgb8_out = torch.empty(sc.rgb_out.shape, dtype=torch.uint8, device=sc.rgb_out.device)
+                p.nbytes += sc.rgb8_out.numel()
+            io.rgb_u8 = sc.rgb8_out.data_ptr()
+        io.status = p.dec_status.data_ptr()
+        self.last_decode_status = p.dec_status
+        tl = None
+        if taps:
+            tl = [torch.empty((B, sc.layer_h[l], sc.layer_w[l]), dtype=torch.float32, device=sc.rgb_out.device) for l in range(3)]
+            for l in range(3):
+                io.tap_layers[l] = tl[l].data_ptr()
+        native.check(self.lib.aeaj_decode_scaled(p.ptr, C.byref(io), scale, p.workspace.data_ptr(), sc.scratch.data_ptr(), _stream()),
+                     "aeaj_decode_scaled")
+        self.last_launches = self.lib.aeaj_plan_last_launches(p.ptr)
+        res = sc.rgb_out if out == "f32" else (sc.rgb8_out if out == "u8" else (sc.rgb_out, sc.rgb8_out))
         return (res, tl) if taps else res
 
     # ------------------------------------------------------------------------------------------

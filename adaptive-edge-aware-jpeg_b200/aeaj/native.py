@@ -28,6 +28,7 @@ EXPORTS = [
     "aeaj_plan_set_peers", "aeaj_copy_segments",
     "aeaj_encode_halo", "aeaj_decode_halo", "aeaj_set_fast_transfer",
     "aeaj_deflate_caps", "aeaj_deflate_coefficients", "aeaj_inflate_scratch_bytes", "aeaj_inflate_coefficients",
+    "aeaj_decode_scaled_geometry", "aeaj_decode_scaled",
 ]
 
 
@@ -117,6 +118,8 @@ def load():
         lib.aeaj_plan_set_qtables.argtypes = [vp, vp, sz, vp]
         lib.aeaj_encode.argtypes = [vp, C.POINTER(EncodeIO), vp, vp]
         lib.aeaj_decode.argtypes = [vp, C.POINTER(DecodeIO), vp, vp]
+        lib.aeaj_decode_scaled_geometry.argtypes = [vp, i, C.POINTER(i), C.POINTER(i), C.POINTER(i), C.POINTER(i), C.POINTER(C.c_int64)]
+        lib.aeaj_decode_scaled.argtypes = [vp, C.POINTER(DecodeIO), i, vp, vp, vp]
         lib.aeaj_plan_last_launches.argtypes = [vp]
         lib.aeaj_plan_set_stream_layout.argtypes = [vp, i]
         lib.aeaj_plan_set_tensor_dct.argtypes = [vp, i]

@@ -151,7 +151,9 @@ struct aeaj_handle {
     float* dct_half_all_dev;
     int32_t* zz_dev[9];           // zigzag tables per log2(size), device
     int32_t* zz_all_dev;
-    int32_t* izz256_dev;          // inverse zigzag permutation for 256x256
+    int32_t* izz_dev[9];          // inverse zigzag permutations per log2(size): row-major index -> stream position
+    int32_t* izz_all_dev;
+    int32_t* izz256_dev;          // izz_dev[8] (k_dct256)
     int32_t* tc_izz_dev[4];       // inverse zigzag permutations for 16 .. 128 (tensor-core kernels)
     int32_t* tc_izz_all_dev;
     float* dct_tc_tiles_dev;      // [size class 16..128][fwd, inv][Ah | Al]: block-diagonal DCT matrices for the tcgen05 path
@@ -323,3 +325,10 @@ int launch_dct_tc(aeaj_handle* h, int size, const PlaneDesc* planes_dev, const C
 int launch_dequant_idct(aeaj_handle* h, const PlaneDesc* planes_dev, const ClassEntry* class_lists, const int* class_counts,
                         const int64_t* class_offsets_host, const int64_t* class_caps_host, int lg_min, int lg_max,
                         cudaStream_t st, int* launches, void (*mark)(void*, const char*), void* mark_ctx, int tensor_dct, float* scratch256);
+// scaled decode (idct_scaled.cu): the leaves of every class to the 1/m planes (the descriptors' layer_f32, ceil(h/m) x ceil(w/m)),
+// and the box reduce of one layer's batch of planes [batch][sh][sw] by f
+int aeaj_idct_scaled_init();
+int launch_idct_scaled(aeaj_handle* h, const PlaneDesc* planes_dev, const ClassEntry* class_lists, const int* class_counts,
+                       const int64_t* class_offsets_host, const int64_t* class_caps_host, int lg_min, int lg_max, int m,
+                       cudaStream_t st, int* launches);
+int launch_box_reduce(const float* src, int sh, int sw, float* dst, int dh, int dw, int f, int batch, cudaStream_t st);

@@ -156,6 +156,8 @@ extern "C" int aeaj_create(int device, aeaj_handle** out) {
     if (rc) { free(h); return rc; }
     rc = aeaj_deflate_init();
     if (rc) { free(h); return rc; }
+    rc = aeaj_idct_scaled_init();
+    if (rc) { free(h); return rc; }
     AEAJ_CUDA(cudaMalloc(&h->srgb_lut_dev, 256 * sizeof(float)));
     *out = h;
     return 0;
@@ -164,7 +166,7 @@ extern "C" int aeaj_create(int device, aeaj_handle** out) {
 extern "C" int aeaj_destroy(aeaj_handle* h) {
     if (!h) return 0;
     cudaSetDevice(h->device);
-    cudaFree(h->pq_tabs_dev); cudaFree(h->srgb_lut_dev); cudaFree(h->dct_all_dev); cudaFree(h->dct_half_all_dev); cudaFree(h->zz_all_dev); cudaFree(h->izz256_dev); cudaFree(h->dct_tc_tiles_dev); cudaFree(h->tc_izz_all_dev); cudaFree(h->tc_err_dev);
+    cudaFree(h->pq_tabs_dev); cudaFree(h->srgb_lut_dev); cudaFree(h->dct_all_dev); cudaFree(h->dct_half_all_dev); cudaFree(h->zz_all_dev); cudaFree(h->izz_all_dev); cudaFree(h->dct_tc_tiles_dev); cudaFree(h->tc_izz_all_dev); cudaFree(h->tc_err_dev);
     free(h);
     return 0;
 }
@@ -429,6 +431,8 @@ struct aeaj_plan {
     DescTable<DeflatePlane> deflate_tab;
     std::vector<InflatePlane> if_planes;
     DescTable<InflatePlane> inflate_tab;
+    std::vector<PlaneDesc> scaled_planes;  // aeaj_decode_scaled: the planes with layer_f32 on the 1/m planes of the caller's scratch
+    DescTable<PlaneDesc> scaled_tab[4];    // one per log2(scale): decodes alternating between scales upload nothing either
     // one image over several GPUs (peer.cu): the other ranks' workspaces / barrier flags, opened through CUDA IPC by the caller
     PeerSet peers = {1, 0, {0}};
     void* peer_ws[AEAJ_MAX_PEERS] = {nullptr};
@@ -858,6 +862,121 @@ static int decode_impl(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, 
 }
 extern "C" int aeaj_decode(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream) {
     return decode_impl(p, io, workspace, ST(stream), 0x3u, 0, -1);
+}
+
+// ---------------------------------------------------------------------------------------------
+// scaled decode (idct_scaled.cu): 1/scale of every layer from the top-left coefficients of each leaf
+// ---------------------------------------------------------------------------------------------
+struct ScaledGeom {
+    int k, m;                        // scale; the IDCT's own factor min(scale, block_min)
+    int out_h, out_w;
+    int hm[3], wm[3];                // the 1/m layers
+    int hk[3], wk[3];                // the 1/scale layers (== the 1/m layers when scale <= block_min)
+};
+static int scaled_geom(const aeaj_plan* p, int scale, ScaledGeom& g) {
+    AEAJ_REQUIRE(scale == 1 || scale == 2 || scale == 4 || scale == 8, "aeaj_decode_scaled: scale must be 1, 2, 4 or 8");
+    g.k = scale; g.m = std::min(scale, p->info.block_min);
+    g.out_h = aeaj_cdiv(p->info.height, scale); g.out_w = aeaj_cdiv(p->info.width, scale);
+    for (int l = 0; l < 3; l++) {
+        g.hm[l] = aeaj_cdiv(p->info.layer_h[l], g.m); g.wm[l] = aeaj_cdiv(p->info.layer_w[l], g.m);
+        g.hk[l] = aeaj_cdiv(p->info.layer_h[l], scale); g.wk[l] = aeaj_cdiv(p->info.layer_w[l], scale);
+    }
+    return 0;
+}
+// the caller's scratch: per layer the batch's 1/m planes, then (scale > block_min) the 1/scale planes; nullptr: size only
+static size_t scaled_carve(const aeaj_plan* p, const ScaledGeom& g, void* scratch, float* mp[3], float* kp[3]) {
+    if (g.k == 1) { for (int l = 0; l < 3; l++) mp[l] = kp[l] = nullptr; return 0; }
+    Bump b(scratch ? (void*)(((uintptr_t)scratch + 255) & ~(uintptr_t)255) : nullptr);
+    const int B = p->info.batch;
+    for (int l = 0; l < 3; l++) {
+        mp[l] = b.take<float>((size_t)B * g.hm[l] * g.wm[l]);
+        kp[l] = (g.k > g.m) ? b.take<float>((size_t)B * g.hk[l] * g.wk[l]) : mp[l];
+    }
+    return b.used() + 256;
+}
+
+extern "C" int aeaj_decode_scaled_geometry(const aeaj_plan* p, int scale, int* out_h, int* out_w, int layer_h[3], int layer_w[3],
+                                           int64_t* scratch_bytes) {
+    AEAJ_REQUIRE(p && out_h && out_w && layer_h && layer_w && scratch_bytes, "aeaj_decode_scaled_geometry: bad arguments");
+    ScaledGeom g;
+    int rc = scaled_geom(p, scale, g); if (rc) return rc;
+    *out_h = g.out_h; *out_w = g.out_w;
+    for (int l = 0; l < 3; l++) { layer_h[l] = g.hk[l]; layer_w[l] = g.wk[l]; }
+    float* mp[3]; float* kp[3];
+    *scratch_bytes = (int64_t)scaled_carve(p, g, nullptr, mp, kp);
+    return 0;
+}
+
+extern "C" int aeaj_decode_scaled(aeaj_plan* p, const aeaj_decode_io* io, int scale, void* workspace, void* scratch, void* stream) {
+    AEAJ_REQUIRE(p && io && workspace && (io->rgb || io->rgb_u8) && io->counts, "aeaj_decode_scaled: bad arguments (rgb or rgb_u8 required)");
+    AEAJ_REQUIRE(p->peers.world == 1, "aeaj_decode_scaled: a plan with peers (multi-GPU halo-split) is not supported");
+    ScaledGeom g;
+    int rc = scaled_geom(p, scale, g); if (rc) return rc;
+    const cudaStream_t st = ST(stream);
+    if (scale == 1) return decode_impl(p, io, workspace, st, 0x3u, 0, -1);
+    AEAJ_REQUIRE(scratch, "aeaj_decode_scaled: NULL scratch");
+    AEAJ_REQUIRE(p->qtab_dev, "aeaj_decode_scaled: quantisation tables not set (aeaj_plan_set_qtables)");
+    aeaj_handle* h = p->h;
+    const int B = p->info.batch, NP = p->nplanes;
+    PlanAux A;
+    plan_carve(p, workspace, A);
+    float* mp[3]; float* kp[3];
+    scaled_carve(p, g, scratch, mp, kp);
+    p->scaled_planes = p->planes;
+    for (int l = 0; l < 3; l++) {
+        AEAJ_REQUIRE(io->coef[l] && io->leaves[l], "aeaj_decode_scaled: NULL input buffer");
+        for (int i = 0; i < B; i++) {
+            PlaneDesc& P = p->scaled_planes[i * 3 + l];
+            P.coef = (int32_t*)io->coef[l] + (size_t)i * p->info.cap_coef[l];
+            P.leaves = (int32_t*)io->leaves[l] + (size_t)i * p->info.cap_leaves[l] * 4;
+            P.counts = (int32_t*)io->counts + ((size_t)i * 3 + l) * 4;
+            P.packed_states = nullptr;
+            P.tap_edge = nullptr;
+            P.ry0 = 0; P.ry1 = P.h; P.peer_up = P.peer_dn = 0;
+            P.zigzag = p->zigzag;
+            for (int k = 0; k < 9; k++) P.zz[k] = h->zz_dev[k];
+            P.layer_f32 = mp[l] + (size_t)i * g.hm[l] * g.wm[l];
+        }
+    }
+    PlaneDesc* Pd;
+    rc = p->scaled_tab[ilog2i(scale)].push(p->scaled_planes, st, Pd); if (rc) return rc;
+    int launches = 0;
+    p->ev_n = 0; p->ev_stream = st; p->mark("start");
+    AEAJ_CUDA(cudaMemsetAsync(A.class_counts, 0, 16 * sizeof(int), st));
+    rc = launch_bucket_leaves(Pd, p->scaled_planes.data(), NP, A.class_lists, A.class_counts, p->class_off_dev, p->lg_min, p->lg_max, st);
+    if (rc) return rc;
+    launches++;
+    p->mark("bucket_leaves");
+    rc = launch_idct_scaled(h, Pd, A.class_lists, A.class_counts, p->cg.off, p->cg.cap, p->lg_min, p->lg_max, g.m, st, &launches);
+    if (rc) return rc;
+    p->mark("idct_scaled");
+    if (g.k > g.m) {
+        for (int l = 0; l < 3; l++) {
+            rc = launch_box_reduce(mp[l], g.hm[l], g.wm[l], kp[l], g.hk[l], g.wk[l], g.k / g.m, B, st); if (rc) return rc;
+            launches++;
+        }
+        p->mark("box_reduce");
+    }
+    if (io->status) {
+        AEAJ_CUDA(cudaMemcpyAsync(io->status + 2, h->tc_err_dev, sizeof(int), cudaMemcpyDeviceToDevice, st));
+        AEAJ_CUDA(cudaMemcpyAsync(io->status + 3, A.class_counts + 15, sizeof(int), cudaMemcpyDeviceToDevice, st));
+    }
+    for (int l = 0; l < 3; l++)
+        if (io->tap_layers[l])
+            AEAJ_CUDA(cudaMemcpyAsync(io->tap_layers[l], kp[l], sizeof(float) * (size_t)B * g.hk[l] * g.wk[l], cudaMemcpyDeviceToDevice, st));
+    // the colour tail reads the 1/scale layers through host descriptors of their final geometry
+    PlaneDesc tail[3];
+    for (int l = 0; l < 3; l++) {
+        memset(&tail[l], 0, sizeof tail[l]);
+        tail[l].h = g.hk[l]; tail[l].w = g.wk[l]; tail[l].ry0 = 0; tail[l].ry1 = g.hk[l]; tail[l].layer = l;
+        tail[l].layer_f32 = kp[l];
+    }
+    rc = launch_upsample_color_inverse(h, p->info.space, tail, B, g.out_h, g.out_w, io->rgb, io->rgb_u8, st);
+    if (rc) return rc;
+    launches++;
+    p->mark("upsample_color_inverse");
+    p->last_launches = launches;
+    return 0;
 }
 
 // ---------------------------------------------------------------------------------------------

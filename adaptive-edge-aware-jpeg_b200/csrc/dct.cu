@@ -768,13 +768,16 @@ int aeaj_dct_init(aeaj_handle* h) {
         h->zz_dev[lg] = h->zz_all_dev + zo;
         zo += (size_t)s * s;
     }
-    {   // inverse permutation for 256 x 256 (row-major index -> stream position), used by k_dct256
-        const int n = 256 * 256;
-        const int32_t* z256 = zh + (h->zz_dev[8] - h->zz_all_dev);
-        std::vector<int32_t> inv((size_t)n);
-        for (int i = 0; i < n; i++) inv[z256[i]] = i;
-        AEAJ_CUDA(cudaMalloc(&h->izz256_dev, (size_t)n * sizeof(int32_t)));
-        AEAJ_CUDA(cudaMemcpy(h->izz256_dev, inv.data(), (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice));
+    {   // inverse permutations (row-major index -> stream position), same layout: k_dct256 and the scaled IDCT (idct_scaled.cu)
+        std::vector<int32_t> inv(ztotal);
+        for (int lg = 1; lg <= 8; lg++) {
+            const size_t o = h->zz_dev[lg] - h->zz_all_dev;
+            for (int i = 0; i < (1 << (2 * lg)); i++) inv[o + zh[o + i]] = i;
+        }
+        AEAJ_CUDA(cudaMalloc(&h->izz_all_dev, ztotal * sizeof(int32_t)));
+        AEAJ_CUDA(cudaMemcpy(h->izz_all_dev, inv.data(), ztotal * sizeof(int32_t), cudaMemcpyHostToDevice));
+        for (int k = 0; k < 9; k++) h->izz_dev[k] = k ? h->izz_all_dev + (h->zz_dev[k] - h->zz_all_dev) : nullptr;
+        h->izz256_dev = h->izz_dev[8];
     }
     AEAJ_CUDA(cudaMemcpy(h->zz_all_dev, zh, ztotal * sizeof(int32_t), cudaMemcpyHostToDevice));
     free(zh);

@@ -141,9 +141,11 @@ class Jpeg:
             raise ValueError("Input array must be a 3D.")
         return self.compress_batch([img])[0]
 
-    def decompress(self, img_encoded: bytes) -> Image:
-        """Decode an .ajpg stream (jpeg.py:274-297); reconfigures itself from the stream header."""
-        return self.decompress_batch([img_encoded])[0]
+    def decompress(self, img_encoded: bytes, scale: int = 1) -> Image:
+        """Decode an .ajpg stream (jpeg.py:274-297); reconfigures itself from the stream header.
+        scale: 2, 4 or 8 decode a (ceil(H/scale), ceil(W/scale), 3) image straight from the coefficients (previews,
+        thumbnails; include/aeaj.h, aeaj_decode_scaled); layer_shape stays the file's full size."""
+        return self.decompress_batch([img_encoded], scale=scale)[0]
 
     def compress_batch(self, imgs: Sequence[Image]) -> List[bytes]:
         """Same-shape images are encoded in one device batch; others fall back to one batch each."""
@@ -185,12 +187,14 @@ class Jpeg:
                 out[i] = self._entropy_encode(downloaded[k], (H, W), imgs[i].extension, streams)
         return out
 
-    def decompress_uint8(self, img_encoded: bytes) -> np.ndarray:
+    def decompress_uint8(self, img_encoded: bytes, scale: int = 1) -> np.ndarray:
         """decompress(...).get_uint8() with the (data * 255).astype(uint8) step (image.py:127) done by the decoding
         kernel: a quarter of the device-to-host bytes when only 8-bit pixels are wanted (Image.save, previews)."""
-        return self.decompress_batch([img_encoded], as_uint8=True)[0]
+        return self.decompress_batch([img_encoded], as_uint8=True, scale=scale)[0]
 
-    def decompress_batch(self, streams: Sequence[bytes], as_uint8: bool = False) -> List[Image]:
+    def decompress_batch(self, streams: Sequence[bytes], as_uint8: bool = False, scale: int = 1) -> List[Image]:
+        if scale not in (1, 2, 4, 8):
+            raise ValueError("scale must be 1, 2, 4 or 8")
         device = self.deflate == "device"
         parsed = [self._entropy_decode(b, inflate=not device) for b in streams]
         out: List[Optional[Image]] = [None] * len(streams)
@@ -206,12 +210,13 @@ class Jpeg:
                 coef = inf.coef
             else:
                 coef, leaves, counts = codec.upload_for_decode(layers, len(idxs), H, W, space, q, b)
-            rgb = codec.decode(coef, leaves, counts, len(idxs), H, W, space, q, b, zigzag=True, out="u8" if as_uint8 else "f32").cpu().numpy()
+            rgb = codec.decode(coef, leaves, counts, len(idxs), H, W, space, q, b, zigzag=True, out="u8" if as_uint8 else "f32",
+                               scale=scale).cpu().numpy()
             if device:
                 _raise_inflate_status(inf.status.cpu().numpy())
             codec.check_status(codec.last_decode_status, "decode")
             for k, i in enumerate(idxs):
-                out[i] = rgb[k] if as_uint8 else Image.from_array(rgb[k].reshape(-1, 3), (H, W, 3), parsed[i]["extension"])
+                out[i] = rgb[k] if as_uint8 else Image.from_array(rgb[k].reshape(-1, 3), rgb.shape[1:], parsed[i]["extension"])
         last = parsed[-1]
         self.extension = last["extension"]
         self.update_settings(JpegCompressionSettings(last["space"], last["quality"], last["blocks"]), (last["H"], last["W"]))

@@ -181,6 +181,23 @@ typedef struct {
 AEAJ_API int aeaj_encode(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, void* stream);
 AEAJ_API int aeaj_decode(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream);
 
+/* Scaled decode: the image at 1/scale of its size, scale in {1, 2, 4, 8} -- previews and thumbnails without decoding, moving
+ * and shrinking every pixel (libjpeg's scale_num / scale_denom, PIL's draft()).  The output is ceil(H/scale) x ceil(W/scale).
+ * With m = min(scale, block_min), each leaf (x, y, s) decodes to (s/m) x (s/m) samples of a 1/m layer from the top-left
+ * t x t (t = s/m) of its dequantised coefficients Y: (1/m) C_t^T Y C_t / scale_l + mid_l, C_t the orthonormal t-point DCT (the
+ * 1/m keeps each leaf's mean); where scale > block_min, each sample of the 1/scale layer is the mean of the in-bounds samples
+ * of its leaf-aligned (scale/m) x (scale/m) group.  The layers then go through aeaj_decode's upsample + inverse colour kernel.
+ * There is no reference counterpart: the reference always decodes at full size (jpeg.py:274-297).
+ * aeaj_decode_scaled_geometry: the output size, the final layer sizes and the bytes of the caller-owned device scratch the call
+ * needs (separate from the plan workspace; 0 for scale 1).  aeaj_decode_scaled: io->rgb / io->rgb_u8 [batch][out_h][out_w][3];
+ * io->tap_layers[l] (optional): the final scaled layers [batch][layer_h[l]][layer_w[l]]; io->status as in aeaj_decode.
+ * scale 1 runs aeaj_decode's schedule (scratch may be NULL).  AEAJ_EINVAL for another scale, a plan with peers, or NULL buffers.
+ * Asynchronous on `stream`, no host sync; after the first call on a plan, steady-state calls issue no host-to-device copy and
+ * can be captured in a CUDA graph. */
+AEAJ_API int aeaj_decode_scaled_geometry(const aeaj_plan* p, int scale, int* out_h, int* out_w, int layer_h[3], int layer_w[3],
+                                         int64_t* scratch_bytes);
+AEAJ_API int aeaj_decode_scaled(aeaj_plan* p, const aeaj_decode_io* io, int scale, void* workspace, void* scratch, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * halo-split of ONE large image over several GPUs of one node (SURVEY 8e, config C4) into `bands` row bands: band b is the
  * full-resolution rows [b*H/bands, (b+1)*H/bands).  H must be a multiple of `bands`; with more than one band the plan holds
