@@ -110,24 +110,23 @@ class _Job:
 
 @dataclass
 class _Scaled:
-    """A plan's buffers for decode(..., scale=k), k > 1 (aeaj_decode_scaled)."""
-    out_h: int
-    out_w: int
-    layer_h: Tuple[int, int, int]  # the final scaled layers
+    """A plan's output buffers for decode(..., scale=k) (aeaj_decode_scaled_geometry)."""
+    layer_h: Tuple[int, int, int]  # the final layers (taps)
     layer_w: Tuple[int, int, int]
-    scratch: torch.Tensor          # the scaled layers of the call
-    rgb_out: torch.Tensor          # float32 [B, out_h, out_w, 3]
+    rgb_out: torch.Tensor          # float32 [B, ceil(H/k), ceil(W/k), 3]
     rgb8_out: Optional[torch.Tensor] = None
+    scratch: Optional[torch.Tensor] = None        # k > 1: the scaled layers of the call
 
 
 @dataclass
 class _Plan:
+    """One cached plan.  Its device buffers (all but an encode's per-call taps) come from DeviceCodec._alloc, which counts them
+    in `nbytes`: the plan cache's MAX_PLAN_BYTES bound holds only if they all do."""
+    key: tuple
     ptr: C.c_void_p
     info: native.PlanInfo
-    workspace: torch.Tensor
-    out: EncodedBatch
-    rgb_out: torch.Tensor
-    rgb8_out: Optional[torch.Tensor] = None
+    workspace: Optional[torch.Tensor] = None
+    out: Optional[EncodedBatch] = None
     qkey: Optional[tuple] = None
     staging: Optional[_HostStaging] = None
     dec_status: Optional[torch.Tensor] = None     # int32 [64]: [2] tensor-IDCT timeout flag, [3] leaves rejected by the device guard
@@ -136,8 +135,16 @@ class _Plan:
     deflate_scratch: Optional[torch.Tensor] = None
     inflated: Optional[InflatedBatch] = None
     inflate_scratch: Optional[torch.Tensor] = None
-    scaled: Dict[int, _Scaled] = field(default_factory=dict)
+    scaled: Dict[int, _Scaled] = field(default_factory=dict)   # decode outputs per scale; [1] exists from the start
     nbytes: int = 0
+
+    @property
+    def rgb_out(self) -> torch.Tensor:
+        return self.scaled[1].rgb_out
+
+    @property
+    def rgb8_out(self) -> Optional[torch.Tensor]:
+        return self.scaled[1].rgb8_out
 
 
 class DeviceCodec:
@@ -169,7 +176,6 @@ class DeviceCodec:
     def _plan(self, B, H, W, space, brange, qrange, instance: int = 0) -> _Plan:
         key = (B, H, W, space, tuple(brange), instance)
         p = self._plans.get(key)
-        dev = torch.device("cuda", self.device)
         if p is not None:
             self._plans.move_to_end(key)
         if p is None:
@@ -180,16 +186,16 @@ class DeviceCodec:
                          "aeaj_plan_create")
             info = native.PlanInfo()
             native.check(self.lib.aeaj_plan_get_info(ptr, C.byref(info)), "aeaj_plan_get_info")
-            ws = torch.empty(int(info.workspace_bytes), dtype=torch.uint8, device=dev)
-            out = EncodedBatch(
-                coef=[torch.empty((B, int(info.cap_coef[l])), dtype=torch.int32, device=dev) for l in range(3)],
-                leaves=[torch.empty((B, int(info.cap_leaves[l]), 4), dtype=torch.int32, device=dev) for l in range(3)],
-                states=[torch.empty((B, int(info.cap_states[l])), dtype=torch.uint8, device=dev) for l in range(3)],
-                counts=torch.zeros((B, 3, 4), dtype=torch.int32, device=dev),
-                status=torch.zeros(64, dtype=torch.int32, device=dev), shape=(B, H, W))
-            rgb_out = torch.empty((B, H, W, 3), dtype=torch.float32, device=dev)
-            p = _Plan(ptr, info, ws, out, rgb_out, dec_status=torch.zeros(64, dtype=torch.int32, device=dev))
-            p.nbytes = ws.numel() + rgb_out.numel() * 4 + sum(t.numel() * t.element_size() for t in out.coef + out.leaves + out.states)
+            p = _Plan(key, ptr, info)
+            p.workspace = self._alloc(p, int(info.workspace_bytes), torch.uint8)
+            p.out = EncodedBatch(
+                coef=[self._alloc(p, (B, int(info.cap_coef[l])), torch.int32) for l in range(3)],
+                leaves=[self._alloc(p, (B, int(info.cap_leaves[l]), 4), torch.int32) for l in range(3)],
+                states=[self._alloc(p, (B, int(info.cap_states[l])), torch.uint8) for l in range(3)],
+                counts=self._alloc(p, (B, 3, 4), torch.int32, zero=True),
+                status=self._alloc(p, 64, torch.int32, zero=True), shape=(B, H, W))
+            p.dec_status = self._alloc(p, 64, torch.int32, zero=True)
+            self._scaled(p, 1)
             self._plans[key] = p
             self._evict(keep=key)
         qkey = tuple(qrange)
@@ -201,6 +207,13 @@ class DeviceCodec:
             torch.cuda.current_stream().synchronize()     # `flat` is pageable host memory
             p.qkey = qkey
         return p
+
+    def _alloc(self, p: _Plan, shape, dtype: torch.dtype, zero: bool = False) -> torch.Tensor:
+        """A device buffer that plan `p` holds: counted in p.nbytes, then the cache is brought back within its bounds."""
+        t = (torch.zeros if zero else torch.empty)(shape, dtype=dtype, device=torch.device("cuda", self.device))
+        p.nbytes += t.numel() * t.element_size()
+        self._evict(keep=p.key)
+        return t
 
     def _evict(self, keep=None):
         """Bound the plan cache (a dataset of mixed image sizes would otherwise hold a workspace per distinct shape until OOM)."""
@@ -267,7 +280,7 @@ class DeviceCodec:
         o.zigzag = bool(stream)
         if stream:
             if o.packed_states is None:
-                o.packed_states = [torch.empty((B, (int(p.info.cap_states[l]) + 3) // 4), dtype=torch.uint8, device=rgb.device) for l in range(3)]
+                o.packed_states = [self._alloc(p, (B, (int(p.info.cap_states[l]) + 3) // 4), torch.uint8) for l in range(3)]
             for l in range(3):
                 io.packed_states[l] = o.packed_states[l].data_ptr()
         if taps:
@@ -294,53 +307,9 @@ class DeviceCodec:
         if scale not in (1, 2, 4, 8):
             raise ValueError("scale must be 1, 2, 4 or 8")
         p = self._plan(B, H, W, space, brange, qrange, instance)
-        if scale != 1:
-            return self._decode_scaled(p, coef, leaves, counts, B, taps, zigzag, out, scale)
-        native.check(self.lib.aeaj_plan_set_stream_layout(p.ptr, int(zigzag)), "aeaj_plan_set_stream_layout")
-        native.check(self.lib.aeaj_plan_set_tensor_dct(p.ptr, self._tensor_mask()), "aeaj_plan_set_tensor_dct")
-        io = native.DecodeIO()
-        for l in range(3):
-            if coef[l].shape[1] != p.info.cap_coef[l] or leaves[l].shape[1] != p.info.cap_leaves[l]:
-                raise ValueError("decode buffers must use the plan's capacities")
-            io.coef[l] = coef[l].data_ptr()
-            io.leaves[l] = leaves[l].data_ptr()
-        io.counts = counts.data_ptr()
-        if out != "u8":
-            io.rgb = p.rgb_out.data_ptr()
-        if out != "f32":
-            if p.rgb8_out is None:
-                p.rgb8_out = torch.empty((B, H, W, 3), dtype=torch.uint8, device=p.rgb_out.device)
-            io.rgb_u8 = p.rgb8_out.data_ptr()
-        io.status = p.dec_status.data_ptr()
-        self.last_decode_status = p.dec_status
-        tl = None
-        if taps:
-            tl = [torch.empty((B, p.info.layer_h[l], p.info.layer_w[l]), dtype=torch.float32, device=p.rgb_out.device) for l in range(3)]
-            for l in range(3):
-                io.tap_layers[l] = tl[l].data_ptr()
-        native.check(self.lib.aeaj_decode(p.ptr, C.byref(io), p.workspace.data_ptr(), _stream()), "aeaj_decode")
-        self.last_launches = self.lib.aeaj_plan_last_launches(p.ptr)
-        res = p.rgb_out if out == "f32" else (p.rgb8_out if out == "u8" else (p.rgb_out, p.rgb8_out))
-        return (res, tl) if taps else res
-
-    def _scaled(self, p: _Plan, scale: int) -> _Scaled:
-        sc = p.scaled.get(scale)
-        if sc is None:
-            oh, ow, scratch = C.c_int(), C.c_int(), C.c_int64()
-            lh, lw = (C.c_int * 3)(), (C.c_int * 3)()
-            native.check(self.lib.aeaj_decode_scaled_geometry(p.ptr, scale, C.byref(oh), C.byref(ow), lh, lw, C.byref(scratch)),
-                         "aeaj_decode_scaled_geometry")
-            dev = p.rgb_out.device
-            sc = _Scaled(oh.value, ow.value, tuple(lh), tuple(lw), torch.empty(int(scratch.value), dtype=torch.uint8, device=dev),
-                         torch.empty((p.info.batch, oh.value, ow.value, 3), dtype=torch.float32, device=dev))
-            p.scaled[scale] = sc
-            p.nbytes += sc.scratch.numel() + sc.rgb_out.numel() * 4
-            self._evict(keep=next(k for k, v in self._plans.items() if v is p))
-        return sc
-
-    def _decode_scaled(self, p: _Plan, coef, leaves, counts, B, taps, zigzag, out, scale):
         sc = self._scaled(p, scale)
         native.check(self.lib.aeaj_plan_set_stream_layout(p.ptr, int(zigzag)), "aeaj_plan_set_stream_layout")
+        native.check(self.lib.aeaj_plan_set_tensor_dct(p.ptr, self._tensor_mask()), "aeaj_plan_set_tensor_dct")
         io = native.DecodeIO()
         for l in range(3):
             if coef[l].shape[1] != p.info.cap_coef[l] or leaves[l].shape[1] != p.info.cap_leaves[l]:
@@ -352,8 +321,7 @@ class DeviceCodec:
             io.rgb = sc.rgb_out.data_ptr()
         if out != "f32":
             if sc.rgb8_out is None:
-                sc.rgb8_out = torch.empty(sc.rgb_out.shape, dtype=torch.uint8, device=sc.rgb_out.device)
-                p.nbytes += sc.rgb8_out.numel()
+                sc.rgb8_out = self._alloc(p, sc.rgb_out.shape, torch.uint8)
             io.rgb_u8 = sc.rgb8_out.data_ptr()
         io.status = p.dec_status.data_ptr()
         self.last_decode_status = p.dec_status
@@ -362,22 +330,36 @@ class DeviceCodec:
             tl = [torch.empty((B, sc.layer_h[l], sc.layer_w[l]), dtype=torch.float32, device=sc.rgb_out.device) for l in range(3)]
             for l in range(3):
                 io.tap_layers[l] = tl[l].data_ptr()
-        native.check(self.lib.aeaj_decode_scaled(p.ptr, C.byref(io), scale, p.workspace.data_ptr(), sc.scratch.data_ptr(), _stream()),
-                     "aeaj_decode_scaled")
+        if scale == 1:          # aeaj_decode: the B = 1 plans aeaj/tiled.py shares may have peers, which aeaj_decode_scaled rejects
+            native.check(self.lib.aeaj_decode(p.ptr, C.byref(io), p.workspace.data_ptr(), _stream()), "aeaj_decode")
+        else:
+            native.check(self.lib.aeaj_decode_scaled(p.ptr, C.byref(io), scale, p.workspace.data_ptr(), sc.scratch.data_ptr(), _stream()),
+                         "aeaj_decode_scaled")
         self.last_launches = self.lib.aeaj_plan_last_launches(p.ptr)
         res = sc.rgb_out if out == "f32" else (sc.rgb8_out if out == "u8" else (sc.rgb_out, sc.rgb8_out))
         return (res, tl) if taps else res
+
+    def _scaled(self, p: _Plan, scale: int) -> _Scaled:
+        sc = p.scaled.get(scale)
+        if sc is None:
+            oh, ow, scratch = C.c_int(), C.c_int(), C.c_int64()
+            lh, lw = (C.c_int * 3)(), (C.c_int * 3)()
+            native.check(self.lib.aeaj_decode_scaled_geometry(p.ptr, scale, C.byref(oh), C.byref(ow), lh, lw, C.byref(scratch)),
+                         "aeaj_decode_scaled_geometry")
+            sc = p.scaled[scale] = _Scaled(tuple(lh), tuple(lw), self._alloc(p, (p.info.batch, oh.value, ow.value, 3), torch.float32))
+            if scratch.value:
+                sc.scratch = self._alloc(p, int(scratch.value), torch.uint8)
+        return sc
 
     # ------------------------------------------------------------------------------------------
     # packed coefficient streams (PCIe form)
     # ------------------------------------------------------------------------------------------
     def _packed(self, p: _Plan) -> PackedBatch:
         if p.packed is None:
-            B, dev = p.info.batch, p.rgb_out.device
-            p.packed = PackedBatch(mask=[torch.empty((B, int(p.info.cap_coef[l]) // 32 + 1), dtype=torch.int32, device=dev) for l in range(3)],
-                                   vals=[torch.empty((B, int(p.info.cap_coef[l])), dtype=torch.int16, device=dev) for l in range(3)],
-                                   counts=torch.zeros((B, 3, 4), dtype=torch.int32, device=dev))
-            p.nbytes += sum(t.numel() * t.element_size() for t in p.packed.mask + p.packed.vals)
+            B = p.info.batch
+            p.packed = PackedBatch(mask=[self._alloc(p, (B, int(p.info.cap_coef[l]) // 32 + 1), torch.int32) for l in range(3)],
+                                   vals=[self._alloc(p, (B, int(p.info.cap_coef[l])), torch.int16) for l in range(3)],
+                                   counts=self._alloc(p, (B, 3, 4), torch.int32, zero=True))
         return p.packed
 
     def pack(self, enc: EncodedBatch, space, qrange, brange, instance: int = 0) -> PackedBatch:
@@ -396,16 +378,14 @@ class DeviceCodec:
 
     def _deflated(self, p: _Plan) -> DeflatedBatch:
         if p.deflated is None:
-            B, dev = p.info.batch, p.rgb_out.device
+            B = p.info.batch
             cap = (C.c_int64 * 3)()
             scratch = C.c_int64()
             native.check(self.lib.aeaj_deflate_caps(p.ptr, cap, C.byref(scratch)), "aeaj_deflate_caps")
-            p.deflated = DeflatedBatch(out=[torch.empty((B, int(cap[l])), dtype=torch.uint8, device=dev) for l in range(3)],
-                                       lengths=torch.zeros((B, 3), dtype=torch.int32, device=dev),
-                                       status=torch.zeros(4, dtype=torch.int32, device=dev))
-            p.deflate_scratch = torch.empty(int(scratch.value), dtype=torch.uint8, device=dev)
-            p.nbytes += sum(t.numel() for t in p.deflated.out) + p.deflate_scratch.numel()
-            self._evict(keep=next(k for k, v in self._plans.items() if v is p))
+            p.deflated = DeflatedBatch(out=[self._alloc(p, (B, int(cap[l])), torch.uint8) for l in range(3)],
+                                       lengths=self._alloc(p, (B, 3), torch.int32, zero=True),
+                                       status=self._alloc(p, 4, torch.int32, zero=True))
+            p.deflate_scratch = self._alloc(p, int(scratch.value), torch.uint8)
         return p.deflated
 
     def deflate(self, enc: EncodedBatch, space, qrange, brange, instance: int = 0) -> DeflatedBatch:
@@ -458,19 +438,16 @@ class DeviceCodec:
         for t, dt in ((offsets, torch.int64), (lengths, torch.int64), (counts, torch.int32)):
             if t.dtype != dt or not t.is_cuda or not t.is_contiguous() or t.shape[:2] != (B, 3):
                 raise TypeError("offsets / lengths: int64 [B, 3], counts: int32 [B, 3, 4], contiguous CUDA tensors")
-        dev = p.rgb_out.device
         if p.inflated is None:
-            p.inflated = InflatedBatch(coef=p.out.coef, status=torch.zeros((B, 3), dtype=torch.int32, device=dev),
-                                       out_bytes=torch.zeros((B, 3), dtype=torch.int64, device=dev),
-                                       segments=torch.zeros((B, 3), dtype=torch.int32, device=dev))
+            p.inflated = InflatedBatch(coef=p.out.coef, status=self._alloc(p, (B, 3), torch.int32, zero=True),
+                                       out_bytes=self._alloc(p, (B, 3), torch.int64, zero=True),
+                                       segments=self._alloc(p, (B, 3), torch.int32, zero=True))
         need = C.c_int64()
         native.check(self.lib.aeaj_inflate_scratch_bytes(p.ptr, zbuf.numel(), C.byref(need)), "aeaj_inflate_scratch_bytes")
         if p.inflate_scratch is None or p.inflate_scratch.numel() < need.value:
             if p.inflate_scratch is not None:
                 p.nbytes -= p.inflate_scratch.numel()
-            p.inflate_scratch = torch.empty(int(need.value), dtype=torch.uint8, device=dev)
-            p.nbytes += p.inflate_scratch.numel()
-            self._evict(keep=next(k for k, v in self._plans.items() if v is p))
+            p.inflate_scratch = self._alloc(p, int(need.value), torch.uint8)
         ib = p.inflated
         io = native.InflateIO()
         io.inp = zbuf.data_ptr() if zbuf.numel() else None
@@ -635,7 +612,7 @@ class DeviceCodec:
             for l in range(3):
                 cc = int(p.info.cap_coef[l])
                 n += (cc // 32 + 1) * 4 + cc * 2 + int(p.info.cap_leaves[l]) * 16 + int(p.info.cap_states[l]) + 4 * 32
-            st.arena_dev = torch.empty(n, dtype=torch.uint8, device=p.rgb_out.device)
+            st.arena_dev = self._alloc(p, n, torch.uint8)
             st.arena_host = torch.empty(n, dtype=torch.uint8).pin_memory()
         return st.arena_dev, st.arena_host
 
@@ -681,7 +658,7 @@ class DeviceCodec:
             st = self._host_staging(p)
             src = st.rgb_dev.get(host_in.dtype)
             if src is None:
-                src = st.rgb_dev[host_in.dtype] = torch.empty((1, H, W, 3), dtype=host_in.dtype, device=dev)
+                src = st.rgb_dev[host_in.dtype] = self._alloc(p, (1, H, W, 3), host_in.dtype)
             f = k % F
             # phase A: upload + encode + counts
             with torch.cuda.stream(self._streams[slot]):

@@ -417,7 +417,8 @@ struct aeaj_plan {
     aeaj_plan_info info;
     int nplanes, lg_min, lg_max;
     std::vector<PlaneDesc> planes;       // host copy, index b*3 + l
-    DescTable<PlaneDesc> planes_tab;
+    // one table per call kind (encode; decode per log2(scale)): calls that alternate between kinds upload nothing
+    DescTable<PlaneDesc> enc_tab, dec_tab[4];
     int ntiles, ring_cap;
     long long* class_off_dev;
     ClassGeom cg;
@@ -431,8 +432,6 @@ struct aeaj_plan {
     DescTable<DeflatePlane> deflate_tab;
     std::vector<InflatePlane> if_planes;
     DescTable<InflatePlane> inflate_tab;
-    std::vector<PlaneDesc> scaled_planes;  // aeaj_decode_scaled: the planes with layer_f32 on the 1/m planes of the caller's scratch
-    DescTable<PlaneDesc> scaled_tab[4];    // one per log2(scale): decodes alternating between scales upload nothing either
     // one image over several GPUs (peer.cu): the other ranks' workspaces / barrier flags, opened through CUDA IPC by the caller
     PeerSet peers = {1, 0, {0}};
     void* peer_ws[AEAJ_MAX_PEERS] = {nullptr};
@@ -662,12 +661,12 @@ extern "C" int aeaj_plan_set_qtables(aeaj_plan* p, const int32_t* tables, size_t
     return 0;
 }
 
-static int plan_push_planes(aeaj_plan* p, cudaStream_t st, PlaneDesc*& planes_dev) {
+static int plan_push_planes(aeaj_plan* p, DescTable<PlaneDesc>& tab, cudaStream_t st, PlaneDesc*& planes_dev) {
     for (auto& P : p->planes) {
         P.zigzag = p->zigzag;
         for (int k = 0; k < 9; k++) P.zz[k] = p->h->zz_dev[k];
     }
-    return p->planes_tab.push(p->planes, st, planes_dev);
+    return tab.push(p->planes, st, planes_dev);
 }
 
 // full-res luma rows [band0, band1) -> rows of every layer (chroma rows scale with the subsampling ratio)
@@ -733,7 +732,7 @@ static int encode_impl(aeaj_plan* p, const aeaj_encode_io* io, void* workspace, 
     }
     int rc = set_band(p, band0, band1); if (rc) return rc;
     PlaneDesc* Pd;
-    rc = plan_push_planes(p, st, Pd); if (rc) return rc;
+    rc = plan_push_planes(p, p->enc_tab, st, Pd); if (rc) return rc;
     p->ev_n = 0; p->ev_stream = st; p->mark("start");
     // a whole-image call on a plan that is one rank of a halo-split is a plain single-GPU call: no partial histograms to sum
     const bool whole = band0 == 0 && (band1 < 0 || band1 == p->info.height);
@@ -810,63 +809,7 @@ extern "C" int aeaj_encode(aeaj_plan* p, const aeaj_encode_io* io, void* workspa
     return encode_impl(p, io, workspace, ST(stream), (1u << (AEAJ_PHASE_DCT + 1)) - 1, 0, -1);      // every phase, whole image
 }
 
-static int decode_impl(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, cudaStream_t st, unsigned phases, int band0, int band1) {
-    AEAJ_REQUIRE(p && io && workspace && (io->rgb || io->rgb_u8) && io->counts, "aeaj_decode: bad arguments (rgb or rgb_u8 required)");
-    AEAJ_REQUIRE(p->qtab_dev, "aeaj_decode: quantisation tables not set (aeaj_plan_set_qtables)");
-    aeaj_handle* h = p->h;
-    const int B = p->info.batch, NP = p->nplanes;
-    int launches = 0;
-    PlanAux A;
-    plan_carve(p, workspace, A);
-    for (int l = 0; l < 3; l++) {
-        AEAJ_REQUIRE(io->coef[l] && io->leaves[l], "aeaj_decode: NULL input buffer");
-        for (int i = 0; i < B; i++) {
-            PlaneDesc& P = p->planes[i * 3 + l];
-            P.coef = (int32_t*)io->coef[l] + (size_t)i * p->info.cap_coef[l];
-            P.leaves = (int32_t*)io->leaves[l] + (size_t)i * p->info.cap_leaves[l] * 4;
-            P.counts = (int32_t*)io->counts + ((size_t)i * 3 + l) * 4;
-            P.packed_states = nullptr;
-            P.tap_edge = nullptr;
-        }
-    }
-    int rc = set_band(p, band0, band1); if (rc) return rc;
-    PlaneDesc* Pd;
-    rc = plan_push_planes(p, st, Pd); if (rc) return rc;
-    p->ev_n = 0; p->ev_stream = st; p->mark("start");
-    if (phases & (1u << AEAJ_DPHASE_IDCT)) {
-        AEAJ_CUDA(cudaMemsetAsync(A.class_counts, 0, 16 * sizeof(int), st));
-        rc = launch_bucket_leaves(Pd, p->planes.data(), NP, A.class_lists, A.class_counts, p->class_off_dev, p->lg_min, p->lg_max, st);
-        if (rc) return rc;
-        launches++;
-        p->mark("bucket_leaves");
-        rc = launch_dequant_idct(h, Pd, A.class_lists, A.class_counts, p->cg.off, p->cg.cap, p->lg_min, p->lg_max, st, &launches,
-                                 plan_mark_cb, p, p->tensor_dct, A.scratch256);
-        if (rc) return rc;
-        if (io->status) {
-            AEAJ_CUDA(cudaMemcpyAsync(io->status + 2, h->tc_err_dev, sizeof(int), cudaMemcpyDeviceToDevice, st));
-            AEAJ_CUDA(cudaMemcpyAsync(io->status + 3, A.class_counts + 15, sizeof(int), cudaMemcpyDeviceToDevice, st));
-        }
-        for (int l = 0; l < 3; l++)
-            if (io->tap_layers[l])
-                AEAJ_CUDA(cudaMemcpyAsync(io->tap_layers[l], p->planes[l].layer_f32, sizeof(float) * (size_t)B * p->info.layer_h[l] * p->info.layer_w[l],
-                                          cudaMemcpyDeviceToDevice, st));
-    }
-    if (phases & (1u << AEAJ_DPHASE_COLOR)) {
-        rc = launch_upsample_color_inverse(h, p->info.space, p->planes.data(), B, p->info.height, p->info.width, io->rgb, io->rgb_u8, st, band0, band1);
-        if (rc) return rc;
-        launches++;
-        p->mark("upsample_color_inverse");
-    }
-    p->last_launches = launches;
-    return 0;
-}
-extern "C" int aeaj_decode(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream) {
-    return decode_impl(p, io, workspace, ST(stream), 0x3u, 0, -1);
-}
-
-// ---------------------------------------------------------------------------------------------
 // scaled decode (idct_scaled.cu): 1/scale of every layer from the top-left coefficients of each leaf
-// ---------------------------------------------------------------------------------------------
 struct ScaledGeom {
     int k, m;                        // scale; the IDCT's own factor min(scale, block_min)
     int out_h, out_w;
@@ -895,6 +838,90 @@ static size_t scaled_carve(const aeaj_plan* p, const ScaledGeom& g, void* scratc
     return b.used() + 256;
 }
 
+// One schedule for every scale.  Scale 1 decodes every leaf into the workspace layers; scale > 1 decodes the top-left
+// coefficients of each leaf into the 1/m planes of the caller's scratch and, where scale > block_min, box-reduces them to 1/scale.
+static int decode_impl(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, int scale, void* scratch, cudaStream_t st,
+                       unsigned phases, int band0, int band1) {
+    AEAJ_REQUIRE(p && io && workspace && (io->rgb || io->rgb_u8) && io->counts, "aeaj_decode: bad arguments (rgb or rgb_u8 required)");
+    ScaledGeom g;
+    int rc = scaled_geom(p, scale, g); if (rc) return rc;
+    AEAJ_REQUIRE(scale == 1 || scratch, "aeaj_decode_scaled: NULL scratch");
+    AEAJ_REQUIRE(p->qtab_dev, "aeaj_decode: quantisation tables not set (aeaj_plan_set_qtables)");
+    aeaj_handle* h = p->h;
+    const int B = p->info.batch, NP = p->nplanes;
+    int launches = 0;
+    PlanAux A;
+    plan_carve(p, workspace, A);
+    float* mp[3]; float* kp[3];          // the layers the IDCT writes, and the final layers (taps, colour phase)
+    scaled_carve(p, g, scratch, mp, kp);
+    for (int l = 0; l < 3; l++) {
+        AEAJ_REQUIRE(io->coef[l] && io->leaves[l], "aeaj_decode: NULL input buffer");
+        if (scale == 1) kp[l] = p->planes[l].layer_f32;
+        for (int i = 0; i < B; i++) {
+            PlaneDesc& P = p->planes[i * 3 + l];
+            P.coef = (int32_t*)io->coef[l] + (size_t)i * p->info.cap_coef[l];
+            P.leaves = (int32_t*)io->leaves[l] + (size_t)i * p->info.cap_leaves[l] * 4;
+            P.counts = (int32_t*)io->counts + ((size_t)i * 3 + l) * 4;
+            P.packed_states = nullptr;
+            P.tap_edge = nullptr;
+            if (scale > 1) P.layer_f32 = mp[l] + (size_t)i * g.hm[l] * g.wm[l];
+        }
+    }
+    rc = set_band(p, band0, band1); if (rc) return rc;
+    PlaneDesc* Pd;
+    rc = plan_push_planes(p, p->dec_tab[ilog2i(scale)], st, Pd); if (rc) return rc;
+    p->ev_n = 0; p->ev_stream = st; p->mark("start");
+    if (phases & (1u << AEAJ_DPHASE_IDCT)) {
+        AEAJ_CUDA(cudaMemsetAsync(A.class_counts, 0, 16 * sizeof(int), st));
+        rc = launch_bucket_leaves(Pd, p->planes.data(), NP, A.class_lists, A.class_counts, p->class_off_dev, p->lg_min, p->lg_max, st);
+        if (rc) return rc;
+        launches++;
+        p->mark("bucket_leaves");
+        if (scale == 1) {
+            rc = launch_dequant_idct(h, Pd, A.class_lists, A.class_counts, p->cg.off, p->cg.cap, p->lg_min, p->lg_max, st, &launches,
+                                     plan_mark_cb, p, p->tensor_dct, A.scratch256);
+            if (rc) return rc;
+        } else {
+            rc = launch_idct_scaled(h, Pd, A.class_lists, A.class_counts, p->cg.off, p->cg.cap, p->lg_min, p->lg_max, g.m, st, &launches);
+            if (rc) return rc;
+            p->mark("idct_scaled");
+            if (g.k > g.m) {
+                for (int l = 0; l < 3; l++) {
+                    rc = launch_box_reduce(mp[l], g.hm[l], g.wm[l], kp[l], g.hk[l], g.wk[l], g.k / g.m, B, st); if (rc) return rc;
+                    launches++;
+                }
+                p->mark("box_reduce");
+            }
+        }
+        if (io->status) {
+            AEAJ_CUDA(cudaMemcpyAsync(io->status + 2, h->tc_err_dev, sizeof(int), cudaMemcpyDeviceToDevice, st));
+            AEAJ_CUDA(cudaMemcpyAsync(io->status + 3, A.class_counts + 15, sizeof(int), cudaMemcpyDeviceToDevice, st));
+        }
+        for (int l = 0; l < 3; l++)
+            if (io->tap_layers[l])
+                AEAJ_CUDA(cudaMemcpyAsync(io->tap_layers[l], kp[l], sizeof(float) * (size_t)B * g.hk[l] * g.wk[l], cudaMemcpyDeviceToDevice, st));
+    }
+    if (phases & (1u << AEAJ_DPHASE_COLOR)) {
+        // the colour kernel reads the layers through host descriptors; at scale > 1, ones of the 1/scale geometry
+        PlaneDesc tail[3];
+        for (int l = 0; l < 3 && scale > 1; l++) {
+            memset(&tail[l], 0, sizeof tail[l]);
+            tail[l].h = g.hk[l]; tail[l].w = g.wk[l]; tail[l].ry0 = 0; tail[l].ry1 = g.hk[l]; tail[l].layer = l;
+            tail[l].layer_f32 = kp[l];
+        }
+        rc = launch_upsample_color_inverse(h, p->info.space, scale == 1 ? p->planes.data() : tail, B, g.out_h, g.out_w, io->rgb, io->rgb_u8,
+                                           st, band0, band1);
+        if (rc) return rc;
+        launches++;
+        p->mark("upsample_color_inverse");
+    }
+    p->last_launches = launches;
+    return 0;
+}
+extern "C" int aeaj_decode(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream) {
+    return decode_impl(p, io, workspace, 1, nullptr, ST(stream), 0x3u, 0, -1);
+}
+
 extern "C" int aeaj_decode_scaled_geometry(const aeaj_plan* p, int scale, int* out_h, int* out_w, int layer_h[3], int layer_w[3],
                                            int64_t* scratch_bytes) {
     AEAJ_REQUIRE(p && out_h && out_w && layer_h && layer_w && scratch_bytes, "aeaj_decode_scaled_geometry: bad arguments");
@@ -908,75 +935,9 @@ extern "C" int aeaj_decode_scaled_geometry(const aeaj_plan* p, int scale, int* o
 }
 
 extern "C" int aeaj_decode_scaled(aeaj_plan* p, const aeaj_decode_io* io, int scale, void* workspace, void* scratch, void* stream) {
-    AEAJ_REQUIRE(p && io && workspace && (io->rgb || io->rgb_u8) && io->counts, "aeaj_decode_scaled: bad arguments (rgb or rgb_u8 required)");
+    AEAJ_REQUIRE(p, "aeaj_decode_scaled: NULL plan");
     AEAJ_REQUIRE(p->peers.world == 1, "aeaj_decode_scaled: a plan with peers (multi-GPU halo-split) is not supported");
-    ScaledGeom g;
-    int rc = scaled_geom(p, scale, g); if (rc) return rc;
-    const cudaStream_t st = ST(stream);
-    if (scale == 1) return decode_impl(p, io, workspace, st, 0x3u, 0, -1);
-    AEAJ_REQUIRE(scratch, "aeaj_decode_scaled: NULL scratch");
-    AEAJ_REQUIRE(p->qtab_dev, "aeaj_decode_scaled: quantisation tables not set (aeaj_plan_set_qtables)");
-    aeaj_handle* h = p->h;
-    const int B = p->info.batch, NP = p->nplanes;
-    PlanAux A;
-    plan_carve(p, workspace, A);
-    float* mp[3]; float* kp[3];
-    scaled_carve(p, g, scratch, mp, kp);
-    p->scaled_planes = p->planes;
-    for (int l = 0; l < 3; l++) {
-        AEAJ_REQUIRE(io->coef[l] && io->leaves[l], "aeaj_decode_scaled: NULL input buffer");
-        for (int i = 0; i < B; i++) {
-            PlaneDesc& P = p->scaled_planes[i * 3 + l];
-            P.coef = (int32_t*)io->coef[l] + (size_t)i * p->info.cap_coef[l];
-            P.leaves = (int32_t*)io->leaves[l] + (size_t)i * p->info.cap_leaves[l] * 4;
-            P.counts = (int32_t*)io->counts + ((size_t)i * 3 + l) * 4;
-            P.packed_states = nullptr;
-            P.tap_edge = nullptr;
-            P.ry0 = 0; P.ry1 = P.h; P.peer_up = P.peer_dn = 0;
-            P.zigzag = p->zigzag;
-            for (int k = 0; k < 9; k++) P.zz[k] = h->zz_dev[k];
-            P.layer_f32 = mp[l] + (size_t)i * g.hm[l] * g.wm[l];
-        }
-    }
-    PlaneDesc* Pd;
-    rc = p->scaled_tab[ilog2i(scale)].push(p->scaled_planes, st, Pd); if (rc) return rc;
-    int launches = 0;
-    p->ev_n = 0; p->ev_stream = st; p->mark("start");
-    AEAJ_CUDA(cudaMemsetAsync(A.class_counts, 0, 16 * sizeof(int), st));
-    rc = launch_bucket_leaves(Pd, p->scaled_planes.data(), NP, A.class_lists, A.class_counts, p->class_off_dev, p->lg_min, p->lg_max, st);
-    if (rc) return rc;
-    launches++;
-    p->mark("bucket_leaves");
-    rc = launch_idct_scaled(h, Pd, A.class_lists, A.class_counts, p->cg.off, p->cg.cap, p->lg_min, p->lg_max, g.m, st, &launches);
-    if (rc) return rc;
-    p->mark("idct_scaled");
-    if (g.k > g.m) {
-        for (int l = 0; l < 3; l++) {
-            rc = launch_box_reduce(mp[l], g.hm[l], g.wm[l], kp[l], g.hk[l], g.wk[l], g.k / g.m, B, st); if (rc) return rc;
-            launches++;
-        }
-        p->mark("box_reduce");
-    }
-    if (io->status) {
-        AEAJ_CUDA(cudaMemcpyAsync(io->status + 2, h->tc_err_dev, sizeof(int), cudaMemcpyDeviceToDevice, st));
-        AEAJ_CUDA(cudaMemcpyAsync(io->status + 3, A.class_counts + 15, sizeof(int), cudaMemcpyDeviceToDevice, st));
-    }
-    for (int l = 0; l < 3; l++)
-        if (io->tap_layers[l])
-            AEAJ_CUDA(cudaMemcpyAsync(io->tap_layers[l], kp[l], sizeof(float) * (size_t)B * g.hk[l] * g.wk[l], cudaMemcpyDeviceToDevice, st));
-    // the colour tail reads the 1/scale layers through host descriptors of their final geometry
-    PlaneDesc tail[3];
-    for (int l = 0; l < 3; l++) {
-        memset(&tail[l], 0, sizeof tail[l]);
-        tail[l].h = g.hk[l]; tail[l].w = g.wk[l]; tail[l].ry0 = 0; tail[l].ry1 = g.hk[l]; tail[l].layer = l;
-        tail[l].layer_f32 = kp[l];
-    }
-    rc = launch_upsample_color_inverse(h, p->info.space, tail, B, g.out_h, g.out_w, io->rgb, io->rgb_u8, st);
-    if (rc) return rc;
-    launches++;
-    p->mark("upsample_color_inverse");
-    p->last_launches = launches;
-    return 0;
+    return decode_impl(p, io, workspace, scale, scratch, ST(stream), 0x3u, 0, -1);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1209,7 +1170,8 @@ extern "C" int aeaj_plan_set_peers(aeaj_plan* p, int rank, int world, void* cons
         AEAJ_REQUIRE(p->peer_ws[r] && p->peer_flags[r], "aeaj_plan_set_peers: NULL peer pointer");
         p->peers.delta[r] = (long long)((const char*)p->peer_ws[r] - (const char*)p->peer_ws[rank]);
     }
-    p->planes_tab.forget();
+    p->enc_tab.forget();
+    for (auto& t : p->dec_tab) t.forget();
     if (world > 1 && !p->peer_segs_dev) {
         AEAJ_CUDA(cudaSetDevice(p->h->device));
         AEAJ_CUDA(cudaMalloc(&p->peer_segs_dev, sizeof(PeerSeg) * 64 * 2));
@@ -1310,7 +1272,7 @@ extern "C" int aeaj_encode_halo(aeaj_plan* p, const aeaj_encode_io* io, void* wo
 extern "C" int aeaj_decode_halo(aeaj_plan* p, const aeaj_decode_io* io, void* workspace, void* stream, int bands) {
     const cudaStream_t st = ST(stream);
     return run_halo(p, DECODE_HALO, bands, workspace, st,
-                    [&](unsigned ph, int b0, int b1) { return decode_impl(p, io, workspace, st, ph, b0, b1); });
+                    [&](unsigned ph, int b0, int b1) { return decode_impl(p, io, workspace, 1, nullptr, st, ph, b0, b1); });
 }
 
 // ---------------------------------------------------------------------------------------------

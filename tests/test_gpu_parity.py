@@ -459,6 +459,57 @@ def test_plan_cache_is_bounded():
     assert len(c._plans) == 0
 
 
+def _device_bytes(obj, seen):
+    """bytes of the distinct CUDA tensors reachable from obj through dataclass fields, lists, tuples and dicts"""
+    import dataclasses
+    import torch
+    if isinstance(obj, torch.Tensor):
+        s = obj.untyped_storage()
+        if not obj.is_cuda or s.data_ptr() in seen:
+            return 0
+        seen.add(s.data_ptr())
+        return s.nbytes()
+    if dataclasses.is_dataclass(obj):
+        obj = [getattr(obj, f.name) for f in dataclasses.fields(obj)]
+    elif isinstance(obj, dict):
+        obj = list(obj.values())
+    return sum(_device_bytes(v, seen) for v in obj) if isinstance(obj, (list, tuple)) else 0
+
+
+def test_plan_bytes_count_every_buffer():
+    """the plan-cache bound counts what a plan holds: after each call that allocates plan buffers on first use, every plan's
+    nbytes equals the bytes of the device tensors it references"""
+    from aeaj.codec import DeviceCodec
+    import torch
+    H, W, space, q, b = 136, 200, "YCbCr", (40, 80), (4, 64)
+    c = DeviceCodec(0)
+
+    def check(what):
+        torch.cuda.synchronize()
+        for key, p in c._plans.items():
+            assert p.nbytes == _device_bytes(p, set()), (what, key, p.nbytes, _device_bytes(p, set()))
+
+    rgb = torch.from_numpy(synth(H, W, seed=6)).cuda()
+    enc = c.encode(rgb, space, q, b, stream=True)
+    check("encode(stream=True)")
+    for k in (1, 2, 4, 8):
+        c.decode(enc.coef, enc.leaves, enc.counts, 1, H, W, space, q, b, zigzag=True, out="both", scale=k)
+        check(f"decode(scale={k})")
+    c.pack(enc, space, q, b)
+    check("pack")
+    df = c.deflate(enc, space, q, b)
+    check("deflate")
+    lengths = df.lengths.long()
+    zbuf = torch.cat([df.out[l][0, :int(lengths[0, l])] for l in range(3)])
+    offsets = torch.cumsum(lengths, 1) - lengths
+    c.inflate(zbuf, offsets.contiguous(), lengths.contiguous(), enc.counts, 1, H, W, space, q, b)
+    check("inflate")
+    frames = torch.from_numpy(synth(H, W, seed=7)).unsqueeze(0).pin_memory()
+    c.roundtrip_host_pipelined(frames, torch.empty_like(frames).pin_memory(), space, q, b, slots=2)
+    check("roundtrip_host_pipelined")
+    c.close()
+
+
 def test_two_streams_with_256_leaves(codec):
     """ADVICE r1: the 256 x 256 kernel's intermediate tiles belong to the call -- two plans running concurrently on two
     streams (roundtrip_device) must not share them."""

@@ -445,8 +445,9 @@ def test_einval(codec):
 
 @pytest.mark.gpu
 def test_cuda_graph_capture(codec):
-    """steady-state scaled decodes upload nothing, also when they alternate with full decodes: captured and replayed, they
-    give the eager bits"""
+    """steady-state encodes (.ajpg layout), full and scaled decodes upload nothing, also when they alternate on one plan:
+    captured and replayed, they give the eager bits -- pixels, and the encode's counts, coefficient streams and packed
+    state streams"""
     import torch
     H, W, space, q, b = 272, 480, "YCbCr", (30, 95), (4, 128)
     rgb = torch.from_numpy(synth(H, W, seed=8)).cuda().unsqueeze(0)
@@ -456,18 +457,24 @@ def test_cuda_graph_capture(codec):
     def run():
         enc = codec.encode(rgb, space, q, b, instance=4400, stream=True)
         full = codec.decode(enc.coef, enc.leaves, enc.counts, 1, H, W, space, q, b, instance=4400, zigzag=True)
-        return full, [codec.decode(enc.coef, enc.leaves, enc.counts, 1, H, W, space, q, b, instance=4400, zigzag=True, out="both",
-                                   scale=k) for k in SCALES]
+        return enc, full, [codec.decode(enc.coef, enc.leaves, enc.counts, 1, H, W, space, q, b, instance=4400, zigzag=True,
+                                        out="both", scale=k) for k in SCALES]
+
+    def streams(enc, counts):
+        """the used part of every coefficient stream and packed state stream"""
+        return [t[0, :n] for l in range(3)
+                for t, n in ((enc.coef[l], int(counts[l, 2])), (enc.packed_states[l], (int(counts[l, 1]) + 3) // 4))]
 
     with torch.cuda.stream(side):
-        full, outs = run()
+        enc, full, outs = run()
     torch.cuda.synchronize()
-    eager = [full.clone()] + [t.clone() for pair in outs for t in pair]
+    counts = enc.counts[0].cpu()
+    eager = [enc.counts.clone(), full.clone()] + [t.clone() for pair in outs for t in pair] + [t.clone() for t in streams(enc, counts)]
     g = torch.cuda.CUDAGraph()
     with torch.cuda.graph(g, stream=side):
-        full, outs = run()
-    got = [full] + [t for pair in outs for t in pair]
-    for t in got:
+        enc, full, outs = run()
+    got = [enc.counts, full] + [t for pair in outs for t in pair] + streams(enc, counts)
+    for t in [enc.counts, full] + [t for pair in outs for t in pair] + enc.coef + enc.packed_states:
         t.zero_()
     g.replay()
     torch.cuda.synchronize()
