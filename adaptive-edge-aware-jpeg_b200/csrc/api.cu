@@ -239,6 +239,11 @@ extern "C" int aeaj_cast_u8(aeaj_handle* h, const float* layer, uint8_t* out, si
 
 // ---- single-plane stage workspace -------------------------------------------------------------
 // The call's descriptor and class-offset table live in the workspace too, so that calls on separate workspaces are independent.
+// Alignment the kernels rely on, checked before anything is enqueued: the workspace is carved at 256-byte offsets from `ws`
+// (16-byte vector and descriptor accesses inside it), and the Canny kernels read and write u8 planes as 32-bit words where
+// w % 4 == 0.
+constexpr uintptr_t STAGE_WS_ALIGN = 256, STAGE_PLANE_ALIGN = 4;
+static bool aligned(const void* p, uintptr_t a) { return ((uintptr_t)p & (a - 1)) == 0; }
 struct StageWs {
     PlaneDesc P;
     PlaneDesc* desc;                      // device copy of P
@@ -297,6 +302,7 @@ static int run_clahe(StageWs& S, cudaStream_t st) {
 
 extern "C" int aeaj_clahe(aeaj_handle* hd, const uint8_t* src, int h, int w, uint8_t* dst, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && src && dst && ws && h > 0 && w > 0, "aeaj_clahe: bad arguments");
+    AEAJ_REQUIRE(aligned(src, STAGE_PLANE_ALIGN) && aligned(dst, STAGE_PLANE_ALIGN) && aligned(ws, STAGE_WS_ALIGN), "aeaj_clahe: src / dst must be 4-byte and ws 256-byte aligned");
     StageWs S; stage_ws(ws, h, w, 0, 0, S);
     S.P.u8a = (uint8_t*)src; S.P.u8b = dst;
     int rc = push_stage(S, ST(stream)); if (rc) return rc;
@@ -311,14 +317,17 @@ static int prefilter_only(const uint8_t* src, int h, int w, uint8_t* dst, void* 
 }
 extern "C" int aeaj_gauss3(aeaj_handle* hd, const uint8_t* src, int h, int w, uint8_t* dst, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && src && dst && ws && h > 0 && w > 0, "aeaj_gauss3: bad arguments");
+    AEAJ_REQUIRE(aligned(src, STAGE_PLANE_ALIGN) && aligned(dst, STAGE_PLANE_ALIGN) && aligned(ws, STAGE_WS_ALIGN), "aeaj_gauss3: src / dst must be 4-byte and ws 256-byte aligned");
     return prefilter_only(src, h, w, dst, ws, stream, 2);
 }
 extern "C" int aeaj_bilateral5(aeaj_handle* hd, const uint8_t* src, int h, int w, uint8_t* dst, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && src && dst && ws && h > 0 && w > 0, "aeaj_bilateral5: bad arguments");
+    AEAJ_REQUIRE(aligned(src, STAGE_PLANE_ALIGN) && aligned(dst, STAGE_PLANE_ALIGN) && aligned(ws, STAGE_WS_ALIGN), "aeaj_bilateral5: src / dst must be 4-byte and ws 256-byte aligned");
     return prefilter_only(src, h, w, dst, ws, stream, 4);
 }
 extern "C" int aeaj_percentile_thresholds(aeaj_handle* hd, const uint8_t* src, int h, int w, double* thr, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && src && thr && ws && h > 0 && w > 0, "aeaj_percentile_thresholds: bad arguments");
+    AEAJ_REQUIRE(aligned(ws, STAGE_WS_ALIGN), "aeaj_percentile_thresholds: ws must be 256-byte aligned");
     StageWs S; stage_ws(ws, h, w, 0, 0, S);
     S.P.thr_d = thr;
     cudaStream_t st = ST(stream);
@@ -337,6 +346,8 @@ static int run_nms_hysteresis(aeaj_handle* hd, StageWs& S, cudaStream_t st) {
 }
 extern "C" int aeaj_canny_u8(aeaj_handle* hd, const uint8_t* src, int h, int w, const double* thr, uint8_t* edge, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && src && thr && edge && ws && h > 0 && w > 0, "aeaj_canny_u8: bad arguments");
+    AEAJ_REQUIRE(aligned(src, STAGE_PLANE_ALIGN) && aligned(edge, STAGE_PLANE_ALIGN) && aligned(ws, STAGE_WS_ALIGN),
+                 "aeaj_canny_u8: src / edge must be 4-byte and ws 256-byte aligned");
     StageWs S; stage_ws(ws, h, w, 0, 0, S);
     S.P.u8b = (uint8_t*)src; S.P.tap_edge = edge;
     cudaStream_t st = ST(stream);
@@ -346,6 +357,7 @@ extern "C" int aeaj_canny_u8(aeaj_handle* hd, const uint8_t* src, int h, int w, 
 }
 extern "C" int aeaj_canny(aeaj_handle* hd, const float* layer, int h, int w, uint8_t* edge, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && layer && edge && ws && h > 0 && w > 0, "aeaj_canny: bad arguments");
+    AEAJ_REQUIRE(aligned(layer, STAGE_PLANE_ALIGN) && aligned(ws, STAGE_WS_ALIGN), "aeaj_canny: layer must be 4-byte and ws 256-byte aligned");
     StageWs S; stage_ws(ws, h, w, 0, 0, S);
     S.P.u8a = S.u8a; S.P.u8b = S.u8b; S.P.tap_edge = edge;
     cudaStream_t st = ST(stream);
@@ -374,6 +386,7 @@ static int check_blocks(int h, int w, int mn, int mx) {
 extern "C" int aeaj_quadtree(aeaj_handle* hd, const uint8_t* edge, int h, int w, int mn, int mx, int32_t* leaves, uint8_t* states,
                              int32_t* counts, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && edge && leaves && states && counts && ws && h > 0 && w > 0, "aeaj_quadtree: bad arguments");
+    AEAJ_REQUIRE(aligned(ws, STAGE_WS_ALIGN), "aeaj_quadtree: ws must be 256-byte aligned");
     int rc = check_blocks(h, w, mn, mx); if (rc) return rc;
     StageWs S; stage_ws(ws, h, w, mn, mx, S);
     S.P.leaves = leaves; S.P.states = states; S.P.counts = counts;
@@ -401,11 +414,13 @@ static int stage_blocks(aeaj_handle* hd, bool inverse, float* layer, int h, int 
 extern "C" int aeaj_dct_quant(aeaj_handle* hd, const float* layer, int h, int w, float mid, float scale, const int32_t* leaves,
                               const int32_t* counts, int mn, int mx, const int32_t* const* qtab, int32_t* coef, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && layer && leaves && counts && qtab && coef && ws && h > 0 && w > 0, "aeaj_dct_quant: bad arguments");
+    AEAJ_REQUIRE(aligned(ws, STAGE_WS_ALIGN), "aeaj_dct_quant: ws must be 256-byte aligned");
     return stage_blocks(hd, false, (float*)layer, h, w, mid, scale, leaves, counts, mn, mx, qtab, coef, ws, ST(stream));
 }
 extern "C" int aeaj_dequant_idct(aeaj_handle* hd, const int32_t* coef, const int32_t* leaves, const int32_t* counts, int mn, int mx,
                                  const int32_t* const* qtab, int h, int w, float mid, float scale, float* layer, void* ws, void* stream) {
     AEAJ_REQUIRE(hd && layer && leaves && counts && qtab && coef && ws && h > 0 && w > 0, "aeaj_dequant_idct: bad arguments");
+    AEAJ_REQUIRE(aligned(ws, STAGE_WS_ALIGN), "aeaj_dequant_idct: ws must be 256-byte aligned");
     return stage_blocks(hd, true, layer, h, w, mid, scale, leaves, counts, mn, mx, qtab, (int32_t*)coef, ws, ST(stream));
 }
 
